@@ -63,8 +63,8 @@ extern "C" {
  * amount for every particle that stays in the beam.  The fast kernels therefore do no
  * arithmetic on it in the element maps: word 1 of an END_TURN record is the length of the
  * pass it closes (the whole lattice, or one segment of a segmented lattice), added once per
- * pass; and every record at which a particle can be lost (the three LIMIT_* tags and the
- * block records) carries `s_here`, the drift lengths from the start of the pass up to the
+ * pass; and every record at which a particle can be lost (the LIMIT_* tags and the block
+ * records) carries `s_here`, the drift lengths from the start of the pass up to the
  * record, added for the particles it removes.  The strict kernels ignore both and keep the
  * reference's per-particle sequential sum.  `element_index` is the position in the reference's
  * `Line.elements` list (what `at_element` reports).  Two encodings exist, selected by
@@ -86,9 +86,9 @@ enum xlb_tag {
   XLB_T_XYSHIFT = 8,        /* [hdr,dx][dy,0]                    elements.py:274-276  */
   XLB_T_SROTATION = 9,      /* [hdr,cos][sin,0]                  elements.py:379-390  */
   XLB_T_DIPOLE_EDGE = 10,   /* [hdr,r21][r43,0]                  elements.py:538-548  */
-  /* The three LIMIT_* records may carry the drift that follows the aperture (pack-time
-     peephole Limit* -> Drift): aux bit 4 (XLB_AUX_DRIFT), bit 5 = it is a DriftExact; the drift
-     length follows the record's own pairs as [length,0].                                     */
+  /* The LIMIT_* records may carry the drift that follows the aperture (pack-time peephole
+     Limit* -> Drift): aux bit 4 (XLB_AUX_DRIFT), bit 5 = it is a DriftExact; the drift length
+     follows the record's own pairs as [length,0] (LIMIT_POLYGON: in word 3, see there).       */
   XLB_T_LIMIT_RECT = 11,    /* aux bit 0: symmetric box (fast encoding only);
                                [hdr,min_x][max_x,min_y][max_y,s_here] elements.py:401-420 */
   XLB_T_LIMIT_ELLIPSE = 12, /* [hdr,a*a][b*b,1/(a*a)][1/(b*b),s_here] elements.py:429-442 */
@@ -103,7 +103,24 @@ enum xlb_tag {
                                interp,3 cubic spline); aux bit 4/5: the kick is followed by
                                a Drift / DriftExact of length word 1  spacecharge.py  */
   XLB_T_BEAMBEAM6D = 18,    /* [hdr,(double)n_slices] ...        BB6D.py:15-155       */
-  XLB_T__COUNT = 19,
+  /* Polygonal aperture (LimitPolygon; the reference's track raises, so the project defines it).
+     Same in both encodings: [hdr,i64 n_edges][s_here,drift_length or 0] then per stored edge
+     [y_lo,y_hi][x_lo,slope].  aux bits XLB_AUX_DRIFT / XLB_AUX_DRIFT_EXACT as on the other
+     LIMIT_* records (the drift length is word 3, always present).
+     The vertices V_k, k = 0..n-1, close into a polygon with edges V_k -> V_(k+1) mod n;
+     orientation does not matter, self-intersecting polygons follow the even-odd rule.  For every
+     edge with y_k != y_(k+1), (x_lo, y_lo) is the end with the smaller y, y_hi the other end's
+     y, and slope = (x_hi - x_lo) / (y_hi - y_lo) in fp64, rounded once at pack time; horizontal
+     edges are dropped (they can never be crossed).  A particle at (x, y) crosses an edge iff
+     y_lo <= y < y_hi and x < v, where t = y - y_lo; u = t * slope; v = x_lo + u are three
+     fp64 operations rounded to nearest with no fused multiply-add.  It is inside iff it crosses
+     an odd number of edges, else lost: NaN / inf coordinates are lost; on an axis-aligned
+     boundary points of the left and bottom edges are inside, of the right and top edges outside.
+     Every implementation of the predicate gives bit-identical loss flags.  A lattice with these
+     records carries XLB_F_POLYGONS.  Added without an ABI version change: a library that
+     predates the tag refuses the lattice in xlb_lattice_validate ("unknown tag").           */
+  XLB_T_LIMIT_POLYGON = 19,
+  XLB_T__COUNT = 20,
   /* Fused thin multipole -> [aperture] -> [drift] records (pack-time peephole).  The tag
      has bit 7 set and describes the block: bits 0-1 aperture kind (0 none, 1 symmetric
      rect, 2 rect, 3 ellipse), bit 2 curved multipole, bit 3 drift present, bit 4 that drift
@@ -170,6 +187,8 @@ typedef struct xlb_lattice {
 #define XLB_F_LOW_ORDER 8u   /* every MULTIPOLE / block record has order (aux) <= 3: the
                                 kernels with a straight-line Horner evaluation may be used
                                 (checked by xlb_lattice_validate; optional, never required) */
+#define XLB_F_POLYGONS 16u   /* the lattice holds LIMIT_POLYGON records (mandatory: checked by
+                                xlb_lattice_validate; the kernels that can track them are used) */
 
 /* Particle set, mirrors the attributes the reference's elements read and write
  * (SURVEY.md §8a row a2).  All arrays have length n.  chi and charge_ratio may be NULL

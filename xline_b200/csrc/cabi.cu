@@ -7,6 +7,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <cmath>
 #include <mutex>
 #include <string>
 #include <vector>
@@ -247,11 +248,12 @@ static const int kNumTables = static_cast<int>(sizeof(kTables) / sizeof(kTables[
 
 // What a call asks of a kernel family.
 struct Need {
-  bool strict, beamfields, bb6d, chi, trace;
+  bool strict, beamfields, bb6d, chi, trace, polygons;
   int max_order;  // highest multipole order the lattice may hold (255 = unknown)
 };
 static bool admits(const Variant &v, const Need &q) {
   if ((v.strict != 0) != q.strict) return false;
+  if ((v.polygons != 0) != q.polygons) return false;  // the twins with the LIMIT_POLYGON case
   if (q.strict) return (v.beamfields != 0) == q.beamfields;
   const int bf = q.beamfields ? (q.bb6d ? 2 : 1) : 0;
   if (v.beamfields != bf) return false;
@@ -361,6 +363,7 @@ static int track_device_impl(const xlb_lattice_t *lat, xlb_particles_t *p,
   need.bb6d = bb6d;
   need.chi = p->chi != nullptr;
   need.trace = o->trace != nullptr;
+  need.polygons = (lat->flags & XLB_F_POLYGONS) != 0;
   need.max_order = (lat->flags & XLB_F_LOW_ORDER) ? 3 : 255;
   const bool trace = need.trace;
   if (trace && (o->num_turns != 1 || o->trace_particles < 1))
@@ -736,6 +739,23 @@ int xlb_lattice_validate(const xlb_lattice_t *lat) {
         case XLB_T_LIMIT_RECT:
         case XLB_T_LIMIT_ELLIPSE: want = 3 + ((aux & XLB_AUX_DRIFT) ? 1 : 0); break;
         case XLB_T_LIMIT_RECT_ELLIPSE: want = 4 + ((aux & XLB_AUX_DRIFT) ? 1 : 0); break;
+        case XLB_T_LIMIT_POLYGON: {  // [hdr,n_edges][s_here,drift] then [y_lo,y_hi][x_lo,slope] per edge
+          const int64_t n_edges = static_cast<int64_t>(w[pos + 1]);
+          if (!(lat->flags & XLB_F_POLYGONS)) return fail(XLB_ELATTICE, "polygon record without XLB_F_POLYGONS");
+          if (n_edges < 1 || n_edges > lat->chunk_words || 2 + 2 * n_edges != pairs)
+            return fail(XLB_ELATTICE, "polygon record: n_edges < 1 or size != 2 + 2 * n_edges pairs");
+          if (pos + 2 * pairs + 2 > lat->chunk_words)
+            return fail(XLB_ELATTICE, "record runs past the end of its chunk");
+          for (int64_t e = 0; e < n_edges; ++e) {
+            double v[4];
+            memcpy(v, &w[pos + 4 + 4 * e], sizeof v);
+            if (!(std::isfinite(v[0]) && std::isfinite(v[1]) && std::isfinite(v[2]) && std::isfinite(v[3])))
+              return fail(XLB_ELATTICE, "polygon record: non-finite edge word");
+            if (!(v[0] < v[1])) return fail(XLB_ELATTICE, "polygon record: edge with y_lo >= y_hi");
+          }
+          want = pairs;
+          break;
+        }
         case XLB_T_MONITOR: want = 5; break;
         case XLB_T_BEAMBEAM4D:
         case XLB_T_SPACECHARGE:

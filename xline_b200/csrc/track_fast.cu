@@ -85,9 +85,12 @@ XLB_DEF_TRACE_VARIANT()
 #define XLB_X_DEF(P, T, M) XLB_DEF_VARIANT(P, T, M)
 XLB_SHAPES(XLB_X_DEF)
 #define XLB_X_ENTRY(P, T, M) XLB_VARIANT_ENTRY("fast/ppt" #P "/t" #T XLB_FAMILY, P, T, M),
+#define XLB_X_POLYGON_ENTRY(P, T, M) XLB_POLYGON_VARIANT_ENTRY("fast/ppt" #P "/t" #T XLB_FAMILY "/polygons", P, T, M),
 static const Variant family_table[] = {
     XLB_SHAPES(XLB_X_ENTRY)
     XLB_TRACE_ENTRY("fast/trace" XLB_FAMILY),
+    XLB_SHAPES(XLB_X_POLYGON_ENTRY)
+    XLB_POLYGON_TRACE_ENTRY("fast/trace" XLB_FAMILY "/polygons"),
 };
 
 #define XLB_CAT2(a, b) a##b

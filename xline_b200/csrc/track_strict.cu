@@ -42,6 +42,13 @@ static const Variant XLB_TABLE[] = {
     XLB_VARIANT_ENTRY("strict/ppt3/t128" XLB_SUFFIX, 3, 128, 3),
 #endif
     XLB_TRACE_ENTRY("strict/trace"),
+    XLB_POLYGON_VARIANT_ENTRY("strict/ppt1" XLB_SUFFIX "/polygons", 1, 256, 1),
+    XLB_POLYGON_VARIANT_ENTRY("strict/ppt2" XLB_SUFFIX "/polygons", 2, 256, 1),
+#if !XLB_BEAMFIELDS
+    XLB_POLYGON_VARIANT_ENTRY("strict/ppt2/t128" XLB_SUFFIX "/polygons", 2, 128, 3),
+    XLB_POLYGON_VARIANT_ENTRY("strict/ppt3/t128" XLB_SUFFIX "/polygons", 3, 128, 3),
+#endif
+    XLB_POLYGON_TRACE_ENTRY("strict/trace/polygons"),
 };
 const Variant *XLB_TABLE_FN(int *n) {
   *n = static_cast<int>(sizeof(XLB_TABLE) / sizeof(XLB_TABLE[0]));

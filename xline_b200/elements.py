@@ -315,9 +315,13 @@ class LimitEllipse(Element):
 
 
 class LimitPolygon(Element):
-    """Polygonal aperture (xline/elements.py:476-483).  The reference's ``track`` raises
-    ``NotImplementedError``; so does packing a line that contains one.  The class exists so that
-    the MAD-X ``octagon`` mapping (xline/loader_mad.py:229-242) and ``Line.from_dict`` work."""
+    """Polygonal aperture (xline/elements.py:476-483), the closed polygon through the vertices
+    ``(x_vertices[k], y_vertices[k])``.  The reference's ``track`` raises ``NotImplementedError``,
+    and by default so does packing a line that contains one.  With ``Line.polygon_apertures = True``
+    the line tracks it by this project's definition (include/xline_b200.h, DESIGN.md): even-odd
+    rule, half-open on axis-aligned boundaries (left and bottom edges inside, right and top edges
+    outside), NaN and inf coordinates lost.  ``LimitPolygon.track(p)`` on its own still raises.
+    The MAD-X ``octagon`` aperture (xline/loader_mad.py:229-242) maps to this class."""
 
     _base = (("x_vertices", tuple), ("y_vertices", tuple))
 

@@ -25,12 +25,13 @@ from . import elements as E
 T_END_TURN, T_END_CHUNK, T_DRIFT, T_DRIFT_EXACT, T_MULTIPOLE, T_MULTIPOLE_CURVED = range(6)
 T_CAVITY, T_RFMULTIPOLE, T_XYSHIFT, T_SROTATION, T_DIPOLE_EDGE = range(6, 11)
 T_LIMIT_RECT, T_LIMIT_ELLIPSE, T_LIMIT_RECT_ELLIPSE, T_MONITOR, T_SAWTOOTH_CAVITY = range(11, 16)
-T_BEAMBEAM4D, T_SPACECHARGE, T_BEAMBEAM6D = 16, 17, 18
+T_BEAMBEAM4D, T_SPACECHARGE, T_BEAMBEAM6D, T_LIMIT_POLYGON = 16, 17, 18, 19
 
 F_STRICT = 1
 F_BEAMFIELDS = 2
 F_BB6D = 4
 F_LOW_ORDER = 8  # every multipole-family record has order <= LOW_ORDER_MAX (straight-line Horner kernels)
+F_POLYGONS = 16  # the lattice holds LIMIT_POLYGON records (only the kernels that carry the case run it)
 LOW_ORDER_MAX = 3
 
 DEFAULT_CHUNK_WORDS = 2048  # 16 KiB per TMA bulk copy, 3 in flight per CTA
@@ -270,7 +271,48 @@ def _is_noop(el, name):
     return False
 
 
-def _pack_element(el, idx, strict, monitors):
+def polygon_edges(x_vertices, y_vertices):
+    """The edges a LIMIT_POLYGON record stores, ``[(y_lo, y_hi, x_lo, slope), ...]`` in vertex
+    order (include/xline_b200.h): every edge V_k -> V_(k+1) mod n that is not horizontal, from
+    its lower end, with ``slope = (x_hi - x_lo) / (y_hi - y_lo)`` rounded once here.  Raises
+    ``ValueError`` for a polygon the predicate is not defined for."""
+    xv = [float(v) for v in x_vertices]
+    yv = [float(v) for v in y_vertices]
+    if len(xv) != len(yv) or len(xv) < 3:
+        raise ValueError("LimitPolygon needs x_vertices and y_vertices of the same length >= 3 "
+                         "(got %d and %d)" % (len(xv), len(yv)))
+    if not all(math.isfinite(v) for v in xv + yv):
+        raise ValueError("LimitPolygon has a non-finite vertex")
+    edges = []
+    n = len(xv)
+    for k in range(n):
+        x0, y0, x1, y1 = xv[k], yv[k], xv[(k + 1) % n], yv[(k + 1) % n]
+        if y0 == y1:
+            continue  # horizontal: never crossed
+        if y1 < y0:
+            x0, y0, x1, y1 = x1, y1, x0, y0
+        slope = (x1 - x0) / (y1 - y0)
+        if not math.isfinite(slope):
+            raise ValueError("LimitPolygon edge %d has a non-finite slope" % k)
+        edges.append((y0, y1, x0, slope))
+    if not edges:
+        raise ValueError("LimitPolygon has no edge that is not horizontal")
+    return edges
+
+
+def _pack_limit_polygon(el, idx):
+    """XLB_T_LIMIT_POLYGON: [hdr,n_edges][s_here,drift_length] then [y_lo,y_hi][x_lo,slope] per
+    stored edge; the same words in both encodings."""
+    edges = polygon_edges(el.x_vertices, el.y_vertices)
+    rec = _Rec(T_LIMIT_POLYGON, 0, idx)
+    rec.w[1] = _i2u(len(edges))
+    rec.path_length_here().f(0.0)  # word 3: the length of a fused drift (pack_line)
+    for y_lo, y_hi, x_lo, slope in edges:
+        rec.f(y_lo, y_hi).f(x_lo, slope)
+    return rec
+
+
+def _pack_element(el, idx, strict, monitors, polygons=False):
     name = type(el).__name__
     if name == "Drift":
         rec = _Rec(T_DRIFT, 0, idx, el.length)
@@ -347,7 +389,11 @@ def _pack_element(el, idx, strict, monitors):
     if name == "BeamBeam6D":
         return _pack_beambeam6d(el, idx)
     if name == "LimitPolygon":
-        raise NotImplementedError  # xline/elements.py:483
+        if polygons:
+            return _pack_limit_polygon(el, idx)
+        # the reference's LimitPolygon.track raises (xline/elements.py:483); tracking one is opt-in
+        raise NotImplementedError("LimitPolygon apertures are tracked only on request: set "
+                                  "Line.polygon_apertures = True (pack_line(..., polygons=True))")
     raise ValueError("element type %s is not supported by the B200 tracking kernel" % name)
 
 
@@ -544,7 +590,7 @@ SEG_MAIN, SEG_BB6D = 0, 1
 
 
 def pack_line(elements, strict=False, chunk_words=DEFAULT_CHUNK_WORDS, drop_noops=True, fuse=True,
-              merge=True, split_lenses=True, hx_only=True):
+              merge=True, split_lenses=True, hx_only=True, polygons=False):
     """Pack ``elements`` (the ``Line.elements`` list).  ``element_index`` in every record
     is the position in that list, so ``at_element`` matches the reference's indexing even
     though exact no-ops (zero-length drifts, all-zero multipoles, disabled lenses) are not
@@ -557,7 +603,11 @@ def pack_line(elements, strict=False, chunk_words=DEFAULT_CHUNK_WORDS, drop_noop
 
     ``hx_only`` (fast encoding only): flag curved block records whose ``hyl`` is exactly zero with
     ``XLB_HDR_HX_ONLY`` so that the kernel leaves the ``hyl`` terms out (same bits, fewer
-    instructions); ``False`` packs them for the general formula (the tests compare the two)."""
+    instructions); ``False`` packs them for the general formula (the tests compare the two).
+
+    ``polygons``: pack ``LimitPolygon`` apertures as XLB_T_LIMIT_POLYGON records (the project's
+    own definition, see include/xline_b200.h).  ``False``, the default, refuses them with
+    ``NotImplementedError`` like the reference's ``LimitPolygon.track``."""
     assert chunk_words % 2 == 0 and chunk_words >= 16
     monitors = dict(layout=[], words=0)
     recs = []
@@ -584,13 +634,18 @@ def pack_line(elements, strict=False, chunk_words=DEFAULT_CHUNK_WORDS, drop_noop
             recs.append((rec.tag, rec.words(), rec.s_word, rec.drift_len, rec.drift_before))
             continue
         nxt = type(live[pos][1]).__name__ if pos < len(live) else None
-        if fuse and name in ("LimitRect", "LimitEllipse", "LimitRectEllipse") and nxt in ("Drift", "DriftExact"):
-            # aperture -> drift in one record (aux bit 4; the drift length in a pair of its own)
+        if fuse and name in ("LimitRect", "LimitEllipse", "LimitRectEllipse", "LimitPolygon") and \
+                nxt in ("Drift", "DriftExact"):
+            # aperture -> drift in one record (aux bit 4; the drift length in a pair of its own,
+            # in word 3 of a polygon record)
             d = live[pos][1]
             pos += 1
-            rec = _pack_element(el, idx, strict, monitors)
+            rec = _pack_element(el, idx, strict, monitors, polygons)
             rec.aux |= AUX_DRIFT | (AUX_DRIFT_EXACT if nxt == "DriftExact" else 0)
-            rec.f(d.length, 0.0)
+            if rec.tag == T_LIMIT_POLYGON:
+                rec.w[3] = _f2u(float(d.length))
+            else:
+                rec.f(d.length, 0.0)
             rec.drift_len = float(d.length)
             counts[rec.tag] = counts.get(rec.tag, 0) + 1
             recs.append((rec.tag, rec.words(), rec.s_word, rec.drift_len, rec.drift_before))
@@ -621,7 +676,7 @@ def pack_line(elements, strict=False, chunk_words=DEFAULT_CHUNK_WORDS, drop_noop
                 pos += 1
             rec = _pack_thin_block(el, idx, aper, drift, strict)
         else:
-            rec = _pack_element(el, idx, strict, monitors)
+            rec = _pack_element(el, idx, strict, monitors, polygons)
         tag = rec.tag
         counts[tag] = counts.get(tag, 0) + 1
         if not hx_only:
@@ -633,6 +688,8 @@ def pack_line(elements, strict=False, chunk_words=DEFAULT_CHUNK_WORDS, drop_noop
             flags |= F_BB6D
         if tag in (T_BEAMBEAM4D, T_SPACECHARGE) or (tag == T_BEAMBEAM6D and not split):
             flags |= F_BEAMFIELDS
+        if tag == T_LIMIT_POLYGON:
+            flags |= F_POLYGONS
     horner_orders = [(int(r[0]) >> 8) & 0xFF for tag, r, _, _, _ in recs
                      if tag in (T_MULTIPOLE, T_MULTIPOLE_CURVED) or (tag & 0xC0) == T_THIN_BLOCK]
     if all(o <= LOW_ORDER_MAX for o in horner_orders):
@@ -723,6 +780,9 @@ def algorithmic_ops(elements):
             total += 6
         elif name == "LimitRectEllipse":
             total += 10
+        elif name == "LimitPolygon":  # per stored edge: two compares (y slab), sub, mul, add, compare
+            yv = list(el.y_vertices)
+            total += 6 * sum(1 for k in range(len(yv)) if yv[k] != yv[(k + 1) % len(yv)])
         elif name in ("BeamBeam4D", "SCCoasting", "SCQGaussProfile", "SCInterpolatedProfile"):
             if el.enabled:
                 msd = 1e-10 if name == "BeamBeam4D" else el.min_sigma_diff

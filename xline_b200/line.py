@@ -26,7 +26,8 @@ def _is_thick(element):
 
 class Line(E.Element):
     _base = (("elements", tuple), ("element_names", tuple))
-    _pack_options = ("fuse_records", "chunk_words", "merge_multipoles", "split_lenses", "flag_horizontal_bends")
+    _pack_options = ("fuse_records", "chunk_words", "merge_multipoles", "split_lenses", "flag_horizontal_bends",
+                     "polygon_apertures")
 
     def __setattr__(self, name, value):
         # edit tracking (elements.py): the element list and the packing options stamp the line,
@@ -50,6 +51,9 @@ class Line(E.Element):
         self.merge_multipoles = True  # fast encoding: co-located thin multipoles become one kick
         self.split_lenses = True      # fast encoding: BeamBeam6D lenses run as kernels of their own
         self.flag_horizontal_bends = True  # fast encoding: XLB_HDR_HX_ONLY on curved blocks with hyl == 0
+        # track LimitPolygon apertures with the project's even-odd rule (include/xline_b200.h); off,
+        # a line that holds one refuses to pack, like the reference's LimitPolygon.track
+        self.polygon_apertures = False
         self._monitor_buf = None
         self._buffers_key = None
         self.loss_tally = None
@@ -297,14 +301,14 @@ class Line(E.Element):
             chunk_words = self.chunk_words
         self._current_stamp()
         key = ("host", bool(strict), chunk_words, self.fuse_records, self.merge_multipoles, self.split_lenses,
-               self.flag_horizontal_bends, getattr(self, "_keep_noops", False))
+               self.flag_horizontal_bends, self.polygon_apertures, getattr(self, "_keep_noops", False))
         hit = self._cache.get("host_%d" % strict)
         if hit is not None and hit[0] == key:
             return hit[1]
         kw = {} if chunk_words is None else {"chunk_words": chunk_words}
         packed = pack_line(self.elements, strict=strict, fuse=self.fuse_records,
                            merge=self.merge_multipoles, split_lenses=self.split_lenses,
-                           hx_only=self.flag_horizontal_bends,
+                           hx_only=self.flag_horizontal_bends, polygons=self.polygon_apertures,
                            drop_noops=not getattr(self, "_keep_noops", False), **kw)
         lat = packed.c_lattice()
         _cabi.check(_cabi.lib().xlb_lattice_validate(C.byref(lat)))
@@ -469,6 +473,8 @@ class Line(E.Element):
             solo = self._cache.get(("solo", i))
             if solo is None or solo.elements[0] is not el:
                 solo = self._cache[("solo", i)] = Line([el], ["e"])
+            if solo.polygon_apertures != self.polygon_apertures:
+                solo.polygon_apertures = self.polygon_apertures
             solo.track(p, _count_turns=False, _element_offset=i)
             out.append(p.copy())
         if end:

@@ -761,7 +761,8 @@ def iter_from_madx_sequence(sequence, classes, ignored_madtypes=(), exact_drift=
                 yield ee.name + "_aperture", classes["LimitEllipse"](a=ap[0], b=ap[0])
             elif ee.apertype == "rectellipse":
                 yield ee.name + "_aperture", classes["LimitRectEllipse"](max_x=ap[0], max_y=ap[1], a=ap[2], b=ap[3])
-            elif ee.apertype == "octagon":  # loader_mad.py:229-242 (LimitPolygon: tracking raises, as there)
+            elif ee.apertype == "octagon":  # loader_mad.py:229-242; tracked with Line.polygon_apertures = True
+                # (8 vertices, 6 stored edges: the top and bottom edges are horizontal)
                 v1 = (ap[0], ap[0] * math.tan(ap[2]))
                 v2 = (ap[1] / math.tan(ap[3]), ap[1])
                 yield ee.name + "_aperture", classes["LimitPolygon"](
