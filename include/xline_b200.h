@@ -290,6 +290,50 @@ int xlb_get_stats(xlb_track_stats_t *out);
 int xlb_compact_alive_device(const int64_t *state, int64_t n, int32_t *idx_out,
                              int32_t *n_out, void *stream);
 
+/* ---------------------------------------------------------------------------------
+ * Beam moments (DESIGN.md §4.6): the number of particles and the first and second moments of
+ * (x, px, y, py, zeta, delta) over the surviving beam, taken on the device.
+ *
+ * A particle counts iff state == 1 and its six coordinates are all finite; alive particles with
+ * a non-finite coordinate are counted apart.  A store is XLB_MOMENT_WORDS fp64 words:
+ *   [0] n   [1] n_nonfinite   then XLB_MOMENT_PAIRS (hi, lo) pairs: the 6 sums  Σu  in the
+ *   order x px y py zeta delta (pair 0..5), then the 21 sums  Σu·v  for u <= v, upper triangle in
+ *   row-major order: xx xpx xy xpy xzeta xdelta pxpx pxy ... deltadelta (pair 6..26).
+ * Each product u·v is taken exactly (TwoProduct with an FMA), so each sum is a sum of exact
+ * terms, accumulated in double-double.
+ * Accuracy: |hi + lo - exact sum| <= 3·2^-106·ceil(log2 n)·Σ|terms| (n = the particle count of
+ *   the call), which is <= 2^-100·Σ|terms| up to n = 2^21.
+ * Reproducibility: the summation order is a fixed binary tree over the slot index 0..n-1, so a
+ *   store is bitwise independent of the kernel family, the particles per thread, the threads per
+ *   block, turns_per_launch, turns_per_item, survivor compaction and the launch-length schedule.
+ * --------------------------------------------------------------------------------- */
+#define XLB_MOMENT_WORDS 56
+#define XLB_MOMENT_PAIRS 27
+#define XLB_MOMENT_FIRST 2  /* word of the first pair (Σx hi) */
+
+/* Store turns of one tracking call: store k is taken after t_k = start + k·skip turns of the
+ * call, for k < num_stores and t_k <= num_turns (t = 0 is the beam before the first turn, at the
+ * start of the line).  Stores with t_k > num_turns are not written; every other store is, also
+ * when the beam is already empty.  num_stores, start >= 0, skip >= 1. */
+typedef struct xlb_moments_spec {
+  int64_t num_stores;
+  int64_t start;
+  int64_t skip;
+} xlb_moments_spec_t;
+
+/* One snapshot of the particles (device pointers; x..delta and state are read) into the
+ * XLB_MOMENT_WORDS words at `out` (device).  Enqueued on `stream`, no synchronisation. */
+int xlb_beam_moments_device(const xlb_particles_t *particles, double *out, void *stream);
+
+/* xlb_track_device, plus the stores of `spec` into out[k·XLB_MOMENT_WORDS ..] (device, capacity
+ * spec->num_stores stores).  Launches are cut so that one ends on every store turn, and the
+ * reduction runs on the stream after it: the particles are tracked exactly as without stores.
+ * Like a job split by turns_per_launch, it synchronises the stream between launches.
+ * Strict, beam-field and segmented lattices; a trace is refused (XLB_EINVAL). */
+int xlb_track_device_moments(const xlb_lattice_t *lattice, xlb_particles_t *particles,
+                             const xlb_track_options_t *opts, const xlb_moments_spec_t *spec,
+                             double *out, void *stream);
+
 /* Register-resident independent-DFMA-chain microbenchmark: the measured FP64 pipe peak of
  * the current device in FLOP/s (2 flops per DFMA), best of `repeats`.  The roofline
  * denominator of bench.py (MEASURED_PEAKS.json has no FP64 entry). */

@@ -9,8 +9,10 @@ __version__ = "0.1.0"
 from . import elements
 from .elements import *  # noqa: F401,F403
 from .line import Line
+from .moments import BeamMoments, beam_moments
 from .particles import Particles
 
 XlineTestParticles = Particles  # the reference's name (xline/particles.py:4)
 
-__all__ = list(elements.__all__) + ["Line", "Particles", "XlineTestParticles", "elements"]
+__all__ = list(elements.__all__) + ["Line", "Particles", "XlineTestParticles", "elements", "BeamMoments",
+                                    "beam_moments"]

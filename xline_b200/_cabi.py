@@ -11,12 +11,16 @@ LIB_PATH = os.path.join(_HERE, "libxline_b200.so")
 
 ABI_VERSION = 4
 OPT_NO_TURN_COUNT = 1  # xlb_track_options_t::flags
+MOMENT_WORDS = 56  # XLB_MOMENT_WORDS: words of one beam-moment store
+MOMENT_PAIRS = 27  # XLB_MOMENT_PAIRS: (hi, lo) sums of a store
+MOMENT_FIRST = 2   # XLB_MOMENT_FIRST: word of the first pair, after n and n_nonfinite
 
 EXPORTS = (
     "xlb_abi_version", "xlb_last_error", "xlb_lattice_validate", "xlb_track_device",
     "xlb_track_device_timed", "xlb_track_host", "xlb_get_stats", "xlb_compact_alive_device",
     "xlb_measure_fp64_peak", "xlb_measure_dfma_latency", "xlb_kernel_variant_count",
-    "xlb_kernel_variant_info", "xlb_selftest_exact_division",
+    "xlb_kernel_variant_info", "xlb_selftest_exact_division", "xlb_beam_moments_device",
+    "xlb_track_device_moments",
 )
 
 
@@ -51,6 +55,10 @@ class TrackOptions(C.Structure):
     ]
 
 
+class MomentsSpec(C.Structure):
+    _fields_ = [("num_stores", C.c_int64), ("start", C.c_int64), ("skip", C.c_int64)]
+
+
 class TrackStats(C.Structure):
     _fields_ = [
         ("n_alive_in", C.c_int64), ("n_alive_out", C.c_int64), ("kernel_launches", C.c_int32),
@@ -79,6 +87,11 @@ def lib():
     for fn in (L.xlb_track_device, L.xlb_track_device_timed):
         fn.argtypes = [C.POINTER(Lattice), C.POINTER(Particles), C.POINTER(TrackOptions), C.c_void_p]
         fn.restype = C.c_int
+    L.xlb_track_device_moments.argtypes = [C.POINTER(Lattice), C.POINTER(Particles), C.POINTER(TrackOptions),
+                                           C.POINTER(MomentsSpec), C.c_void_p, C.c_void_p]
+    L.xlb_track_device_moments.restype = C.c_int
+    L.xlb_beam_moments_device.argtypes = [C.POINTER(Particles), C.c_void_p, C.c_void_p]
+    L.xlb_beam_moments_device.restype = C.c_int
     L.xlb_track_host.argtypes = [C.POINTER(Lattice), C.POINTER(Particles), C.POINTER(TrackOptions)]
     L.xlb_track_host.restype = C.c_int
     L.xlb_get_stats.argtypes = [C.POINTER(TrackStats)]

@@ -160,6 +160,8 @@ struct Scratch {
   const double *sched_x = nullptr;
   long long sched_n = 0;
   double sched_rate = -1.0;
+  double *moments = nullptr;  // beam-moment partial sums (moments.cu)
+  size_t moments_cap = 0;     // doubles
 };
 
 // Launch length for a loss rate: lanes of lost particles idle until the next launch boundary,
@@ -223,6 +225,43 @@ static int ensure_compaction_scratch(Scratch *s, long long n) {
   }
   return XLB_OK;
 }
+
+// One beam-moment store of slots 0..n-1 into out[0..XLB_MOMENT_WORDS), enqueued on `st`.
+static int beam_moments(Scratch *s, const xlb_particles_t *p, double *out, cudaStream_t st) {
+  const size_t words = beam_moments_scratch_words(p->n);
+  if (words > s->moments_cap) {
+    if (s->moments) cudaFree(s->moments);
+    s->moments = nullptr;
+    s->moments_cap = 0;
+    XLB_CUDA(cudaMalloc(&s->moments, words * sizeof(double)));
+    s->moments_cap = words;
+  }
+  XLB_CUDA(beam_moments_launch(p->x, p->px, p->y, p->py, p->zeta, p->delta,
+                               reinterpret_cast<const long long *>(p->state), p->n, s->moments, out, st));
+  return XLB_OK;
+}
+
+// The stores of one xlb_track_device_moments call: store k after t_k = start + k * skip turns.
+struct MomentStores {
+  xlb_moments_spec_t spec;
+  double *out;
+  long long k = 0;  // next store
+  // turn of the next store, or past num_turns when none is left
+  long long next_turn(long long num_turns) const {
+    if (k >= spec.num_stores || spec.start > num_turns) return num_turns + 1;
+    if (k > 0 && spec.skip > (num_turns - spec.start) / k) return num_turns + 1;
+    return spec.start + k * spec.skip;
+  }
+  // takes every store due after `done` turns (t_k <= done <= num_turns)
+  int take(Scratch *s, const xlb_particles_t *p, long long done, long long num_turns, cudaStream_t st) {
+    int rc;
+    while (next_turn(num_turns) <= done) {
+      if ((rc = beam_moments(s, p, out + static_cast<size_t>(k) * XLB_MOMENT_WORDS, st)) != XLB_OK) return rc;
+      ++k;
+    }
+    return XLB_OK;
+  }
+};
 
 static int compact_alive(const long long *state, long long n, int *idx_out, int *block_sums,
                          int *n_out, cudaStream_t st) {
@@ -337,15 +376,28 @@ static int check_particles(const xlb_particles_t *p) {
   return XLB_OK;
 }
 
+// `stores` (optional): beam-moment stores taken on the stream after the launch that ends on their
+// turn; launches are cut at the store turns.
 static int track_device_impl(const xlb_lattice_t *lat, xlb_particles_t *p,
-                             const xlb_track_options_t *o, cudaStream_t st, bool timed) {
+                             const xlb_track_options_t *o, cudaStream_t st, bool timed,
+                             MomentStores *stores = nullptr) {
   memset(&g_stats, 0, sizeof(g_stats));
   int rc;
   if ((rc = check_lattice_header(lat)) != XLB_OK) return rc;
   if ((rc = check_particles(p)) != XLB_OK) return rc;
   if (!o) return fail(XLB_EINVAL, "options is null");
   if (o->num_turns < 0) return fail(XLB_EINVAL, "num_turns < 0");
-  if (p->n == 0 || o->num_turns == 0) return XLB_OK;
+  if (stores && o->trace) return fail(XLB_EINVAL, "beam-moment stores do not combine with a trace");
+  if (p->n == 0 || o->num_turns == 0) {
+    if (!stores) return XLB_OK;
+    Scratch *s = nullptr;
+    if ((rc = get_scratch(&s)) != XLB_OK) return rc;
+    std::lock_guard<std::recursive_mutex> call_lock(s->call_mu);
+    if (s->have_done) XLB_CUDA(cudaStreamWaitEvent(st, s->done, 0));
+    rc = stores->take(s, p, o->num_turns, o->num_turns, st);
+    if (cudaEventRecord(s->done, st) == cudaSuccess) s->have_done = true;
+    return rc;
+  }
 
   const bool strict = (lat->flags & XLB_F_STRICT) != 0;
   const bool beamfields = (lat->flags & XLB_F_BEAMFIELDS) != 0;
@@ -474,7 +526,7 @@ static int track_device_impl(const xlb_lattice_t *lat, xlb_particles_t *p,
   const int *idx = nullptr;
   long long lost_since_compact = 0;
   const bool segmented = seg < o->num_turns;
-  if (segmented) XLB_CUDA(cudaMemsetAsync(s->n_lost, 0, sizeof(unsigned int), st));
+  if (segmented || stores) XLB_CUDA(cudaMemsetAsync(s->n_lost, 0, sizeof(unsigned int), st));
   // Launch-length ramp: a beam that is scraped hard in its first turns (SURVEY 8(d): 80 % of the
   // C2 beam within a few turns) would keep those lanes idle for a whole launch.  A segmented job
   // on a particle set not seen before starts with a launch of ONE turn; after every launch the
@@ -507,8 +559,10 @@ static int track_device_impl(const xlb_lattice_t *lat, xlb_particles_t *p,
   }
   float total_ms = 0.f;
   long long lost_before_launch = 0;
+  if (stores && (rc = stores->take(s, p, 0, o->num_turns, st)) != XLB_OK) return rc;
   for (int done = 0; done < o->num_turns && n_active > 0;) {
-    const int turns = std::min(ramp ? cur_len : seg, o->num_turns - done);
+    int turns = std::min(ramp ? cur_len : seg, o->num_turns - done);
+    if (stores) turns = static_cast<int>(std::min<long long>(turns, stores->next_turn(o->num_turns) - done));
     a.num_turns = turns;
     a.n = n_active;
     a.idx = idx;
@@ -581,6 +635,7 @@ static int track_device_impl(const xlb_lattice_t *lat, xlb_particles_t *p,
     g_stats.threads = threads;
     }
     done += turns;
+    if (stores && (rc = stores->take(s, p, done, o->num_turns, st)) != XLB_OK) return rc;
     if (done >= o->num_turns) break;
     // survivors: read the loss counter; re-compact when enough lanes went idle
     XLB_CUDA(cudaMemcpyAsync(&s->h_pinned[0], s->n_lost, sizeof(unsigned int),
@@ -606,6 +661,8 @@ static int track_device_impl(const xlb_lattice_t *lat, xlb_particles_t *p,
       g_stats.compactions += 1;
     }
   }
+  // a beam lost entirely before num_turns: the remaining stores see it empty
+  if (stores && (rc = stores->take(s, p, o->num_turns, o->num_turns, st)) != XLB_OK) return rc;
   if (timed) {
     XLB_CUDA(cudaEventRecord(s->ev1, st));
     XLB_CUDA(cudaEventSynchronize(s->ev1));
@@ -835,6 +892,31 @@ int xlb_track_device(const xlb_lattice_t *lattice, xlb_particles_t *particles,
 int xlb_track_device_timed(const xlb_lattice_t *lattice, xlb_particles_t *particles,
                            const xlb_track_options_t *opts, void *stream) {
   return track_device_impl(lattice, particles, opts, static_cast<cudaStream_t>(stream), true);
+}
+
+int xlb_track_device_moments(const xlb_lattice_t *lattice, xlb_particles_t *particles,
+                             const xlb_track_options_t *opts, const xlb_moments_spec_t *spec, double *out,
+                             void *stream) {
+  if (!spec) return fail(XLB_EINVAL, "moments spec is null");
+  if (spec->num_stores < 0 || spec->start < 0 || spec->skip < 1)
+    return fail(XLB_EINVAL, "moments spec needs num_stores >= 0, start >= 0, skip >= 1");
+  if (spec->num_stores > 0 && !out) return fail(XLB_EINVAL, "moments out is null");
+  MomentStores stores{*spec, out};
+  return track_device_impl(lattice, particles, opts, static_cast<cudaStream_t>(stream), false, &stores);
+}
+
+int xlb_beam_moments_device(const xlb_particles_t *particles, double *out, void *stream) {
+  int rc;
+  if ((rc = check_particles(particles)) != XLB_OK) return rc;
+  if (!out) return fail(XLB_EINVAL, "out is null");
+  Scratch *s = nullptr;
+  if ((rc = get_scratch(&s)) != XLB_OK) return rc;
+  std::lock_guard<std::recursive_mutex> call_lock(s->call_mu);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (s->have_done) XLB_CUDA(cudaStreamWaitEvent(st, s->done, 0));
+  rc = beam_moments(s, particles, out, st);
+  if (cudaEventRecord(s->done, st) == cudaSuccess) s->have_done = true;
+  return rc;
 }
 
 int xlb_compact_alive_device(const int64_t *state, int64_t n, int32_t *idx_out, int32_t *n_out,

@@ -61,6 +61,13 @@ int strict_selftest_division(const double *d_divisors, int n_div, int mode, int 
                              unsigned long long seed, int span, unsigned long long *d_mismatches,
                              void *stream);
 
+// Beam moments of slots 0..n-1 into the XLB_MOMENT_WORDS words at `out` (moments.cu); `scratch`
+// holds beam_moments_scratch_words(n) doubles.
+size_t beam_moments_scratch_words(long long n);
+cudaError_t beam_moments_launch(const double *x, const double *px, const double *y, const double *py,
+                                const double *zeta, const double *delta, const long long *state, long long n,
+                                double *scratch, double *out, cudaStream_t st);
+
 // variant tables, one per translation unit (kernel family)
 const Variant *fast_lean_variants(int *n);
 const Variant *fast_lean_nc_variants(int *n);

@@ -24,6 +24,23 @@ def _is_thick(element):
     return bool(getattr(element, "isthick", False)) or isinstance(element, _thick)
 
 
+def _c_particles(p):
+    """``(xlb_particles_t, {column: tensor})`` over the columns of ``p`` (made contiguous in place)."""
+    cols = {}
+    for k, t in p._columns():
+        if not t.is_contiguous():
+            t = t.contiguous()
+            p._assign(k, t)
+        cols[k] = t
+    cp = _cabi.Particles()
+    cp.n = len(p)
+    for k, t in cols.items():
+        setattr(cp, k, t.data_ptr())
+    cp.q0, cp.mass0, cp.p0c = p.q0, p.mass0, p.p0c
+    cp.beta0, cp.gamma0, cp.energy0 = p.beta0, p.gamma0, p.energy0
+    return cp, cols
+
+
 class Line(E.Element):
     _base = (("elements", tuple), ("element_names", tuple))
     _pack_options = ("fuse_records", "chunk_words", "merge_multipoles", "split_lenses", "flag_horizontal_bends",
@@ -327,8 +344,8 @@ class Line(E.Element):
 
     # ------------------------------------------------------------------ the hot path
     def track(self, p, num_turns=1, strict=False, turns_per_launch=0, particles_per_thread=0,
-              threads_per_block=0, timed=False, turns_per_item=0, compact_threshold=0.0, _trace=None,
-              _count_turns=True,
+              threads_per_block=0, timed=False, turns_per_item=0, compact_threshold=0.0, moments=None,
+              _trace=None, _count_turns=True,
               _element_offset=0, _general_kernels=False):
         """``for el in self.elements: el.track(p)`` (xline/line.py:89-95), ``num_turns``
         times, in one fused kernel launch on ``p``'s GPU.  Mutates ``p`` in place and
@@ -337,6 +354,8 @@ class Line(E.Element):
         ``strict=True`` selects the reference-operation-order kernel (parity instrument).
         ``turns_per_launch`` > 0 splits the job and re-compacts survivors between launches
         (when more than ``compact_threshold`` of the lanes went idle; 0 = the library's 1/128).
+        ``moments``: a ``BeamMoments`` that receives the beam moments on its store turns of this
+        call (``xline_b200.moments``); the particles are tracked exactly as without.
         """
         if p.device.type != "cuda":
             raise RuntimeError(
@@ -347,21 +366,14 @@ class Line(E.Element):
         with torch.cuda.device(dev):
             packed, words = self._device_lattice(dev, strict)
             n = len(p)
-            if n == 0 or num_turns == 0:
+            if moments is not None:
+                moments._check_target(p)
+            elif n == 0 or num_turns == 0:
                 return None
             lat = packed.c_lattice(words.data_ptr())
             if _general_kernels:  # test hook: the unspecialised kernel family (chi column, any order)
                 lat.flags &= ~F_LOW_ORDER
-            cols = {}
-            for k, t in p._columns():
-                if not t.is_contiguous():
-                    t = t.contiguous()
-                    p._assign(k, t)
-                cols[k] = t
-            cp = _cabi.Particles()
-            cp.n = n
-            for k, t in cols.items():
-                setattr(cp, k, t.data_ptr())
+            cp, cols = _c_particles(p)
             # one species (chi == 1 throughout, the reference's default) is the fast case of the C ABI:
             # no chi column is handed over and the kernels without a chi register run (4 particles per
             # thread).  The answer is cached on the tensor's storage and version counter, so an in-place
@@ -373,8 +385,6 @@ class Line(E.Element):
                     p._chi_key, p._chi_trivial = ckey, bool((chi == 1.0).all())
                 if p._chi_trivial and not _general_kernels:
                     cp.chi = None
-            cp.q0, cp.mass0, cp.p0c = p.q0, p.mass0, p.p0c
-            cp.beta0, cp.gamma0, cp.energy0 = p.beta0, p.gamma0, p.energy0
             # tallies and monitor storage belong to one state of the line on one device: a line that
             # was edited since (other element count, other monitor layout) gets fresh ones
             bkey = (self._cache.get("generation"), packed.n_elements, packed.monitor_words, dev)
@@ -413,8 +423,16 @@ class Line(E.Element):
                 opts.monitor_data = self._monitor_buf.data_ptr()
                 opts.monitor_words = packed.monitor_words
             stream = torch.cuda.current_stream(dev).cuda_stream
-            fn = lib.xlb_track_device_timed if timed else lib.xlb_track_device
-            _cabi.check(fn(C.byref(lat), C.byref(cp), C.byref(opts), C.c_void_p(stream)))
+            if moments is not None:
+                if timed:
+                    raise ValueError("timed=True does not combine with moments")
+                _cabi.check(lib.xlb_track_device_moments(C.byref(lat), C.byref(cp), C.byref(opts),
+                                                         C.byref(moments._spec()), C.c_void_p(moments.data.data_ptr()),
+                                                         C.c_void_p(stream)))
+                moments.beta0gamma0 = p.beta0 * p.gamma0
+            else:
+                fn = lib.xlb_track_device_timed if timed else lib.xlb_track_device
+                _cabi.check(fn(C.byref(lat), C.byref(cp), C.byref(opts), C.c_void_p(stream)))
             self.last_stats = _cabi.stats()
             if packed.monitor_words > 0:
                 self._publish_monitors(packed)

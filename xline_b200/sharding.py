@@ -6,7 +6,7 @@ shards into independent units: rank ``r`` owns the contiguous block
 ``[r*N/W, (r+1)*N/W)``, the packed lattice (<= a few MB) is replicated, and there is no
 data-path collective.  ``torch.distributed`` (NCCL over NVLink on GPUs, gloo in the CPU
 tests) is used only after the kernel: a SUM all-reduce of the per-element loss tallies and
-a gather of BeamMonitor slabs / survivor counts.
+a gather of BeamMonitor slabs / survivor counts, and a fold of the per-rank beam-moment sums.
 """
 import torch
 import torch.distributed as dist
@@ -62,6 +62,28 @@ def merge_monitor(data, dst=0):
     dist.all_reduce(filled, op=dist.ReduceOp.SUM)
     dist.all_reduce(count, op=dist.ReduceOp.SUM)
     out = torch.where(count > 0, filled, torch.full_like(filled, float("nan")))
+    return out
+
+
+def merge_moments(m):
+    """Global beam moments from the per-rank ``BeamMoments`` ``m``: all-gathers the stores of every
+    rank and folds them in rank order (counts exactly, the double-double sums with the addition of
+    the device reduction), so every rank holds the same bits.  Returns a new ``BeamMoments``."""
+    from .moments import BeamMoments, dd_add
+
+    out = BeamMoments(m.num_stores, m.start, m.skip, device=m.data.device)
+    out.beta0gamma0 = m.beta0gamma0
+    if not (_initialized() and dist.get_world_size() > 1):
+        out.data.copy_(m.data)
+        return out
+    parts = [torch.empty_like(m.data) for _ in range(dist.get_world_size())]
+    dist.all_gather(parts, m.data.contiguous())
+    acc = parts[0].clone()
+    for w in parts[1:]:
+        acc[:, :2] += w[:, :2]
+        hi, lo = dd_add(acc[:, 2::2], acc[:, 3::2], w[:, 2::2], w[:, 3::2])
+        acc[:, 2::2], acc[:, 3::2] = hi, lo
+    out.data.copy_(acc)
     return out
 
 
