@@ -274,19 +274,35 @@ def test_compaction_kernel_matches_numpy():
         assert np.array_equal(idx[: len(want)].cpu().numpy(), want)
 
 
-@pytest.mark.parametrize("pinned,n", [(False, 3000), (True, 3000), (True, 40_000)])
-def test_host_entry_point_matches_device_entry_point(pinned, n):
+HOST_ENTRY_CASES = [
+    pytest.param(False, 3000, None, id="False-3000"), pytest.param(True, 3000, None, id="True-3000"),
+    pytest.param(True, 40_000, None, id="True-40000")] + [
+    pytest.param(pinned, 3000, case, id="%s-3000-%s" % (pinned, case))
+    for case in ("tally", "monitor", "species", "launches") for pinned in (False, True)]
+
+
+@pytest.mark.parametrize("pinned,n,case", HOST_ENTRY_CASES)
+def test_host_entry_point_matches_device_entry_point(pinned, n, case):
     """xlb_track_host == Line.track on device tensors: pageable host buffers (copies inside),
     small pinned buffers (tracked in place through their device aliases, no copies) and pinned
     buffers above the in-place limit (copies again); apertures so that lost particles are written
-    back through the same path."""
+    back through the same path.  The extra cases add a loss tally, BeamMonitor storage, chi and
+    charge_ratio columns of two species, and launches of 3 turns (survivors re-compacted between
+    them)."""
     import xline_b200 as xl
     from xline_b200 import _cabi, configs
 
     line, cols, p0c, m0 = configs.config_fodo(n)
-    line = xl.Line(list(line.elements) + [xl.LimitEllipse(a=3.5e-3, b=3.5e-3)])
+    elements = list(line.elements) + [xl.LimitEllipse(a=3.5e-3, b=3.5e-3)]
+    if case == "monitor":
+        elements.append(xl.BeamMonitor(num_stores=3, start=1, skip=2, min_particle_id=100, max_particle_id=2099))
+    line = xl.Line(elements)
+    if case == "species":
+        other = np.random.default_rng(3).random(n) < 0.5
+        cols = dict(cols, charge_ratio=np.where(other, 2.0, 1.0), chi=np.where(other, 0.5, 1.0))
+    turns_per_launch = 3 if case == "launches" else 0
     p = make_particles(cols, p0c, m0)
-    line.track(p, num_turns=7)
+    line.track(p, num_turns=7, turns_per_launch=turns_per_launch)
     want = p.to_numpy()
     assert 0 < (want["state"] == 0).sum() < n
     hp = xl.Particles(p0c=p0c, mass0=m0, device="cpu", pinned=pinned, **cols)
@@ -301,10 +317,23 @@ def test_host_entry_point_matches_device_entry_point(pinned, n):
     cp.beta0, cp.gamma0, cp.energy0 = hp.beta0, hp.gamma0, hp.energy0
     opts = _cabi.TrackOptions()
     opts.num_turns = 7
+    opts.turns_per_launch = turns_per_launch
+    if case == "tally":
+        tally = torch.zeros(packed.n_elements, dtype=torch.int64, pin_memory=pinned)
+        opts.loss_tally = tally.data_ptr()
+    if case == "monitor":
+        mon = torch.full((packed.monitor_words,), float("nan"), dtype=torch.float64, pin_memory=pinned)
+        opts.monitor_data, opts.monitor_words = mon.data_ptr(), packed.monitor_words
     _cabi.check(_cabi.lib().xlb_track_host(C.byref(lat), C.byref(cp), C.byref(opts)))
     got = hp.to_numpy()
     for k in want:
         assert np.array_equal(want[k], got[k], equal_nan=True), k
+    if case == "tally":
+        assert int(tally.sum()) == (want["state"] == 0).sum()
+        assert np.array_equal(tally.numpy(), line.loss_tally[: packed.n_elements].cpu().numpy())
+    if case == "monitor":
+        assert np.isfinite(mon.numpy()).any()
+        assert np.array_equal(mon.numpy(), line._monitor_buf.cpu().numpy(), equal_nan=True)
 
 
 def test_monitor_records_like_oracle():

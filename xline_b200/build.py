@@ -32,8 +32,8 @@ UNITS = [
     ("track_fast_bf6", "track_fast.cu", ["-DXLB_BEAMFIELDS=2"]),       # + BeamBeam6D
     ("track_strict_bf", "track_strict.cu", ["-DXLB_BEAMFIELDS=2", "-fmad=false"]),
 ]
-HEADERS = ["track_impl.cuh", "kargs.h", "variants.inc", "beamfields.cuh", "faddeeva_coeffs.inc",
-           os.path.join("..", "..", "include", "xline_b200.h")]
+HEADERS = ["track_impl.cuh", "kargs.h", "launch_plan.h", "variants.inc", "beamfields.cuh",
+           "faddeeva_coeffs.inc", os.path.join("..", "..", "include", "xline_b200.h")]
 
 
 def _nvcc():

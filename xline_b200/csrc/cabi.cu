@@ -10,10 +10,12 @@
 #include <cmath>
 #include <mutex>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/xline_b200.h"
 #include "kargs.h"
+#include "launch_plan.h"
 
 namespace xlb {
 
@@ -145,13 +147,13 @@ struct Scratch {
   // host entry point arena
   unsigned char *arena = nullptr;
   size_t arena_bytes = 0;
-  cudaStream_t stream = nullptr;
+  cudaStream_t stream = nullptr;  // host entry point stream
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   // One call at a time per device: the queue, the survivor list, the counters and the pinned
   // read-back words above are shared by every xlb_track_* call on this GPU.  Host threads
   // serialise on `call_mu` (recursive: the host entry point calls the device one); work that a
   // previous call left running on ANOTHER stream is ordered before the next call's by `done`,
-  // recorded at the end of every call and waited for at the start of the next.
+  // recorded at the end of every call and waited for at the start of the next (CallScope).
   std::recursive_mutex call_mu;
   cudaEvent_t done = nullptr;
   bool have_done = false;
@@ -164,14 +166,6 @@ struct Scratch {
   size_t moments_cap = 0;     // doubles
 };
 
-// Launch length for a loss rate: lanes of lost particles idle until the next launch boundary,
-// on average rate * length / 2 of the lanes over a launch -- keep that near 3 %.
-static int launch_length_for_rate(double rate_per_turn, int longest) {
-  if (!(rate_per_turn > 0)) return longest;
-  const double len = 0.06 / rate_per_turn;
-  if (len >= longest) return longest;
-  return len < 1.0 ? 1 : static_cast<int>(len);
-}
 static std::mutex g_mu;
 static std::vector<Scratch *> g_scratch;
 
@@ -190,6 +184,7 @@ static int get_scratch(Scratch **out) {
   XLB_CUDA(cudaMalloc(&s->n_active, sizeof(int)));
   XLB_CUDA(cudaMemset(s->n_lost, 0, sizeof(unsigned int)));
   XLB_CUDA(cudaMallocHost(&s->h_pinned, 2 * sizeof(unsigned int)));
+  XLB_CUDA(cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking));
   XLB_CUDA(cudaEventCreate(&s->ev0));
   XLB_CUDA(cudaEventCreate(&s->ev1));
   XLB_CUDA(cudaEventCreateWithFlags(&s->done, cudaEventDisableTiming));
@@ -198,44 +193,53 @@ static int get_scratch(Scratch **out) {
   return XLB_OK;
 }
 
-static int ensure_queue(Scratch *s, size_t words) {
-  if (words > s->queue_cap) {
-    if (s->queue) cudaFree(s->queue);
-    s->queue = nullptr;
-    s->queue_cap = 0;
-    XLB_CUDA(cudaMalloc(&s->queue, words * sizeof(unsigned int)));
-    s->queue_cap = words;
+namespace {
+// The scope of one call on the current device: holds its Scratch's `call_mu`, makes `st` wait for
+// what the previous call enqueued and, whatever way the call ends, records `done` on `st` so that
+// the next call waits for what this one enqueued.
+class CallScope {
+ public:
+  Scratch *s = nullptr;
+  int open(cudaStream_t st) {
+    int rc;
+    if ((rc = get_scratch(&s)) != XLB_OK) return rc;
+    lock_ = std::unique_lock<std::recursive_mutex>(s->call_mu);
+    st_ = st;
+    if (s->have_done) XLB_CUDA(cudaStreamWaitEvent(st, s->done, 0));
+    return XLB_OK;
   }
+  ~CallScope() {
+    if (lock_.owns_lock() && cudaEventRecord(s->done, st_) == cudaSuccess) s->have_done = true;
+  }
+
+ private:
+  std::unique_lock<std::recursive_mutex> lock_;
+  cudaStream_t st_ = nullptr;
+};
+}  // namespace
+
+// Grows the device buffer `*buf` to at least `count` elements; what it held is not kept.
+template <typename T, typename N>
+static int grow(T **buf, N *cap, N count) {
+  if (count <= *cap) return XLB_OK;
+  if (*buf) cudaFree(*buf);
+  *buf = nullptr;
+  *cap = 0;
+  XLB_CUDA(cudaMalloc(buf, static_cast<size_t>(count) * sizeof(T)));
+  *cap = count;
   return XLB_OK;
 }
 
-static int ensure_compaction_scratch(Scratch *s, long long n) {
-  const int nblocks = static_cast<int>((n + CP_THREADS * CP_ITEMS - 1) / (CP_THREADS * CP_ITEMS));
-  if (n > s->cap) {
-    if (s->idx) cudaFree(s->idx);
-    s->idx = nullptr;
-    XLB_CUDA(cudaMalloc(&s->idx, static_cast<size_t>(n) * sizeof(int)));
-    s->cap = n;
-  }
-  if (nblocks > s->nblocks_cap) {
-    if (s->block_sums) cudaFree(s->block_sums);
-    s->block_sums = nullptr;
-    XLB_CUDA(cudaMalloc(&s->block_sums, static_cast<size_t>(nblocks) * sizeof(int)));
-    s->nblocks_cap = nblocks;
-  }
-  return XLB_OK;
+// The address of a pointer field, as the slot a device pointer is written to.
+template <typename T>
+static void **slot(T **field) {
+  return reinterpret_cast<void **>(const_cast<std::remove_const_t<T> **>(field));
 }
 
 // One beam-moment store of slots 0..n-1 into out[0..XLB_MOMENT_WORDS), enqueued on `st`.
 static int beam_moments(Scratch *s, const xlb_particles_t *p, double *out, cudaStream_t st) {
-  const size_t words = beam_moments_scratch_words(p->n);
-  if (words > s->moments_cap) {
-    if (s->moments) cudaFree(s->moments);
-    s->moments = nullptr;
-    s->moments_cap = 0;
-    XLB_CUDA(cudaMalloc(&s->moments, words * sizeof(double)));
-    s->moments_cap = words;
-  }
+  int rc;
+  if ((rc = grow(&s->moments, &s->moments_cap, beam_moments_scratch_words(p->n))) != XLB_OK) return rc;
   XLB_CUDA(beam_moments_launch(p->x, p->px, p->y, p->py, p->zeta, p->delta,
                                reinterpret_cast<const long long *>(p->state), p->n, s->moments, out, st));
   return XLB_OK;
@@ -246,12 +250,7 @@ struct MomentStores {
   xlb_moments_spec_t spec;
   double *out;
   long long k = 0;  // next store
-  // turn of the next store, or past num_turns when none is left
-  long long next_turn(long long num_turns) const {
-    if (k >= spec.num_stores || spec.start > num_turns) return num_turns + 1;
-    if (k > 0 && spec.skip > (num_turns - spec.start) / k) return num_turns + 1;
-    return spec.start + k * spec.skip;
-  }
+  long long next_turn(long long num_turns) const { return moment_store_turn(spec, k, num_turns); }
   // takes every store due after `done` turns (t_k <= done <= num_turns)
   int take(Scratch *s, const xlb_particles_t *p, long long done, long long num_turns, cudaStream_t st) {
     int rc;
@@ -263,17 +262,32 @@ struct MomentStores {
   }
 };
 
-static int compact_alive(const long long *state, long long n, int *idx_out, int *block_sums,
-                         int *n_out, cudaStream_t st) {
+// Survivor list of slots 0..n-1 into idx_out and its length into *n_out, enqueued on `st`.
+static int compact_alive(Scratch *s, const long long *state, long long n, int *idx_out, int *n_out,
+                         cudaStream_t st) {
   if (n <= 0) {
     XLB_CUDA(cudaMemsetAsync(n_out, 0, sizeof(int), st));
     return XLB_OK;
   }
   const int nblocks = static_cast<int>((n + CP_THREADS * CP_ITEMS - 1) / (CP_THREADS * CP_ITEMS));
-  compact_count<<<nblocks, CP_THREADS, 0, st>>>(state, n, block_sums);
-  compact_scan<<<1, 1024, 0, st>>>(block_sums, nblocks, n_out);
-  compact_scatter<<<nblocks, CP_THREADS, 0, st>>>(state, n, block_sums, idx_out);
+  int rc;
+  if ((rc = grow(&s->block_sums, &s->nblocks_cap, nblocks)) != XLB_OK) return rc;
+  compact_count<<<nblocks, CP_THREADS, 0, st>>>(state, n, s->block_sums);
+  compact_scan<<<1, 1024, 0, st>>>(s->block_sums, nblocks, n_out);
+  compact_scatter<<<nblocks, CP_THREADS, 0, st>>>(state, n, s->block_sums, idx_out);
   XLB_CUDA(cudaGetLastError());
+  return XLB_OK;
+}
+
+// Re-compacts the survivors of slots 0..n-1 into s->idx and waits for their number.
+static int recompact(Scratch *s, const long long *state, long long n, cudaStream_t st, long long *n_alive) {
+  int rc;
+  if ((rc = grow(&s->idx, &s->cap, n)) != XLB_OK) return rc;
+  if ((rc = compact_alive(s, state, n, s->idx, s->n_active, st)) != XLB_OK) return rc;
+  XLB_CUDA(cudaMemcpyAsync(&s->h_pinned[1], s->n_active, sizeof(int), cudaMemcpyDeviceToHost, st));
+  XLB_CUDA(cudaStreamSynchronize(st));
+  g_stats.compactions += 1;
+  *n_alive = static_cast<int>(s->h_pinned[1]);
   return XLB_OK;
 }
 
@@ -333,6 +347,40 @@ static const Variant *pick_variant(const Need &q, int ppt, int threads) {
   return fallback;
 }
 
+// A variant, its CTA size, the CTAs the device holds at once and its registers per thread.
+struct Shape {
+  const Variant *v;
+  int threads, resident, regs;
+};
+// The shape of a launch over the `n_now` particles still in the beam: a small (or scraped-down)
+// beam is spread over all SMs first -- fewer particles per thread as long as the CTAs of the
+// preferred shape would leave CTA slots empty (strong scaling, C1, the heavy-loss C2 beam).  All
+// variants give the same bits, so the choice is invisible in the results.
+static int choose(const Need &q, const xlb_track_options_t &o, int sms, size_t smem, long long n_now,
+                  Shape *out) {
+  const LaunchRequest r =
+      launch_request(o.particles_per_thread, o.threads_per_block, q.strict, q.beamfields, q.chi, n_now, sms);
+  const Variant *v = pick_variant(q, r.ppt, r.threads);
+  if (!v) return fail(XLB_EINVAL, "no kernel variant compiled for this lattice");
+  const int threads =
+      q.trace ? v->threads : (o.threads_per_block > 0 ? o.threads_per_block : std::min(v->threads, r.threads));
+  if (threads % 32 || threads > v->threads)
+    return fail(XLB_EINVAL, "threads_per_block must be a multiple of 32 and <= the variant's limit");
+  XLB_CUDA(cudaFuncSetAttribute(v->func, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+  cudaFuncAttributes fa;
+  XLB_CUDA(cudaFuncGetAttributes(&fa, v->func));
+  int occ = 1;
+  XLB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, v->func, threads, smem));
+  *out = {v, threads, std::max(1, occ) * sms, fa.numRegs};
+  return XLB_OK;
+}
+
+static int launch(const Variant &v, const KArgs &a, int grid, int threads, size_t smem, cudaStream_t st) {
+  void *args[] = {const_cast<KArgs *>(&a)};
+  XLB_CUDA(cudaLaunchKernel(v.func, dim3(grid), dim3(threads), args, smem, st));
+  return XLB_OK;
+}
+
 static int check_lattice_header(const xlb_lattice_t *lat) {
   if (!lat || !lat->words) return fail(XLB_EINVAL, "lattice is null");
   if (lat->chunk_words < 4 || (lat->chunk_words & 1))
@@ -376,121 +424,33 @@ static int check_particles(const xlb_particles_t *p) {
   return XLB_OK;
 }
 
-// `stores` (optional): beam-moment stores taken on the stream after the launch that ends on their
-// turn; launches are cut at the store turns.
-static int track_device_impl(const xlb_lattice_t *lat, xlb_particles_t *p,
-                             const xlb_track_options_t *o, cudaStream_t st, bool timed,
-                             MomentStores *stores = nullptr) {
-  memset(&g_stats, 0, sizeof(g_stats));
+// The arguments of a tracking call; a call without particles or turns has nothing more to check.
+static int check_call(const xlb_lattice_t *lat, const xlb_particles_t *p, const xlb_track_options_t *o,
+                      const MomentStores *stores) {
   int rc;
   if ((rc = check_lattice_header(lat)) != XLB_OK) return rc;
   if ((rc = check_particles(p)) != XLB_OK) return rc;
   if (!o) return fail(XLB_EINVAL, "options is null");
   if (o->num_turns < 0) return fail(XLB_EINVAL, "num_turns < 0");
   if (stores && o->trace) return fail(XLB_EINVAL, "beam-moment stores do not combine with a trace");
-  if (p->n == 0 || o->num_turns == 0) {
-    if (!stores) return XLB_OK;
-    Scratch *s = nullptr;
-    if ((rc = get_scratch(&s)) != XLB_OK) return rc;
-    std::lock_guard<std::recursive_mutex> call_lock(s->call_mu);
-    if (s->have_done) XLB_CUDA(cudaStreamWaitEvent(st, s->done, 0));
-    rc = stores->take(s, p, o->num_turns, o->num_turns, st);
-    if (cudaEventRecord(s->done, st) == cudaSuccess) s->have_done = true;
-    return rc;
-  }
-
-  const bool strict = (lat->flags & XLB_F_STRICT) != 0;
-  const bool beamfields = (lat->flags & XLB_F_BEAMFIELDS) != 0;
-  const bool split = lat->n_segments > 1;  // 6D lenses run as kernels of their own
-  const bool bb6d = (lat->flags & XLB_F_BB6D) != 0 && !split;
-  // Defaults from the B200 sweeps (scripts/probe_variants.py, scripts/probe_strict.py).  Thin-lens
-  // lattices of one species (chi == NULL): 4 particles per thread in 128-thread CTAs, 3 CTAs/SM at
-  // 168 registers = 1 536 particles in flight per SM (C2 +5 %, C4 +23 % over 3 x 128 x 3); with a
-  // chi column 3 x 128 (162 registers, no spills).  Strict C2: 1.08e7 particle-turns/s with 3 x 128
-  // against 9.1e6 (2 x 128), 7.3e6 (1 x 256), 6.7e6 (2 x 256).  Beam-field lattices: 2 x 256 unless
-  // the caller knows the lenses are sparse (xline_b200/line.py decides from the record counts).
-  Need need;
-  need.strict = strict;
-  need.beamfields = beamfields;
-  need.bb6d = bb6d;
-  need.chi = p->chi != nullptr;
-  need.trace = o->trace != nullptr;
-  need.polygons = (lat->flags & XLB_F_POLYGONS) != 0;
-  need.max_order = (lat->flags & XLB_F_LOW_ORDER) ? 3 : 255;
-  const bool trace = need.trace;
-  if (trace && (o->num_turns != 1 || o->trace_particles < 1))
+  if (p->n == 0 || o->num_turns == 0) return XLB_OK;
+  if (o->trace && (o->num_turns != 1 || o->trace_particles < 1))
     return fail(XLB_EINVAL, "element-by-element trace needs num_turns == 1 and trace_particles >= 1");
-  if (split && (trace || strict))
+  if (lat->n_segments > 1 && (o->trace || (lat->flags & XLB_F_STRICT)))
     return fail(XLB_EINVAL, "segmented lattices are for the fast kernels without trace");
-  int dev = 0, sms = 0;
-  XLB_CUDA(cudaGetDevice(&dev));
-  XLB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  const size_t chunk_bytes = static_cast<size_t>(lat->chunk_words) * 8;
-  const size_t smem = XLB_STAGES * chunk_bytes + (2 * XLB_STAGES + 2) * sizeof(unsigned long long);
-  // The launch shape is chosen per launch from the number of particles still in the beam: a small
-  // (or scraped-down) beam is spread over all SMs first -- fewer particles per thread as long as
-  // the CTAs of the preferred shape would leave CTA slots empty (strong scaling, C1, the heavy-loss
-  // C2 beam).  All variants give the same bits, so the choice is invisible in the results.
-  struct Shape {
-    const Variant *v;
-    int threads, resident, regs;
-  };
-  auto choose = [&](long long n_now, Shape *out) -> int {
-    int ppt_req = o->particles_per_thread;
-    if (ppt_req <= 0) {
-      if (beamfields) ppt_req = 2;
-      else if (strict || need.chi) ppt_req = 3;
-      else ppt_req = 4;
-      if (!beamfields && o->threads_per_block <= 0) {
-        // (below 2 only for beams that cannot give every SM one 128-thread CTA: one particle per
-        // thread doubles the warps but also the per-record instructions issued, and loses on the
-        // C2 lattice from 30 000 particles on -- profiles/r2_sweep_n.json; C1's 10 000 particles
-        // on 79 CTAs instead of 40: 3.3e9 against 2.3e9 particle-turns/s)
-        // (three per thread wins nowhere in the closing sweep, profiles/r2c_sweep_n.json: 200 k
-        // particles 2.45e7 with two, 2.38e7 with three, 2.11e7 with four)
-        if (ppt_req > 2 && n_now < static_cast<long long>(ppt_req) * 128 * 3 * sms) ppt_req = 2;
-        if (ppt_req == 2 && n_now < 128LL * sms) ppt_req = 1;
-      }
-    }
-    const int threads_req =
-        o->threads_per_block > 0 ? o->threads_per_block : (beamfields && ppt_req < 3 ? 256 : 128);
-    const Variant *v = pick_variant(need, ppt_req, threads_req);
-    if (!v) return fail(XLB_EINVAL, "no kernel variant compiled for this lattice");
-    const int threads =
-        trace ? v->threads : (o->threads_per_block > 0 ? o->threads_per_block : std::min(v->threads, threads_req));
-    if (threads % 32 || threads > v->threads)
-      return fail(XLB_EINVAL, "threads_per_block must be a multiple of 32 and <= the variant's limit");
-    XLB_CUDA(cudaFuncSetAttribute(v->func, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    cudaFuncAttributes fa;
-    XLB_CUDA(cudaFuncGetAttributes(&fa, v->func));
-    int occ = 1;
-    XLB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, v->func, threads, smem));
-    out->v = v;
-    out->threads = threads;
-    out->resident = std::max(1, occ) * sms;  // CTAs the device holds at once
-    out->regs = fa.numRegs;
-    return XLB_OK;
-  };
-  Shape shape;
-  if ((rc = choose(p->n, &shape)) != XLB_OK) return rc;  // also validates the caller's request
+  return XLB_OK;
+}
 
-  Scratch *s = nullptr;
-  if ((rc = get_scratch(&s)) != XLB_OK) return rc;
-  std::lock_guard<std::recursive_mutex> call_lock(s->call_mu);
-  if (s->have_done) XLB_CUDA(cudaStreamWaitEvent(st, s->done, 0));
-  struct DoneMark {  // whatever way the call ends, later calls wait for what it enqueued
-    Scratch *s;
-    cudaStream_t st;
-    ~DoneMark() {
-      if (cudaEventRecord(s->done, st) == cudaSuccess) s->have_done = true;
-    }
-  } done_mark{s, st};
-
+// The kernel arguments of a call, over all its particles (a launch over the survivors sets a.n and
+// a.idx).
+static KArgs kernel_args(const xlb_lattice_t *lat, const xlb_particles_t *p, const xlb_track_options_t *o,
+                         unsigned int *n_lost) {
   KArgs a;
   memset(&a, 0, sizeof(a));
   a.lat = lat->words;
   a.chunk_words = lat->chunk_words;
   a.n_chunks = lat->n_chunks;
+  a.n = p->n;
   a.x = p->x; a.px = p->px; a.y = p->y; a.py = p->py; a.zeta = p->zeta; a.delta = p->delta;
   a.rpp = p->rpp; a.rvv = p->rvv; a.s = p->s; a.chi = p->chi; a.qr = p->charge_ratio;
   a.state = reinterpret_cast<long long *>(p->state);
@@ -502,12 +462,106 @@ static int track_device_impl(const xlb_lattice_t *lat, xlb_particles_t *p,
   a.loss_tally = reinterpret_cast<long long *>(o->loss_tally);
   a.mon = o->monitor_data;
   a.mon_words = o->monitor_words;
-  a.n_lost = s->n_lost;
+  a.n_lost = n_lost;
   a.trace = o->trace;
   a.trace_n = o->trace_particles;
   a.elem_off = static_cast<int>(o->element_index_offset);
-  const int count_turns = (o->flags & XLB_OPT_NO_TURN_COUNT) ? 0 : 1;
+  a.count_turns = (o->flags & XLB_OPT_NO_TURN_COUNT) ? 0 : 1;
+  return a;
+}
 
+// Enqueues `turns` turns of the a.n particles (survivor list a.idx) in the shape `sh`, and sets
+// the launch stats.  `tpi`: turns per work item of the persistent queue, <= 0 = no queue.
+static int enqueue_turns(const xlb_lattice_t *lat, KArgs a, const Shape &sh, int turns, int tpi, size_t smem,
+                         int sms, Scratch *s, cudaStream_t st) {
+  const long long per_block = static_cast<long long>(sh.threads) * sh.v->ppt;
+  const int blocks = static_cast<int>((a.n + per_block - 1) / per_block);
+  g_stats.blocks = blocks;
+  g_stats.threads = sh.threads;
+  a.num_turns = turns;
+  a.queue = nullptr;
+  a.n_blocks = static_cast<unsigned int>(blocks);
+  a.n_items = static_cast<unsigned int>(blocks);
+  a.turns_per_item = turns;
+  if (lat->n_segments > 1) {
+    // turn by turn, segment by segment: tracking kernel up to the next 6D lens, the lens
+    // kernel, and so on; the closing MAIN segment counts the turn
+    const int count_turns = a.count_turns;
+    a.num_turns = 1;
+    a.turns_per_item = 1;
+    const int lens_threads = 128;
+    const int lens_blocks = static_cast<int>((a.n + lens_threads - 1) / lens_threads);
+    int rc;
+    for (int t = 0; t < turns; ++t) {
+      for (int k = 0; k < lat->n_segments; ++k) {
+        const int32_t *sg = lat->segments + 3 * k;
+        const uint64_t *first = lat->words + static_cast<size_t>(sg[0]) * lat->chunk_words;
+        if (sg[2] == XLB_SEG_BB6D) {
+          fast_bb6d_launch(a, reinterpret_cast<const unsigned long long *>(first), lens_blocks, lens_threads, st);
+        } else {
+          a.lat = first;
+          a.n_chunks = sg[1];
+          a.count_turns = (k == lat->n_segments - 1) ? count_turns : 0;
+          if ((rc = launch(*sh.v, a, blocks, sh.threads, smem, st)) != XLB_OK) return rc;
+        }
+        g_stats.kernel_launches += 1;
+      }
+    }
+    XLB_CUDA(cudaGetLastError());
+    return XLB_OK;
+  }
+  int grid = blocks;
+  if (tpi > 0 && turns > tpi && blocks > sms) {
+    // persistent CTAs + a device-side ring of ready (block, turn segment) items (track_impl.cuh).
+    // Also when every CTA could be resident at once (sms < blocks <= resident): SMs would hold
+    // different numbers of CTAs, a CTA on a fuller SM runs slower, and with one item per CTA
+    // the launch lasts as long as its slowest CTA.
+    const long long segs = (turns + tpi - 1) / tpi;
+    if (static_cast<long long>(blocks) * segs < (1LL << 26)) {  // ring of at most 512 MiB
+      // two counters + one 64-bit ready entry per item beyond the first segment of every block
+      const size_t qwords = 2 + 2 * static_cast<size_t>(blocks) * static_cast<size_t>(segs - 1);
+      int rc;
+      if ((rc = grow(&s->queue, &s->queue_cap, qwords)) != XLB_OK) return rc;
+      XLB_CUDA(cudaMemsetAsync(s->queue, 0, qwords * sizeof(unsigned int), st));
+      a.queue = s->queue;
+      a.n_items = static_cast<unsigned int>(blocks * segs);
+      a.turns_per_item = tpi;
+      grid = persistent_grid(blocks, sh.resident, sms);
+    }
+  }
+  g_stats.kernel_launches += 1;
+  return launch(*sh.v, a, grid, sh.threads, smem, st);
+}
+
+// `stores` (optional): beam-moment stores taken on the stream after the launch that ends on their
+// turn; launches are cut at the store turns.
+static int track_device_impl(const xlb_lattice_t *lat, xlb_particles_t *p,
+                             const xlb_track_options_t *o, cudaStream_t st, bool timed,
+                             MomentStores *stores = nullptr) {
+  memset(&g_stats, 0, sizeof(g_stats));
+  int rc;
+  if ((rc = check_call(lat, p, o, stores)) != XLB_OK) return rc;
+  const bool empty = p->n == 0 || o->num_turns == 0;
+  if (empty && !stores) return XLB_OK;
+  const bool split = lat->n_segments > 1;  // 6D lenses run as kernels of their own
+  const Need need{(lat->flags & XLB_F_STRICT) != 0, (lat->flags & XLB_F_BEAMFIELDS) != 0,
+                  (lat->flags & XLB_F_BB6D) != 0 && !split, p->chi != nullptr, o->trace != nullptr,
+                  (lat->flags & XLB_F_POLYGONS) != 0, (lat->flags & XLB_F_LOW_ORDER) ? 3 : 255};
+  const size_t smem = XLB_STAGES * static_cast<size_t>(lat->chunk_words) * 8 +
+                      (2 * XLB_STAGES + 2) * sizeof(unsigned long long);
+  int dev = 0, sms = 0;
+  Shape shape{};
+  if (!empty) {
+    XLB_CUDA(cudaGetDevice(&dev));
+    XLB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    if ((rc = choose(need, *o, sms, smem, p->n, &shape)) != XLB_OK) return rc;  // validates the caller's shape
+  }
+  CallScope call;
+  if ((rc = call.open(st)) != XLB_OK) return rc;
+  Scratch *s = call.s;
+  if (empty) return stores->take(s, p, o->num_turns, o->num_turns, st);
+
+  KArgs a = kernel_args(lat, p, o, s->n_lost);
   // Work-item length.  An item costs a load and a store of its block's particles and a ticket
   // (microseconds); a shorter item leaves a shorter tail at the end of a launch (the last, partly
   // filled round of items) and rotates the blocks faster.  Automatic: one turn when a turn streams
@@ -515,15 +569,9 @@ static int track_device_impl(const xlb_lattice_t *lat, xlb_particles_t *p,
   // as many turns as make 16 chunks (PS Booster: 6).
   const int tpi = (o->turns_per_item == 0) ? std::max(1, (16 + lat->n_chunks - 1) / lat->n_chunks)
                                            : o->turns_per_item;
-  // 0 = automatic: long jobs are cut into launches of 100 turns so that survivors get
-  // re-compacted now and then; < 0 = one launch whatever the length
-  // (the kernel counts the chunks of a launch in 32 bits: a launch never exceeds 2^31 / n_chunks turns)
-  const int seg_cap = std::max(1, static_cast<int>(0x7fffffffLL / std::max(1, lat->n_chunks)));
-  const int seg = std::min(seg_cap, (o->turns_per_launch > 0) ? o->turns_per_launch
-                  : (o->turns_per_launch == 0 && o->num_turns > 150 ? 100 : o->num_turns));
+  const int seg = launch_cap(o->turns_per_launch, o->num_turns, lat->n_chunks);
   const double thr = (o->compact_threshold > 0) ? o->compact_threshold : (1.0 / 128.0);
   long long n_active = p->n;
-  const int *idx = nullptr;
   long long lost_since_compact = 0;
   const bool segmented = seg < o->num_turns;
   if (segmented || stores) XLB_CUDA(cudaMemsetAsync(s->n_lost, 0, sizeof(unsigned int), st));
@@ -543,126 +591,47 @@ static int track_device_impl(const xlb_lattice_t *lat, xlb_particles_t *p,
   double last_rate = -1.0;
 
   if (timed) XLB_CUDA(cudaEventRecord(s->ev0, st));
-  if (o->turns_per_launch > 0 || seg < o->num_turns) {
+  if (o->turns_per_launch > 0 || segmented) {
     // particles lost in earlier calls still sit in the caller's arrays (state 0): start from
     // the compacted survivor list so they do not occupy lanes
-    if ((rc = ensure_compaction_scratch(s, p->n)) != XLB_OK) return rc;
-    if ((rc = compact_alive(a.state, p->n, s->idx, s->block_sums, s->n_active, st)) != XLB_OK)
-      return rc;
-    XLB_CUDA(cudaMemcpyAsync(&s->h_pinned[1], s->n_active, sizeof(int), cudaMemcpyDeviceToHost, st));
-    XLB_CUDA(cudaStreamSynchronize(st));
-    g_stats.compactions += 1;
-    if (static_cast<long long>(s->h_pinned[1]) < p->n) {
-      n_active = static_cast<int>(s->h_pinned[1]);
-      idx = s->idx;
+    long long alive = 0;
+    if ((rc = recompact(s, a.state, p->n, st, &alive)) != XLB_OK) return rc;
+    if (alive < p->n) {
+      a.n = n_active = alive;
+      a.idx = s->idx;
     }
   }
-  float total_ms = 0.f;
   long long lost_before_launch = 0;
   if (stores && (rc = stores->take(s, p, 0, o->num_turns, st)) != XLB_OK) return rc;
   for (int done = 0; done < o->num_turns && n_active > 0;) {
     int turns = std::min(ramp ? cur_len : seg, o->num_turns - done);
     if (stores) turns = static_cast<int>(std::min<long long>(turns, stores->next_turn(o->num_turns) - done));
-    a.num_turns = turns;
-    a.n = n_active;
-    a.idx = idx;
-    if ((rc = choose(n_active, &shape)) != XLB_OK) return rc;
-    const Variant *v = shape.v;
-    const int threads = shape.threads, resident = shape.resident;
-    const long long per_block = static_cast<long long>(threads) * v->ppt;
-    const int blocks = static_cast<int>((n_active + per_block - 1) / per_block);
-    int grid = blocks;
-    a.queue = nullptr;
-    a.n_blocks = static_cast<unsigned int>(blocks);
-    a.n_items = static_cast<unsigned int>(blocks);
-    a.turns_per_item = turns;
-    a.count_turns = count_turns;
-    if (split) {
-      // turn by turn, segment by segment: tracking kernel up to the next 6D lens, the lens
-      // kernel, and so on; the closing MAIN segment counts the turn
-      a.num_turns = 1;
-      a.turns_per_item = 1;
-      const int lens_threads = 128;
-      const int lens_blocks = static_cast<int>((n_active + lens_threads - 1) / lens_threads);
-      for (int t = 0; t < turns; ++t) {
-        for (int k = 0; k < lat->n_segments; ++k) {
-          const int32_t *sg = lat->segments + 3 * k;
-          const uint64_t *first = lat->words + static_cast<size_t>(sg[0]) * lat->chunk_words;
-          if (sg[2] == XLB_SEG_BB6D) {
-            fast_bb6d_launch(a, reinterpret_cast<const unsigned long long *>(first), lens_blocks,
-                             lens_threads, st);
-          } else {
-            a.lat = first;
-            a.n_chunks = sg[1];
-            a.count_turns = (k == lat->n_segments - 1) ? count_turns : 0;
-            v->launch(a, blocks, threads, smem, st);
-          }
-          g_stats.kernel_launches += 1;
-        }
-      }
-      XLB_CUDA(cudaGetLastError());
-      g_stats.blocks = blocks;
-      g_stats.threads = threads;
-    } else {
-    if (tpi > 0 && turns > tpi && blocks > sms) {
-      // persistent CTAs + a device-side ring of ready (block, turn segment) items (track_impl.cuh).
-      // Also when every CTA could be resident at once (sms < blocks <= resident): SMs would hold
-      // different numbers of CTAs, a CTA on a fuller SM runs slower, and with one item per CTA
-      // the launch lasts as long as its slowest CTA.
-      const long long segs = (turns + tpi - 1) / tpi;
-      if (static_cast<long long>(blocks) * segs < (1LL << 26)) {  // ring of at most 512 MiB
-        // two counters + one 64-bit ready entry per item beyond the first segment of every block
-        const size_t qwords = 2 + 2 * static_cast<size_t>(blocks) * static_cast<size_t>(segs - 1);
-        if ((rc = ensure_queue(s, qwords)) != XLB_OK) return rc;
-        XLB_CUDA(cudaMemsetAsync(s->queue, 0, qwords * sizeof(unsigned int), st));
-        a.queue = s->queue;
-        a.n_items = static_cast<unsigned int>(blocks * segs);
-        a.turns_per_item = tpi;
-        // Fewer CTAs than blocks (unless the blocks load every SM equally): the blocks beyond the
-        // grid wait in the ring, whose FIFO
-        // order then rotates the blocks over the CTAs, and all of them advance at the average speed.  (With every block resident on a CTA of its own a finishing CTA finds only its
-        // own block in the ring -- a static assignment, as slow as the CTAs of the fullest SMs:
-        // C2 at 125 k particles 1.9e7 against 2.2e7.)  Preferably the same number of CTAs on every
-        // SM; when that would idle more than 15 % of the CTAs, a backlog of 1/16 of the blocks.
-        const int q = std::min(blocks, resident), rem = q % sms;
-        grid = (rem * 100 <= q * 15) ? q - rem : q - std::max(1, q / 16);
-      }
-    }
-    v->launch(a, grid, threads, smem, st);
-    XLB_CUDA(cudaGetLastError());
-    g_stats.kernel_launches += 1;
-    g_stats.blocks = blocks;
-    g_stats.threads = threads;
-    }
+    if ((rc = choose(need, *o, sms, smem, n_active, &shape)) != XLB_OK) return rc;
+    if ((rc = enqueue_turns(lat, a, shape, turns, tpi, smem, sms, s, st)) != XLB_OK) return rc;
     done += turns;
     if (stores && (rc = stores->take(s, p, done, o->num_turns, st)) != XLB_OK) return rc;
     if (done >= o->num_turns) break;
     // survivors: read the loss counter; re-compact when enough lanes went idle
-    XLB_CUDA(cudaMemcpyAsync(&s->h_pinned[0], s->n_lost, sizeof(unsigned int),
-                             cudaMemcpyDeviceToHost, st));
+    XLB_CUDA(cudaMemcpyAsync(&s->h_pinned[0], s->n_lost, sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
     XLB_CUDA(cudaStreamSynchronize(st));
     const long long lost_total = s->h_pinned[0];
     if (ramp) {
       last_rate = static_cast<double>(lost_total - lost_before_launch) /
                   (static_cast<double>(n_active) * static_cast<double>(turns));
-      cur_len = std::min(launch_length_for_rate(last_rate, seg), 2 * cur_len);
+      cur_len = ramp_step(last_rate, seg, cur_len);
     }
     lost_before_launch = lost_total;
     const long long newly = lost_total - lost_since_compact;
     if (newly > 0 && static_cast<double>(newly) >= thr * static_cast<double>(n_active)) {
-      if ((rc = ensure_compaction_scratch(s, p->n)) != XLB_OK) return rc;
-      if ((rc = compact_alive(a.state, p->n, s->idx, s->block_sums, s->n_active, st)) != XLB_OK)
-        return rc;
-      XLB_CUDA(cudaMemcpyAsync(&s->h_pinned[1], s->n_active, sizeof(int), cudaMemcpyDeviceToHost, st));
-      XLB_CUDA(cudaStreamSynchronize(st));
-      n_active = static_cast<int>(s->h_pinned[1]);
-      idx = s->idx;
+      if ((rc = recompact(s, a.state, p->n, st, &n_active)) != XLB_OK) return rc;
+      a.n = n_active;
+      a.idx = s->idx;
       lost_since_compact = lost_total;
-      g_stats.compactions += 1;
     }
   }
   // a beam lost entirely before num_turns: the remaining stores see it empty
   if (stores && (rc = stores->take(s, p, o->num_turns, o->num_turns, st)) != XLB_OK) return rc;
+  float total_ms = 0.f;
   if (timed) {
     XLB_CUDA(cudaEventRecord(s->ev1, st));
     XLB_CUDA(cudaEventSynchronize(s->ev1));
@@ -909,42 +878,19 @@ int xlb_beam_moments_device(const xlb_particles_t *particles, double *out, void 
   int rc;
   if ((rc = check_particles(particles)) != XLB_OK) return rc;
   if (!out) return fail(XLB_EINVAL, "out is null");
-  Scratch *s = nullptr;
-  if ((rc = get_scratch(&s)) != XLB_OK) return rc;
-  std::lock_guard<std::recursive_mutex> call_lock(s->call_mu);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (s->have_done) XLB_CUDA(cudaStreamWaitEvent(st, s->done, 0));
-  rc = beam_moments(s, particles, out, st);
-  if (cudaEventRecord(s->done, st) == cudaSuccess) s->have_done = true;
-  return rc;
+  CallScope call;
+  if ((rc = call.open(static_cast<cudaStream_t>(stream))) != XLB_OK) return rc;
+  return beam_moments(call.s, particles, out, static_cast<cudaStream_t>(stream));
 }
 
 int xlb_compact_alive_device(const int64_t *state, int64_t n, int32_t *idx_out, int32_t *n_out,
                              void *stream) {
   if (n < 0 || (n > 0 && (!state || !idx_out)) || !n_out) return fail(XLB_EINVAL, "bad argument");
   if (n > 2147483647LL) return fail(XLB_EINVAL, "n too large");
-  Scratch *s = nullptr;
-  int rc = get_scratch(&s);
-  if (rc != XLB_OK) return rc;
-  std::lock_guard<std::recursive_mutex> call_lock(s->call_mu);
-  cudaStream_t cst = static_cast<cudaStream_t>(stream);
-  if (s->have_done) XLB_CUDA(cudaStreamWaitEvent(cst, s->done, 0));
-  struct DoneMark {
-    Scratch *s;
-    cudaStream_t st;
-    ~DoneMark() {
-      if (cudaEventRecord(s->done, st) == cudaSuccess) s->have_done = true;
-    }
-  } done_mark{s, cst};
-  if ((rc = ensure_compaction_scratch(s, 1)) != XLB_OK) return rc;
-  const int nblocks = static_cast<int>((n + CP_THREADS * CP_ITEMS - 1) / (CP_THREADS * CP_ITEMS));
-  if (nblocks > s->nblocks_cap) {
-    if (s->block_sums) cudaFree(s->block_sums);
-    s->block_sums = nullptr;
-    XLB_CUDA(cudaMalloc(&s->block_sums, static_cast<size_t>(nblocks) * sizeof(int)));
-    s->nblocks_cap = nblocks;
-  }
-  return compact_alive(reinterpret_cast<const long long *>(state), n, idx_out, s->block_sums, n_out,
+  CallScope call;
+  int rc;
+  if ((rc = call.open(static_cast<cudaStream_t>(stream))) != XLB_OK) return rc;
+  return compact_alive(call.s, reinterpret_cast<const long long *>(state), n, idx_out, n_out,
                        static_cast<cudaStream_t>(stream));
 }
 
@@ -959,35 +905,12 @@ int xlb_track_host(const xlb_lattice_t *hl, xlb_particles_t *hp, const xlb_track
   if (n == 0 || o->num_turns == 0) return XLB_OK;
   Scratch *s = nullptr;
   if ((rc = get_scratch(&s)) != XLB_OK) return rc;
-  std::lock_guard<std::recursive_mutex> call_lock(s->call_mu);
-  if (!s->stream) XLB_CUDA(cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking));
-  cudaStream_t st = s->stream;
+  const cudaStream_t st = s->stream;
+  CallScope call;
+  if ((rc = call.open(st)) != XLB_OK) return rc;
 
-  // device arena: lattice | 11 fp64 columns | 4 int64 columns | tally | monitor
-  auto al = [](size_t v) { return (v + 255) & ~static_cast<size_t>(255); };
-  const size_t col = al(static_cast<size_t>(n) * 8);
-  const size_t lat_bytes = al(static_cast<size_t>(hl->n_words) * 8);
-  const size_t tally_bytes = o->loss_tally ? al(static_cast<size_t>(hl->n_elements) * 8) : 0;
-  const size_t mon_bytes = o->monitor_data ? al(static_cast<size_t>(o->monitor_words) * 8) : 0;
-  const size_t need = lat_bytes + 15 * col + tally_bytes + mon_bytes;
-  if (need > s->arena_bytes) {
-    if (s->arena) cudaFree(s->arena);
-    s->arena = nullptr;
-    s->arena_bytes = 0;
-    XLB_CUDA(cudaMalloc(&s->arena, need));
-    s->arena_bytes = need;
-  }
-  unsigned char *cur = s->arena;
-  auto take = [&](size_t bytes) { unsigned char *r = cur; cur += bytes; return r; };
-  xlb_lattice_t dl = *hl;
-  dl.words = reinterpret_cast<const uint64_t *>(take(lat_bytes));
-  XLB_CUDA(cudaMemcpyAsync(const_cast<uint64_t *>(dl.words), hl->words,
-                           static_cast<size_t>(hl->n_words) * 8, cudaMemcpyHostToDevice, st));
   xlb_particles_t dp = *hp;
-  double **dcols[] = {&dp.x, &dp.px, &dp.y, &dp.py, &dp.zeta, &dp.delta, &dp.rpp, &dp.rvv, &dp.s};
-  double *const hcols[] = {hp->x, hp->px, hp->y, hp->py, hp->zeta, hp->delta, hp->rpp, hp->rvv, hp->s};
-  int64_t **dicols[] = {&dp.state, &dp.at_element, &dp.at_turn};
-  int64_t *const hicols[] = {hp->state, hp->at_element, hp->at_turn};
+  xlb_track_options_t od = *o;
   // a chi column of ones is the one-species case: not uploaded, and the kernels without a chi
   // register serve the call (see xlb_particles_t)
   bool chi_trivial = true;
@@ -996,86 +919,78 @@ int xlb_track_host(const xlb_lattice_t *hl, xlb_particles_t *hp, const xlb_track
       if (hp->chi[i] != 1.0) { chi_trivial = false; break; }
   if (chi_trivial) dp.chi = nullptr;
 
+  // The arrays of the call: host array (NULL = none), the field of the device-side call that
+  // receives its device address, its size, and whether the tracking writes it.  The particle
+  // columns come first.
+  struct Column {
+    const void *host;
+    void **dev;
+    size_t bytes;
+    bool back;
+  };
+  const size_t col = static_cast<size_t>(n) * 8;
+  const Column cols[] = {
+      {hp->x, slot(&dp.x), col, true},
+      {hp->px, slot(&dp.px), col, true},
+      {hp->y, slot(&dp.y), col, true},
+      {hp->py, slot(&dp.py), col, true},
+      {hp->zeta, slot(&dp.zeta), col, true},
+      {hp->delta, slot(&dp.delta), col, true},
+      {hp->rpp, slot(&dp.rpp), col, true},
+      {hp->rvv, slot(&dp.rvv), col, true},
+      {hp->s, slot(&dp.s), col, true},
+      {hp->state, slot(&dp.state), col, true},
+      {hp->at_element, slot(&dp.at_element), col, true},
+      {hp->at_turn, slot(&dp.at_turn), col, true},
+      {hp->particle_id, slot(&dp.particle_id), col, false},
+      {dp.chi, slot(&dp.chi), col, false},
+      {hp->charge_ratio, slot(&dp.charge_ratio), col, false},
+      {o->loss_tally, slot(&od.loss_tally), static_cast<size_t>(hl->n_elements) * 8, true},
+      {o->monitor_data, slot(&od.monitor_data), static_cast<size_t>(o->monitor_words) * 8, true},
+  };
+  const int n_cols = static_cast<int>(sizeof(cols) / sizeof(cols[0])), n_particle_cols = 15;
+
   // Small single-launch calls on PINNED host buffers (C1: 10 000 particles x 100 turns): the
   // kernel reads and writes the caller's arrays in place through their device aliases -- the
   // particle state crosses the bus once each way inside the kernel's own entry and exit, instead
   // of 26 separate DMA transfers of 80 kB whose set-up latencies dominate a 0.3 ms call.
-  const int seg_len = (o->turns_per_launch > 0) ? o->turns_per_launch
-                      : (o->turns_per_launch == 0 && o->num_turns > 150 ? 100 : o->num_turns);
-  bool in_place = n <= 16384 && seg_len >= o->num_turns;
-  if (in_place) {
-    auto alias = [&](const void *h, void **d) {
-      cudaPointerAttributes at;
-      if (cudaPointerGetAttributes(&at, h) != cudaSuccess) {
-        cudaGetLastError();
-        return false;
-      }
-      if (at.type != cudaMemoryTypeHost || !at.devicePointer) return false;
-      *d = at.devicePointer;
-      return true;
-    };
-    xlb_particles_t ap = dp;
-    bool ok = true;
-    double **acols[] = {&ap.x, &ap.px, &ap.y, &ap.py, &ap.zeta, &ap.delta, &ap.rpp, &ap.rvv, &ap.s};
-    for (int c = 0; c < 9 && ok; ++c) ok = alias(hcols[c], reinterpret_cast<void **>(acols[c]));
-    int64_t **aicols[] = {&ap.state, &ap.at_element, &ap.at_turn};
-    for (int c = 0; c < 3 && ok; ++c) ok = alias(hicols[c], reinterpret_cast<void **>(aicols[c]));
-    if (ok) ok = alias(hp->particle_id, reinterpret_cast<void **>(const_cast<int64_t **>(&ap.particle_id)));
-    if (ok && ap.chi) ok = alias(hp->chi, reinterpret_cast<void **>(const_cast<double **>(&ap.chi)));
-    if (ok && ap.charge_ratio)
-      ok = alias(hp->charge_ratio, reinterpret_cast<void **>(const_cast<double **>(&ap.charge_ratio)));
-    in_place = ok;
-    if (ok) dp = ap;
-  }
-  if (!in_place)
-    for (int c = 0; c < 9; ++c) {
-      *dcols[c] = reinterpret_cast<double *>(take(col));
-      XLB_CUDA(cudaMemcpyAsync(*dcols[c], hcols[c], static_cast<size_t>(n) * 8, cudaMemcpyHostToDevice, st));
+  auto alias = [](const void *h, void **d) {
+    cudaPointerAttributes at;
+    if (cudaPointerGetAttributes(&at, h) != cudaSuccess) {
+      cudaGetLastError();
+      return false;
     }
-  if (!in_place && hp->chi && !chi_trivial) {
-    double *d = reinterpret_cast<double *>(take(col));
-    XLB_CUDA(cudaMemcpyAsync(d, hp->chi, static_cast<size_t>(n) * 8, cudaMemcpyHostToDevice, st));
-    dp.chi = d;
-  }
-  if (!in_place && hp->charge_ratio) {
-    double *d = reinterpret_cast<double *>(take(col));
-    XLB_CUDA(cudaMemcpyAsync(d, hp->charge_ratio, static_cast<size_t>(n) * 8, cudaMemcpyHostToDevice, st));
-    dp.charge_ratio = d;
-  }
-  if (!in_place)
-    for (int c = 0; c < 3; ++c) {
-      *dicols[c] = reinterpret_cast<int64_t *>(take(col));
-      XLB_CUDA(cudaMemcpyAsync(*dicols[c], hicols[c], static_cast<size_t>(n) * 8, cudaMemcpyHostToDevice, st));
-    }
-  if (!in_place) {
-    int64_t *d = reinterpret_cast<int64_t *>(take(col));
-    XLB_CUDA(cudaMemcpyAsync(d, hp->particle_id, static_cast<size_t>(n) * 8, cudaMemcpyHostToDevice, st));
-    dp.particle_id = d;
-  }
-  xlb_track_options_t od = *o;
-  if (o->loss_tally) {
-    od.loss_tally = reinterpret_cast<int64_t *>(take(tally_bytes));
-    XLB_CUDA(cudaMemcpyAsync(od.loss_tally, o->loss_tally, static_cast<size_t>(hl->n_elements) * 8,
-                             cudaMemcpyHostToDevice, st));
-  }
-  if (o->monitor_data) {
-    od.monitor_data = reinterpret_cast<double *>(take(mon_bytes));
-    XLB_CUDA(cudaMemcpyAsync(od.monitor_data, o->monitor_data, static_cast<size_t>(o->monitor_words) * 8,
-                             cudaMemcpyHostToDevice, st));
+    if (at.type != cudaMemoryTypeHost || !at.devicePointer) return false;
+    *d = at.devicePointer;
+    return true;
+  };
+  bool in_place = n <= 16384 && launch_cap(o->turns_per_launch, o->num_turns, hl->n_chunks) >= o->num_turns;
+  for (int c = 0; c < n_particle_cols && in_place; ++c)
+    in_place = !cols[c].host || alias(cols[c].host, cols[c].dev);
+  const int first = in_place ? n_particle_cols : 0;  // the arrays copied to and from the device
+
+  // device arena: lattice | copied arrays
+  auto al = [](size_t v) { return (v + 255) & ~static_cast<size_t>(255); };
+  const size_t lat_bytes = al(static_cast<size_t>(hl->n_words) * 8);
+  size_t need = lat_bytes;
+  for (int c = first; c < n_cols; ++c)
+    if (cols[c].host) need += al(cols[c].bytes);
+  if ((rc = grow(&s->arena, &s->arena_bytes, need)) != XLB_OK) return rc;
+  xlb_lattice_t dl = *hl;
+  dl.words = reinterpret_cast<const uint64_t *>(s->arena);
+  XLB_CUDA(cudaMemcpyAsync(s->arena, hl->words, static_cast<size_t>(hl->n_words) * 8, cudaMemcpyHostToDevice, st));
+  unsigned char *cur = s->arena + lat_bytes;
+  for (int c = first; c < n_cols; ++c) {
+    if (!cols[c].host) continue;
+    *cols[c].dev = cur;
+    cur += al(cols[c].bytes);
+    XLB_CUDA(cudaMemcpyAsync(*cols[c].dev, cols[c].host, cols[c].bytes, cudaMemcpyHostToDevice, st));
   }
   if ((rc = track_device_impl(&dl, &dp, &od, st, !in_place)) != XLB_OK) return rc;
-  if (!in_place) {
-    for (int c = 0; c < 9; ++c)
-      XLB_CUDA(cudaMemcpyAsync(hcols[c], *dcols[c], static_cast<size_t>(n) * 8, cudaMemcpyDeviceToHost, st));
-    for (int c = 0; c < 3; ++c)
-      XLB_CUDA(cudaMemcpyAsync(hicols[c], *dicols[c], static_cast<size_t>(n) * 8, cudaMemcpyDeviceToHost, st));
-  }
-  if (o->loss_tally)
-    XLB_CUDA(cudaMemcpyAsync(o->loss_tally, od.loss_tally, static_cast<size_t>(hl->n_elements) * 8,
-                             cudaMemcpyDeviceToHost, st));
-  if (o->monitor_data)
-    XLB_CUDA(cudaMemcpyAsync(o->monitor_data, od.monitor_data, static_cast<size_t>(o->monitor_words) * 8,
-                             cudaMemcpyDeviceToHost, st));
+  for (int c = first; c < n_cols; ++c)
+    if (cols[c].host && cols[c].back)  // the caller's writable arrays
+      XLB_CUDA(cudaMemcpyAsync(const_cast<void *>(cols[c].host), *cols[c].dev, cols[c].bytes,
+                               cudaMemcpyDeviceToHost, st));
   XLB_CUDA(cudaStreamSynchronize(st));
   return XLB_OK;
 }

@@ -48,8 +48,7 @@ struct Variant {
   int nochi;     // 1 = compiled for chi == 1 throughout (xlb_particles_t::chi == NULL)
   int maxorder;  // 0 = any multipole order; else the highest order the kernel evaluates (XLB_F_LOW_ORDER)
   int polygons;  // 1 = track_kernel_polygons: for the lattices flagged XLB_F_POLYGONS, and only those
-  const void *func;
-  void (*launch)(const KArgs &, int blocks, int threads, size_t smem, void *stream);
+  const void *func;  // the kernel's host stub
 };
 
 // The 6D beam-beam lens as a kernel of its own (segmented lattices): one particle per thread,

@@ -58,7 +58,6 @@
 
 namespace xlb {
 using namespace XLB_NS;
-XLB_DEF_TRACE_VARIANT()
 
 // (particles per thread, launch-bounds threads, resident CTAs per SM asked for)
 #if XLB_BEAMFIELDS == 2
@@ -82,8 +81,6 @@ XLB_DEF_TRACE_VARIANT()
 #define XLB_SHAPES(X) X(1, 128, 5) X(1, 256, 3) X(1, 512, 2) X(2, 128, 3) X(2, 256, 2) X(3, 128, 3) X(4, 128, 2)
 #endif
 
-#define XLB_X_DEF(P, T, M) XLB_DEF_VARIANT(P, T, M)
-XLB_SHAPES(XLB_X_DEF)
 #define XLB_X_ENTRY(P, T, M) XLB_VARIANT_ENTRY("fast/ppt" #P "/t" #T XLB_FAMILY, P, T, M),
 #define XLB_X_POLYGON_ENTRY(P, T, M) XLB_POLYGON_VARIANT_ENTRY("fast/ppt" #P "/t" #T XLB_FAMILY "/polygons", P, T, M),
 static const Variant family_table[] = {

@@ -17,13 +17,6 @@
 
 namespace xlb {
 using namespace XLB_NS;
-XLB_DEF_TRACE_VARIANT()
-XLB_DEF_VARIANT(1, 256, 1)
-XLB_DEF_VARIANT(2, 256, 1)
-#if !XLB_BEAMFIELDS
-XLB_DEF_VARIANT(2, 128, 3)
-XLB_DEF_VARIANT(3, 128, 3)
-#endif
 
 #if XLB_BEAMFIELDS
 #define XLB_TABLE strict_bf_table
