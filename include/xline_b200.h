@@ -334,6 +334,50 @@ int xlb_track_device_moments(const xlb_lattice_t *lattice, xlb_particles_t *part
                              const xlb_track_options_t *opts, const xlb_moments_spec_t *spec,
                              double *out, void *stream);
 
+/* ---------------------------------------------------------------------------------
+ * NAFF tunes (DESIGN.md §4.7): the frequency and amplitude of the largest spectral line of
+ * turn-by-turn signals, for tune footprints and frequency maps.
+ *
+ * A signal is T = num_turns samples u_t (and optionally pu_t), t = 0 .. T-1.  The analysed z_t:
+ *   complex (pu given):  z_t = u_t/√β - i·(α·u_t + β·pu_t)/√β  (√(2J)·e^{+iφ_t} for linear motion
+ *                        at a point with Twiss β > 0, α: the peak sits at +ν, ν in [0, 1));
+ *                        β = 1, α = 0 gives x - i·px;
+ *   real (pu NULL):      z_t = u_t, ν in [0, 1/2]; β and α are ignored.
+ * 1. z_t <- z_t - (1/T)·Σ z_t.
+ * 2. Hann window w_t = 1 - cos(2πt/T)  (Σ w_t = T).
+ * 3. Z(ν) = Σ_t w_t·z_t·e^{-2πiν(t - T/2)}  (the centred phase changes the phase of Z only).
+ * 4. Coarse peak: M = the smallest power of two >= T; k = argmax |Z(k/M)| (zero-padded DFT) over
+ *    k = 1 .. M-1 (complex) or k = 1 .. M/2 (real), the lowest k on ties.
+ * 5. The root ν of D(ν) = Re(conj(Z)·Z') (Z', Z'' derivatives in ν) in [(k-1)/M, (k+1)/M]:
+ *    Newton from k/M, D'(ν) = |Z'|² + Re(conj(Z)·Z''), with a bisection safeguard (a step that
+ *    leaves the bracket, or D' >= 0, bisects; D > 0 raises the lower end, else the upper one).
+ *    It stops when a step is below 1e-15, when D = 0 with D' < 0, or after 40 steps (D = 0 with
+ *    D' >= 0 -- e.g. ν = 1/2 between a real signal's line and its mirror image -- bisects).
+ * 6. tune = ν folded into the range above (the brackets of k = M-1 and k = M/2 reach past
+ *    it): ν - 1 for a complex ν >= 1, 1 - ν for a real ν > 1/2, both exact;  amplitude = |Z|/Σ w_t at the last evaluation (|Z| is stationary there), which is
+ *    √(2J) for a linear particle in normalised coordinates.
+ * 7. A non-finite sample (a particle lost inside the window, an id never stored): tune and
+ *    amplitude NaN.  z = 0 after step 1: tune NaN, amplitude 0.
+ * Accuracy: a pure complex tone is recovered to ~1e-11 at T ~ 1000 (real tones ~1e-9: the mirror
+ *   line at -ν leaks through the window; within ~1/T of 0 or 1/2 the two lines merge and the real
+ *   tune comes out near 0 or 1/2); most of the remaining error is leakage from the
+ *   subtracted mean.  The device computes the same root of D as a float64 evaluation of the
+ *   steps above to ~1e-12 (1e-12 relative in amplitude) unless the two largest coarse bins are
+ *   within ~1e-9 of each other.
+ * Reproducibility: every sum runs in an order fixed by t alone, so a signal's tune and amplitude
+ *   are bitwise independent of n, its position in the batch, the row stride and the launch shape.
+ * --------------------------------------------------------------------------------- */
+#define XLB_NAFF_MIN_TURNS 64
+#define XLB_NAFF_MAX_TURNS 8192
+
+/* NAFF of the n signals j = 0 .. n-1 of a turn-major slab (device pointers): sample t of signal
+ * j at u[t·stride + j] and pu[t·stride + j] (the layout of a BeamMonitor field), pu NULL for real
+ * signals.  Writes tune_out[j] and amplitude_out[j].  Enqueued on `stream`, no synchronisation.
+ * XLB_EINVAL for n < 0, num_turns outside [XLB_NAFF_MIN_TURNS, XLB_NAFF_MAX_TURNS], stride < n,
+ * a null pointer with n > 0, or (pu given) β not (finite and > 0) or α not finite.  n = 0: no-op. */
+int xlb_naff_device(const double *u, const double *pu, int64_t n, int64_t num_turns, int64_t stride,
+                    double beta, double alpha, double *tune_out, double *amplitude_out, void *stream);
+
 /* Register-resident independent-DFMA-chain microbenchmark: the measured FP64 pipe peak of
  * the current device in FLOP/s (2 flops per DFMA), best of `repeats`.  The roofline
  * denominator of bench.py (MEASURED_PEAKS.json has no FP64 entry). */

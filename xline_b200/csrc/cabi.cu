@@ -883,6 +883,25 @@ int xlb_beam_moments_device(const xlb_particles_t *particles, double *out, void 
   return beam_moments(call.s, particles, out, static_cast<cudaStream_t>(stream));
 }
 
+int xlb_naff_device(const double *u, const double *pu, int64_t n, int64_t num_turns, int64_t stride,
+                    double beta, double alpha, double *tune_out, double *amplitude_out, void *stream) {
+  if (n < 0) return fail(XLB_EINVAL, "n < 0");
+  if (num_turns < XLB_NAFF_MIN_TURNS || num_turns > XLB_NAFF_MAX_TURNS)
+    return fail(XLB_EINVAL, "num_turns outside [XLB_NAFF_MIN_TURNS, XLB_NAFF_MAX_TURNS]");
+  if (stride < n) return fail(XLB_EINVAL, "stride < n");
+  if (n > 0 && (!u || !tune_out || !amplitude_out)) return fail(XLB_EINVAL, "null pointer");
+  if (pu && !(std::isfinite(beta) && beta > 0.0 && std::isfinite(alpha)))
+    return fail(XLB_EINVAL, "beta must be finite and > 0, alpha finite");
+  if (n > 2147483647LL) return fail(XLB_EINVAL, "n too large");
+  if (n == 0) return XLB_OK;
+  CallScope call;
+  int rc;
+  if ((rc = call.open(static_cast<cudaStream_t>(stream))) != XLB_OK) return rc;
+  XLB_CUDA(naff_launch(u, pu, n, static_cast<int>(num_turns), stride, beta, alpha, tune_out, amplitude_out,
+                       static_cast<cudaStream_t>(stream)));
+  return XLB_OK;
+}
+
 int xlb_compact_alive_device(const int64_t *state, int64_t n, int32_t *idx_out, int32_t *n_out,
                              void *stream) {
   if (n < 0 || (n > 0 && (!state || !idx_out)) || !n_out) return fail(XLB_EINVAL, "bad argument");

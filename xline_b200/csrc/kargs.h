@@ -67,6 +67,11 @@ cudaError_t beam_moments_launch(const double *x, const double *px, const double 
                                 const double *zeta, const double *delta, const long long *state, long long n,
                                 double *scratch, double *out, cudaStream_t st);
 
+// NAFF tune and amplitude of n turn-major signals (naff.cu): sample t of signal j at
+// u[t * stride + j] (and pu[..], nullptr for real signals); arguments checked by the caller.
+cudaError_t naff_launch(const double *u, const double *pu, long long n, int num_turns, long long stride,
+                        double beta, double alpha, double *tune, double *amplitude, cudaStream_t st);
+
 // variant tables, one per translation unit (kernel family)
 const Variant *fast_lean_variants(int *n);
 const Variant *fast_lean_nc_variants(int *n);
