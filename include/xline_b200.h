@@ -378,6 +378,40 @@ int xlb_track_device_moments(const xlb_lattice_t *lattice, xlb_particles_t *part
 int xlb_naff_device(const double *u, const double *pu, int64_t n, int64_t num_turns, int64_t stride,
                     double beta, double alpha, double *tune_out, double *amplitude_out, void *stream);
 
+/* ---------------------------------------------------------------------------------
+ * Tangent map (DESIGN.md §4.8): particles tracked as xlb_track_device tracks them, each carrying
+ * its Jacobian  J = dz/dz0  over z = (x, px, y, py, zeta, delta), for chaos indicators, closed
+ * orbits and one-turn matrices of the tracked map itself.
+ *
+ * Lattice: one record per element -- no block records (tags >= 0x80), no segments, the fast
+ *   encoding (XLB_F_STRICT clear); BEAMBEAM6D is refused.  MONITOR records are the identity and
+ *   store nothing.  rpp and rvv are functions of delta throughout.
+ * Layout: jac[i*36 + r*6 + c] = dz_r/dz0_c of particle i (row-major 6x6, r, c in the order of z);
+ *   the caller initialises it (the identity for a fresh start).  The true Jacobian is
+ *   jac[i] * 2^log2_scale[i].
+ * Per turn: J <- J_elem(z before the element) . J for every element; at the end of every turn of a
+ *   surviving particle, with m = max|J|: if m > 2^512, J <- J * 2^-ilogb(m) and
+ *   log2_scale += ilogb(m) (exact: the result does not depend on when it happens), then
+ *     fli <- max(fli, log10 ||J||_F + log2_scale * log10 2).
+ *   The caller initialises fli (log10 sqrt(6), the identity's, for a fresh start).
+ * Losses: state, at_element, at_turn, s and the loss tally as xlb_track_device; a lost particle's
+ *   jac, log2_scale and fli are written where it was lost and not touched again.  Particles with
+ *   state != 1 at the call are left alone.
+ * Reproducibility: one particle per thread with nothing shared, so results are bitwise independent
+ *   of n, the particle's slot and threads_per_block; T1 turns then T2 turns equal T1 + T2 turns.
+ * Options: num_turns, loss_tally, flags, element_index_offset and threads_per_block (0 = 128, a
+ *   multiple of 32 <= 256) are used; particles_per_thread must be 0 or 1; trace is refused.
+ * One launch, enqueued on `stream`; the lattice words are read back to the host once per call to
+ *   check the tags (a stream synchronisation).  XLB_EINVAL for the refusals above (the message names
+ *   the element) and a null jac / log2_scale / fli with n > 0.
+ * --------------------------------------------------------------------------------- */
+#define XLB_TANGENT_SCALE_LOG2 512  /* the overflow guard's threshold, 2^512 */
+#define XLB_TANGENT_MAX_THREADS 256
+
+int xlb_track_tangent_device(const xlb_lattice_t *lattice, xlb_particles_t *particles,
+                             const xlb_track_options_t *opts, double *jac /*[n][6][6]*/, int64_t *log2_scale,
+                             double *fli, void *stream);
+
 /* Register-resident independent-DFMA-chain microbenchmark: the measured FP64 pipe peak of
  * the current device in FLOP/s (2 flops per DFMA), best of `repeats`.  The roofline
  * denominator of bench.py (MEASURED_PEAKS.json has no FP64 entry). */

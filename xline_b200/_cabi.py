@@ -16,13 +16,15 @@ MOMENT_PAIRS = 27  # XLB_MOMENT_PAIRS: (hi, lo) sums of a store
 MOMENT_FIRST = 2   # XLB_MOMENT_FIRST: word of the first pair, after n and n_nonfinite
 NAFF_MIN_TURNS = 64    # XLB_NAFF_MIN_TURNS: shortest signal xlb_naff_device takes
 NAFF_MAX_TURNS = 8192  # XLB_NAFF_MAX_TURNS: longest
+TANGENT_SCALE_LOG2 = 512     # XLB_TANGENT_SCALE_LOG2: the tangent map's overflow guard, 2^512
+TANGENT_MAX_THREADS = 256    # XLB_TANGENT_MAX_THREADS
 
 EXPORTS = (
     "xlb_abi_version", "xlb_last_error", "xlb_lattice_validate", "xlb_track_device",
     "xlb_track_device_timed", "xlb_track_host", "xlb_get_stats", "xlb_compact_alive_device",
     "xlb_measure_fp64_peak", "xlb_measure_dfma_latency", "xlb_kernel_variant_count",
     "xlb_kernel_variant_info", "xlb_selftest_exact_division", "xlb_beam_moments_device",
-    "xlb_track_device_moments", "xlb_naff_device",
+    "xlb_track_device_moments", "xlb_naff_device", "xlb_track_tangent_device",
 )
 
 
@@ -97,6 +99,9 @@ def lib():
     L.xlb_naff_device.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_double,
                                   C.c_double, C.c_void_p, C.c_void_p, C.c_void_p]
     L.xlb_naff_device.restype = C.c_int
+    L.xlb_track_tangent_device.argtypes = [C.POINTER(Lattice), C.POINTER(Particles), C.POINTER(TrackOptions),
+                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.xlb_track_tangent_device.restype = C.c_int
     L.xlb_track_host.argtypes = [C.POINTER(Lattice), C.POINTER(Particles), C.POINTER(TrackOptions)]
     L.xlb_track_host.restype = C.c_int
     L.xlb_get_stats.argtypes = [C.POINTER(TrackStats)]

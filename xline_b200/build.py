@@ -24,6 +24,7 @@ UNITS = [
     ("cabi", "cabi.cu", []),
     ("moments", "moments.cu", []),                                            # beam-moment reduction
     ("naff", "naff.cu", []),                                                  # NAFF tunes of monitor data
+    ("tangent", "tangent.cu", []),                                            # tangent map (Jacobians, FLI)
     ("track_fast", "track_fast.cu", []),
     ("track_fast_nc", "track_fast.cu", ["-DXLB_NOCHI=1"]),                      # chi == 1 throughout
     ("track_fast_nc_lo", "track_fast.cu", ["-DXLB_NOCHI=1", "-DXLB_MAXORDER=3"]),  # + multipole order <= 3

@@ -902,6 +902,54 @@ int xlb_naff_device(const double *u, const double *pu, int64_t n, int64_t num_tu
   return XLB_OK;
 }
 
+int xlb_track_tangent_device(const xlb_lattice_t *lat, xlb_particles_t *p, const xlb_track_options_t *o,
+                             double *jac, int64_t *log2_scale, double *fli, void *stream) {
+  memset(&g_stats, 0, sizeof(g_stats));
+  int rc;
+  if ((rc = check_call(lat, p, o, nullptr)) != XLB_OK) return rc;
+  if (o->trace) return fail(XLB_EINVAL, "tangent tracking does not combine with a trace");
+  if (lat->flags & XLB_F_STRICT) return fail(XLB_EINVAL, "tangent tracking needs a lattice in the fast encoding");
+  if (lat->n_segments > 0) return fail(XLB_EINVAL, "tangent tracking needs an unsegmented lattice");
+  if (o->particles_per_thread != 0 && o->particles_per_thread != 1)
+    return fail(XLB_EINVAL, "tangent tracking runs one particle per thread");
+  const int threads = o->threads_per_block > 0 ? o->threads_per_block : 128;
+  if (threads % 32 || threads > XLB_TANGENT_MAX_THREADS)
+    return fail(XLB_EINVAL, "threads_per_block must be a multiple of 32 and <= XLB_TANGENT_MAX_THREADS");
+  if (p->n == 0 || o->num_turns == 0) return XLB_OK;
+  if (!jac || !log2_scale || !fli) return fail(XLB_EINVAL, "jac, log2_scale and fli must not be null");
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  CallScope call;
+  if ((rc = call.open(st)) != XLB_OK) return rc;
+  // The kernel knows one record per element: refuse the block records and the 6D lens up front.
+  std::vector<uint64_t> w(static_cast<size_t>(lat->n_words));
+  XLB_CUDA(cudaMemcpyAsync(w.data(), lat->words, w.size() * 8, cudaMemcpyDefault, st));
+  XLB_CUDA(cudaStreamSynchronize(st));
+  for (int c = 0; c < lat->n_chunks; ++c) {
+    for (size_t pos = static_cast<size_t>(c) * lat->chunk_words; pos < static_cast<size_t>(c + 1) * lat->chunk_words;) {
+      const uint64_t hdr = w[pos];
+      const int tag = static_cast<int>(hdr & 0xff), pairs = static_cast<int>((hdr >> 16) & 0x3fff);
+      if (tag == XLB_T_END_TURN || tag == XLB_T_END_CHUNK) break;
+      if (tag == XLB_T_BEAMBEAM6D || tag >= XLB_T__COUNT) {
+        char buf[160];
+        snprintf(buf, sizeof buf, "tangent tracking: element %d is %s", static_cast<int>(hdr >> 32),
+                 tag == XLB_T_BEAMBEAM6D ? "a BeamBeam6D lens (its Jacobian is not implemented)"
+                                         : "a fused block record (pack one record per element)");
+        return fail(XLB_EINVAL, buf);
+      }
+      if (pairs < 1) return fail(XLB_ELATTICE, "record of size 0");
+      pos += 2 * static_cast<size_t>(pairs);
+    }
+  }
+  KArgs a = kernel_args(lat, p, o, call.s->n_lost);
+  a.num_turns = o->num_turns;
+  XLB_CUDA(tangent_launch(a, jac, reinterpret_cast<long long *>(log2_scale), fli, threads, st));
+  g_stats.kernel_launches = 1;
+  g_stats.threads = threads;
+  g_stats.blocks = static_cast<int>((p->n + threads - 1) / threads);
+  g_stats.n_alive_in = p->n;
+  return XLB_OK;
+}
+
 int xlb_compact_alive_device(const int64_t *state, int64_t n, int32_t *idx_out, int32_t *n_out,
                              void *stream) {
   if (n < 0 || (n > 0 && (!state || !idx_out)) || !n_out) return fail(XLB_EINVAL, "bad argument");

@@ -72,6 +72,11 @@ cudaError_t beam_moments_launch(const double *x, const double *px, const double 
 cudaError_t naff_launch(const double *u, const double *pu, long long n, int num_turns, long long stride,
                         double beta, double alpha, double *tune, double *amplitude, cudaStream_t st);
 
+// Tangent-map tracking of the a.n particles (tangent.cu): one particle per thread, `threads` per CTA,
+// all a.num_turns turns in one launch; arguments checked by the caller.
+cudaError_t tangent_launch(const KArgs &a, double *jac, long long *log2_scale, double *fli, int threads,
+                           cudaStream_t st);
+
 // variant tables, one per translation unit (kernel family)
 const Variant *fast_lean_variants(int *n);
 const Variant *fast_lean_nc_variants(int *n);
