@@ -120,7 +120,49 @@ enum xlb_tag {
      records carries XLB_F_POLYGONS.  Added without an ABI version change: a library that
      predates the tag refuses the lattice in xlb_lattice_validate ("unknown tag").           */
   XLB_T_LIMIT_POLYGON = 19,
-  XLB_T__COUNT = 20,
+  /* Radiating multipole (DESIGN.md §4.9): a Multipole of length L > 0 on a line tracked with
+     synchrotron radiation.  Fast encoding only.  aux = order;
+       [hdr,i64 mode (1 mean, 2 quantum)][L,1/L][K_e,hbar_c][alpha,u64 seed]
+       then the element's own MULTIPOLE or MULTIPOLE_CURVED record, header word included, exactly
+       as it is packed on its own (hxl, hyl come from there; 0 for the straight one).
+     K_e = e^2/(4 pi eps0) and hbar_c in eV m, alpha the fine-structure constant: taken at pack
+     time, nothing physical is compiled into the kernel.  q0, mass0, p0c come from the call.
+     Map, with (dpx_f, dpy_f) the Horner polynomial of knl/ksl (k0l included) at the element's
+     (x, y) -- the field part of the kick, without the hxl/hyl reference-frame terms:
+       kappa = sqrt(dpx_f^2 + dpy_f^2) / ((1 + delta) L),  l_h = (L + hxl x - hyl y) / 2;
+       1. radiate over l_h;  2. the multipole map of the embedded record, unchanged;
+       3. radiate over l_h with kappa recomputed from the new delta (x, y and the field unchanged).
+     Radiating an energy dE < 0 (P = (1+delta) p0c, E = sqrt(P^2 + m^2), gamma = E/m, beta = P/E, with
+     m^2 = (energy0 - p0c)(energy0 + p0c) from the call's reference particle -- for a 6 GeV electron
+     the rounding of energy0 leaves m, and so the loss, uncertain at the 1e-8 level):
+       Pyparticles.add_to_energy(dE) as Cavity does (delta, rpp, rvv, zeta rvv'/rvv), then px and
+       py times (1+delta')/(1+delta): the photon leaves along the direction of motion.
+       mean:    dE = -(2/3) q0^2 K_e beta^3 gamma^4 kappa^2 l_h;
+       quantum: k ~ Poisson(nbar), nbar = (5/(2 sqrt 3)) q0^2 alpha gamma kappa l_h, k <= 255;
+                dE = -u_c sum_{i=1..k} x_i, u_c = (3/2) hbar_c gamma^3 kappa, x_i = F^-1(U_i) of
+                the photon-number spectrum dN/dx ~ int_x^inf K_5/3 (csrc/synrad_table.inc).
+       The quantum mode's expected loss is (2/3) q0^2 K_e gamma^4 kappa^2 l_h: the mean mode's up to
+       the factor beta^3 = 1 - O(1/gamma^2).  A half with kappa == 0 (mean) or k == 0 (quantum)
+       leaves the particle untouched.
+     Random numbers: Philox4x32-10, key (lo32(seed), hi32(seed)), counter (lo32(particle_id),
+       hi32(particle_id), lo32(turn), element << 8 | half << 7 | j), where turn = the particle's
+       at_turn at the element (stored value + turns of this call), element = the record's element
+       index + element_index_offset (< 2^24), half 0 / 1 (entrance / exit).  Output words
+       r0..r3 of call j give the uniforms 2j (from w = r1 2^32 + r0) and 2j + 1 (w = r3 2^32 + r2),
+       U = ((w >> 11) + 0.5) 2^-53 in (0, 1).  Uniform 0 gives k: the smallest i with U <= C_i,
+       C_0 = p_0 = exp(-nbar), p_i = p_(i-1) nbar / i, C_i = C_(i-1) + p_i (capped at 255; never
+       reached for nbar below ~100).  Uniforms 1..k give x_1..x_k.
+     Reproducibility: every draw is a function of (seed, particle_id, turn, element, half) alone,
+       so results are bitwise independent of particles per thread, threads per block,
+       turns_per_launch, the work queue, survivor compaction and the rest of the batch; T1 turns
+       then T2 turns equal T1 + T2 turns.
+     A lattice with these records carries XLB_F_RADIATION.  Refused (XLB_ELATTICE): a strict
+     lattice, beam-field records, more than 2^24 elements.  Refused (XLB_EINVAL) at tracking
+     time: a chi column (multi-species beams), element_index_offset + n_elements > 2^24, and the
+     tangent map.  Added without an ABI version change: a library that predates the tag refuses
+     the lattice in xlb_lattice_validate ("unknown tag").                                       */
+  XLB_T_MULTIPOLE_RAD = 20,
+  XLB_T__COUNT = 21,
   /* Fused thin multipole -> [aperture] -> [drift] records (pack-time peephole).  The tag
      has bit 7 set and describes the block: bits 0-1 aperture kind (0 none, 1 symmetric
      rect, 2 rect, 3 ellipse), bit 2 curved multipole, bit 3 drift present, bit 4 that drift
@@ -189,6 +231,12 @@ typedef struct xlb_lattice {
                                 (checked by xlb_lattice_validate; optional, never required) */
 #define XLB_F_POLYGONS 16u   /* the lattice holds LIMIT_POLYGON records (mandatory: checked by
                                 xlb_lattice_validate; the kernels that can track them are used) */
+#define XLB_F_RADIATION 32u  /* the lattice holds MULTIPOLE_RAD records (mandatory: checked by
+                                xlb_lattice_validate; only the one-species thin-lens fast
+                                kernels carry the case)                                  */
+#define XLB_RAD_MEAN 1
+#define XLB_RAD_QUANTUM 2
+#define XLB_RAD_MAX_ELEMENTS (1 << 24)
 
 /* Particle set, mirrors the attributes the reference's elements read and write
  * (SURVEY.md §8a row a2).  All arrays have length n.  chi and charge_ratio may be NULL

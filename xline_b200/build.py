@@ -35,7 +35,7 @@ UNITS = [
     ("track_strict_bf", "track_strict.cu", ["-DXLB_BEAMFIELDS=2", "-fmad=false"]),
 ]
 HEADERS = ["track_impl.cuh", "kargs.h", "launch_plan.h", "variants.inc", "beamfields.cuh",
-           "faddeeva_coeffs.inc", os.path.join("..", "..", "include", "xline_b200.h")]
+           "faddeeva_coeffs.inc", "synrad_table.inc", os.path.join("..", "..", "include", "xline_b200.h")]
 
 
 def _nvcc():

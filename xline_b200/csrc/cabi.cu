@@ -303,10 +303,13 @@ static const int kNumTables = static_cast<int>(sizeof(kTables) / sizeof(kTables[
 struct Need {
   bool strict, beamfields, bb6d, chi, trace, polygons;
   int max_order;  // highest multipole order the lattice may hold (255 = unknown)
+  bool radiation;
 };
 static bool admits(const Variant &v, const Need &q) {
   if ((v.strict != 0) != q.strict) return false;
-  if ((v.polygons != 0) != q.polygons) return false;  // the twins with the LIMIT_POLYGON case
+  if ((v.radiation != 0) != q.radiation) return false;  // the twins with the MULTIPOLE_RAD case
+  // the twins with the LIMIT_POLYGON case (the radiation twins carry it as well)
+  if (!q.radiation && (v.polygons != 0) != q.polygons) return false;
   if (q.strict) return (v.beamfields != 0) == q.beamfields;
   const int bf = q.beamfields ? (q.bb6d ? 2 : 1) : 0;
   if (v.beamfields != bf) return false;
@@ -438,6 +441,14 @@ static int check_call(const xlb_lattice_t *lat, const xlb_particles_t *p, const 
     return fail(XLB_EINVAL, "element-by-element trace needs num_turns == 1 and trace_particles >= 1");
   if (lat->n_segments > 1 && (o->trace || (lat->flags & XLB_F_STRICT)))
     return fail(XLB_EINVAL, "segmented lattices are for the fast kernels without trace");
+  if (lat->flags & XLB_F_RADIATION) {
+    if (lat->flags & (XLB_F_STRICT | XLB_F_BEAMFIELDS | XLB_F_BB6D))
+      return fail(XLB_ELATTICE, "radiation: a strict or beam-field lattice cannot carry radiating multipoles");
+    if (p->chi) return fail(XLB_EINVAL, "radiation: one species only (a chi column was given)");
+    if (o->element_index_offset < 0 ||
+        o->element_index_offset + static_cast<int64_t>(lat->n_elements) > XLB_RAD_MAX_ELEMENTS)
+      return fail(XLB_EINVAL, "radiation: element_index_offset + n_elements exceeds 2^24");
+  }
   return XLB_OK;
 }
 
@@ -546,7 +557,8 @@ static int track_device_impl(const xlb_lattice_t *lat, xlb_particles_t *p,
   const bool split = lat->n_segments > 1;  // 6D lenses run as kernels of their own
   const Need need{(lat->flags & XLB_F_STRICT) != 0, (lat->flags & XLB_F_BEAMFIELDS) != 0,
                   (lat->flags & XLB_F_BB6D) != 0 && !split, p->chi != nullptr, o->trace != nullptr,
-                  (lat->flags & XLB_F_POLYGONS) != 0, (lat->flags & XLB_F_LOW_ORDER) ? 3 : 255};
+                  (lat->flags & XLB_F_POLYGONS) != 0, (lat->flags & XLB_F_LOW_ORDER) ? 3 : 255,
+                  (lat->flags & XLB_F_RADIATION) != 0};
   const size_t smem = XLB_STAGES * static_cast<size_t>(lat->chunk_words) * 8 +
                       (2 * XLB_STAGES + 2) * sizeof(unsigned long long);
   int dev = 0, sms = 0;
@@ -782,6 +794,26 @@ int xlb_lattice_validate(const xlb_lattice_t *lat) {
           want = pairs;
           break;
         }
+        case XLB_T_MULTIPOLE_RAD: {  // [hdr,mode][L,1/L][K_e,hbar_c][alpha,seed] + MULTIPOLE(_CURVED) record
+          if (!(lat->flags & XLB_F_RADIATION)) return fail(XLB_ELATTICE, "radiating multipole without XLB_F_RADIATION");
+          if ((lat->flags & XLB_F_LOW_ORDER) && aux > 3)
+            return fail(XLB_ELATTICE, "XLB_F_LOW_ORDER set but a multipole has order > 3");
+          if (pos + 10 > lat->chunk_words) return fail(XLB_ELATTICE, "record runs past the end of its chunk");
+          const int64_t mode = static_cast<int64_t>(w[pos + 1]);
+          if (mode != XLB_RAD_MEAN && mode != XLB_RAD_QUANTUM) return fail(XLB_ELATTICE, "radiating multipole: bad mode");
+          double v[5];
+          memcpy(v, &w[pos + 2], sizeof v);  // L, 1/L, K_e, hbar_c, alpha
+          for (double x : v)
+            if (!(std::isfinite(x) && x > 0)) return fail(XLB_ELATTICE, "radiating multipole: L, 1/L and the constants must be finite and > 0");
+          const uint64_t sub = w[pos + 8];
+          const int st = static_cast<int>(sub & 0xff), saux = static_cast<int>((sub >> 8) & 0xff);
+          const int spairs = static_cast<int>((sub >> 16) & 0x3fff);
+          if ((st != XLB_T_MULTIPOLE && st != XLB_T_MULTIPOLE_CURVED) || saux != aux ||
+              spairs != (st == XLB_T_MULTIPOLE ? 1 : 3) + aux + 1 || (sub & 0xc0000000u))
+            return fail(XLB_ELATTICE, "radiating multipole: the embedded record is not a multipole of the same order");
+          want = 4 + spairs;
+          break;
+        }
         case XLB_T_MONITOR: want = 5; break;
         case XLB_T_BEAMBEAM4D:
         case XLB_T_SPACECHARGE:
@@ -850,6 +882,12 @@ int xlb_lattice_validate(const xlb_lattice_t *lat) {
     if (!closed) return fail(XLB_ELATTICE, "chunk not terminated by END_CHUNK/END_TURN");
   }
   if (!saw_end_turn) return fail(XLB_ELATTICE, "no END_TURN record");
+  if (lat->flags & XLB_F_RADIATION) {
+    if (lat->flags & XLB_F_STRICT) return fail(XLB_ELATTICE, "radiation: the strict encoding has no radiating multipoles");
+    if (lat->flags & (XLB_F_BEAMFIELDS | XLB_F_BB6D))
+      return fail(XLB_ELATTICE, "radiation: beam-field lattices cannot carry radiating multipoles");
+    if (lat->n_elements > XLB_RAD_MAX_ELEMENTS) return fail(XLB_ELATTICE, "radiation: more than 2^24 elements");
+  }
   return XLB_OK;
 }
 
@@ -908,6 +946,8 @@ int xlb_track_tangent_device(const xlb_lattice_t *lat, xlb_particles_t *p, const
   int rc;
   if ((rc = check_call(lat, p, o, nullptr)) != XLB_OK) return rc;
   if (o->trace) return fail(XLB_EINVAL, "tangent tracking does not combine with a trace");
+  if (lat->flags & XLB_F_RADIATION)
+    return fail(XLB_EINVAL, "tangent tracking: radiating multipoles are not in the tangent map");
   if (lat->flags & XLB_F_STRICT) return fail(XLB_EINVAL, "tangent tracking needs a lattice in the fast encoding");
   if (lat->n_segments > 0) return fail(XLB_EINVAL, "tangent tracking needs an unsegmented lattice");
   if (o->particles_per_thread != 0 && o->particles_per_thread != 1)

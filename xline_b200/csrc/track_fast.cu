@@ -23,6 +23,10 @@
 #ifndef XLB_MAXORDER
 #define XLB_MAXORDER 0
 #endif
+// Synchrotron radiation (MULTIPOLE_RAD, track_kernel_radiation): the one-species thin-lens families.
+#if XLB_NOCHI && !XLB_BEAMFIELDS
+#define XLB_RADIATION 1
+#endif
 
 // Beam-field kernels keep the warps of a CTA in step: one CTA barrier per lattice chunk.  Their
 // hot code (field maps, Faddeeva loop, the thin-lens records in between) is several times the L0
@@ -83,11 +87,17 @@ using namespace XLB_NS;
 
 #define XLB_X_ENTRY(P, T, M) XLB_VARIANT_ENTRY("fast/ppt" #P "/t" #T XLB_FAMILY, P, T, M),
 #define XLB_X_POLYGON_ENTRY(P, T, M) XLB_POLYGON_VARIANT_ENTRY("fast/ppt" #P "/t" #T XLB_FAMILY "/polygons", P, T, M),
+#define XLB_X_RADIATION_ENTRY(P, T, M) \
+  XLB_RADIATION_VARIANT_ENTRY("fast/ppt" #P "/t" #T XLB_FAMILY "/radiation", P, T, M),
 static const Variant family_table[] = {
     XLB_SHAPES(XLB_X_ENTRY)
     XLB_TRACE_ENTRY("fast/trace" XLB_FAMILY),
     XLB_SHAPES(XLB_X_POLYGON_ENTRY)
     XLB_POLYGON_TRACE_ENTRY("fast/trace" XLB_FAMILY "/polygons"),
+#if XLB_RADIATION
+    XLB_SHAPES(XLB_X_RADIATION_ENTRY)
+    XLB_RADIATION_TRACE_ENTRY("fast/trace" XLB_FAMILY "/radiation"),
+#endif
 };
 
 #define XLB_CAT2(a, b) a##b

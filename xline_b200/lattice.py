@@ -19,19 +19,24 @@ import numpy as np
 from scipy.constants import c as clight
 from scipy.constants import e as qe
 from scipy.constants import epsilon_0
+from scipy.constants import alpha as fine_structure
+from scipy.constants import hbar
 
 from . import elements as E
 
 T_END_TURN, T_END_CHUNK, T_DRIFT, T_DRIFT_EXACT, T_MULTIPOLE, T_MULTIPOLE_CURVED = range(6)
 T_CAVITY, T_RFMULTIPOLE, T_XYSHIFT, T_SROTATION, T_DIPOLE_EDGE = range(6, 11)
 T_LIMIT_RECT, T_LIMIT_ELLIPSE, T_LIMIT_RECT_ELLIPSE, T_MONITOR, T_SAWTOOTH_CAVITY = range(11, 16)
-T_BEAMBEAM4D, T_SPACECHARGE, T_BEAMBEAM6D, T_LIMIT_POLYGON = 16, 17, 18, 19
+T_BEAMBEAM4D, T_SPACECHARGE, T_BEAMBEAM6D, T_LIMIT_POLYGON, T_MULTIPOLE_RAD = 16, 17, 18, 19, 20
 
 F_STRICT = 1
 F_BEAMFIELDS = 2
 F_BB6D = 4
 F_LOW_ORDER = 8  # every multipole-family record has order <= LOW_ORDER_MAX (straight-line Horner kernels)
 F_POLYGONS = 16  # the lattice holds LIMIT_POLYGON records (only the kernels that carry the case run it)
+F_RADIATION = 32  # the lattice holds MULTIPOLE_RAD records (only the kernels that carry the case run it)
+RADIATION_MODES = {"mean": 1, "quantum": 2}
+RAD_MAX_ELEMENTS = 1 << 24
 LOW_ORDER_MAX = 3
 
 DEFAULT_CHUNK_WORDS = 2048  # 16 KiB per TMA bulk copy, 3 in flight per CTA
@@ -312,6 +317,38 @@ def _pack_limit_polygon(el, idx):
     return rec
 
 
+def radiation_constants():
+    """(K_e = e^2/(4 pi eps0), hbar c) in eV m and the fine-structure constant, from scipy.constants."""
+    return qe / (4.0 * math.pi * epsilon_0), hbar * clight / qe, fine_structure
+
+
+def check_radiation(radiation, radiation_seed):
+    """The radiation options: None, "mean" or "quantum", and a seed in [0, 2^64)."""
+    if radiation is not None and radiation not in RADIATION_MODES:
+        raise ValueError("radiation must be None, 'mean' or 'quantum' (got %r)" % (radiation,))
+    if not (isinstance(radiation_seed, (int, np.integer)) and 0 <= int(radiation_seed) < (1 << 64)):
+        raise ValueError("radiation_seed must be an integer in [0, 2^64) (got %r)" % (radiation_seed,))
+
+
+def radiates(el, radiation):
+    """Does ``el`` radiate when the line is tracked with ``radiation``: a Multipole with length > 0."""
+    return radiation is not None and type(el).__name__ == "Multipole" and float(el.length) > 0
+
+
+def _pack_multipole_rad(el, idx, radiation, seed):
+    """XLB_T_MULTIPOLE_RAD: [hdr,mode][L,1/L][K_e,hbar_c][alpha,seed] then the element's own
+    (fast-encoding) MULTIPOLE / MULTIPOLE_CURVED record, header word included."""
+    plain = _pack_element(el, idx, False, None)
+    length = float(el.length)
+    ke, hbarc, alpha = radiation_constants()
+    rec = _Rec(T_MULTIPOLE_RAD, plain.aux, idx)
+    rec.w[1] = _i2u(RADIATION_MODES[radiation])
+    rec.f(length, 1.0 / length).f(ke, hbarc).f(alpha)
+    rec.w.append(np.uint64(int(seed)))
+    rec.w.extend(plain.words())
+    return rec
+
+
 def _pack_element(el, idx, strict, monitors, polygons=False):
     name = type(el).__name__
     if name == "Drift":
@@ -557,9 +594,9 @@ def _pack_merged_block(k1, idx1, a1, k2, idx2, a2, drift):
     return rec.path_length_here()
 
 
-def _try_merge(live, pos):
+def _try_merge(live, pos, radiation=None):
     """Match [K1 straight, low order][LimitEllipse?][K2][LimitRect|LimitEllipse?][Drift?]
-    starting at live[pos]; returns (record, new_pos) or None."""
+    starting at live[pos]; returns (record, new_pos) or None.  Radiating multipoles do not merge."""
     def kind(i):
         return type(live[i][1]).__name__ if i < len(live) else None
 
@@ -571,7 +608,7 @@ def _try_merge(live, pos):
     if kind(i) == "LimitEllipse":
         a1 = live[i]
         i += 1
-    if kind(i) != "Multipole":
+    if kind(i) != "Multipole" or radiates(live[i][1], radiation):
         return None
     idx2, k2 = live[i]
     i += 1
@@ -590,7 +627,7 @@ SEG_MAIN, SEG_BB6D = 0, 1
 
 
 def pack_line(elements, strict=False, chunk_words=DEFAULT_CHUNK_WORDS, drop_noops=True, fuse=True,
-              merge=True, split_lenses=True, hx_only=True, polygons=False):
+              merge=True, split_lenses=True, hx_only=True, polygons=False, radiation=None, radiation_seed=0):
     """Pack ``elements`` (the ``Line.elements`` list).  ``element_index`` in every record
     is the position in that list, so ``at_element`` matches the reference's indexing even
     though exact no-ops (zero-length drifts, all-zero multipoles, disabled lenses) are not
@@ -607,8 +644,19 @@ def pack_line(elements, strict=False, chunk_words=DEFAULT_CHUNK_WORDS, drop_noop
 
     ``polygons``: pack ``LimitPolygon`` apertures as XLB_T_LIMIT_POLYGON records (the project's
     own definition, see include/xline_b200.h).  ``False``, the default, refuses them with
-    ``NotImplementedError`` like the reference's ``LimitPolygon.track``."""
+    ``NotImplementedError`` like the reference's ``LimitPolygon.track``.
+
+    ``radiation`` (None, "mean" or "quantum") and ``radiation_seed``: synchrotron radiation in every
+    Multipole of length > 0, packed as XLB_T_MULTIPOLE_RAD records that never enter a block
+    (include/xline_b200.h, DESIGN.md §4.9).  Fast encoding, one-species thin-lens lattices only:
+    ``ValueError`` for ``strict=True``, beam-field elements, or more than 2^24 elements."""
     assert chunk_words % 2 == 0 and chunk_words >= 16
+    check_radiation(radiation, radiation_seed)
+    if radiation is not None:
+        if strict:
+            raise ValueError("radiation: the strict encoding has no radiating multipoles (set radiation=None)")
+        if len(elements) > RAD_MAX_ELEMENTS:
+            raise ValueError("radiation: lines of more than 2^24 elements are not supported")
     monitors = dict(layout=[], words=0)
     recs = []
     flags = F_STRICT if strict else 0
@@ -661,8 +709,12 @@ def pack_line(elements, strict=False, chunk_words=DEFAULT_CHUNK_WORDS, drop_noop
             counts[rec.tag] = counts.get(rec.tag, 0) + 1
             recs.append((rec.tag, rec.words(), rec.s_word, rec.drift_len, rec.drift_before))
             continue
-        merged = _try_merge(live, pos - 1) if (fuse and merge and not strict and name == "Multipole") else None
-        if merged is not None:
+        rad = radiates(el, radiation)
+        merged = (_try_merge(live, pos - 1, radiation) if (fuse and merge and not strict and name == "Multipole"
+                                                            and not rad) else None)
+        if rad:
+            rec = _pack_multipole_rad(el, idx, radiation, radiation_seed)
+        elif merged is not None:
             # two co-located thin multipoles (apertures in between allowed): one summed kick
             rec, pos = merged
         elif fuse and name == "Multipole":
@@ -690,8 +742,13 @@ def pack_line(elements, strict=False, chunk_words=DEFAULT_CHUNK_WORDS, drop_noop
             flags |= F_BEAMFIELDS
         if tag == T_LIMIT_POLYGON:
             flags |= F_POLYGONS
+        if tag == T_MULTIPOLE_RAD:
+            flags |= F_RADIATION
+    if (flags & F_RADIATION) and (flags & (F_BEAMFIELDS | F_BB6D)):
+        raise ValueError("radiation: lines with beam-beam or space-charge elements are not supported "
+                         "(set radiation=None)")
     horner_orders = [(int(r[0]) >> 8) & 0xFF for tag, r, _, _, _ in recs
-                     if tag in (T_MULTIPOLE, T_MULTIPOLE_CURVED) or (tag & 0xC0) == T_THIN_BLOCK]
+                     if tag in (T_MULTIPOLE, T_MULTIPOLE_CURVED, T_MULTIPOLE_RAD) or (tag & 0xC0) == T_THIN_BLOCK]
     if all(o <= LOW_ORDER_MAX for o in horner_orders):
         flags |= F_LOW_ORDER
     biggest = max([len(r[1]) for r in recs] + [0])
@@ -751,13 +808,23 @@ def element_specs(elements):
     return out
 
 
-def algorithmic_ops(elements):
+RAD_OPS = {"mean": 74, "quantum": 82}  # per radiating multipole, photon sampling not counted
+
+
+def algorithmic_ops(elements, radiation=None):
     """FP64 operations per particle-turn by the SURVEY.md §8(a)/(d) convention (every
-    + - * / and **2 counts 1, each sqrt/sin/cos/exp 1, a wofz call taken as 100)."""
+    + - * / and **2 counts 1, each sqrt/sin/cos/exp 1, a wofz call taken as 100).  With
+    ``radiation``, every radiating multipole adds ``RAD_OPS[radiation]``: the field magnitude and
+    path length (8), and per half the particle's gamma, beta, kappa (9), the energy loss (mean: 9;
+    quantum: n̄, exp, the first Poisson step: 13), add_to_energy (13) and the px, py scaling (3).
+    The data-dependent rest of the quantum mode (further Poisson steps, ~23 per photon) is not
+    counted."""
     WOFZ = 100
     total = 0
     for el in elements:
         name = type(el).__name__
+        if radiates(el, radiation):
+            total += RAD_OPS[radiation]
         if name == "Drift":
             total += 15
         elif name == "DriftExact":

@@ -13,7 +13,7 @@ import torch
 
 from . import _cabi
 from . import elements as E
-from .lattice import F_LOW_ORDER, MONITOR_FIELDS, algorithmic_ops, element_specs, pack_line
+from .lattice import F_LOW_ORDER, MONITOR_FIELDS, algorithmic_ops, check_radiation, element_specs, pack_line
 
 _thick = (E.Drift, E.DriftExact)
 deg2rad = np.pi / 180.0
@@ -44,7 +44,7 @@ def _c_particles(p):
 class Line(E.Element):
     _base = (("elements", tuple), ("element_names", tuple))
     _pack_options = ("fuse_records", "chunk_words", "merge_multipoles", "split_lenses", "flag_horizontal_bends",
-                     "polygon_apertures")
+                     "polygon_apertures", "radiation", "radiation_seed")
 
     def __setattr__(self, name, value):
         # edit tracking (elements.py): the element list and the packing options stamp the line,
@@ -71,6 +71,10 @@ class Line(E.Element):
         # track LimitPolygon apertures with the project's even-odd rule (include/xline_b200.h); off,
         # a line that holds one refuses to pack, like the reference's LimitPolygon.track
         self.polygon_apertures = False
+        # synchrotron radiation in every Multipole of length > 0: None (off), "mean" or "quantum", and
+        # the seed of its counter-based random stream (include/xline_b200.h, DESIGN.md §4.9)
+        self.radiation = None
+        self.radiation_seed = 0
         self._monitor_buf = None
         self._buffers_key = None
         self.loss_tally = None
@@ -286,7 +290,7 @@ class Line(E.Element):
         return element_specs(self.elements)
 
     def algorithmic_ops_per_turn(self):
-        return algorithmic_ops(self.elements)
+        return algorithmic_ops(self.elements, self.radiation)
 
     def _content_stamp(self):
         """(ids of the elements, newest edit stamp among them and the line): changes whenever the
@@ -318,7 +322,8 @@ class Line(E.Element):
             chunk_words = self.chunk_words
         self._current_stamp()
         key = ("host", bool(strict), chunk_words, self.fuse_records, self.merge_multipoles, self.split_lenses,
-               self.flag_horizontal_bends, self.polygon_apertures, getattr(self, "_keep_noops", False))
+               self.flag_horizontal_bends, self.polygon_apertures, self.radiation, self.radiation_seed,
+               getattr(self, "_keep_noops", False))
         hit = self._cache.get("host_%d" % strict)
         if hit is not None and hit[0] == key:
             return hit[1]
@@ -326,6 +331,7 @@ class Line(E.Element):
         packed = pack_line(self.elements, strict=strict, fuse=self.fuse_records,
                            merge=self.merge_multipoles, split_lenses=self.split_lenses,
                            hx_only=self.flag_horizontal_bends, polygons=self.polygon_apertures,
+                           radiation=self.radiation, radiation_seed=self.radiation_seed,
                            drop_noops=not getattr(self, "_keep_noops", False), **kw)
         lat = packed.c_lattice()
         _cabi.check(_cabi.lib().xlb_lattice_validate(C.byref(lat)))
@@ -361,6 +367,10 @@ class Line(E.Element):
             raise RuntimeError(
                 "xline_b200.Line.track needs particles resident on a CUDA device (got %s); "
                 "there is no CPU tracking path in this package" % p.device)
+        if self.radiation is not None:
+            check_radiation(self.radiation, self.radiation_seed)
+            if strict:
+                raise ValueError("radiation: strict=True has no radiating kernel (set Line.radiation = None)")
         lib = _cabi.lib()
         dev = p.x.device  # the tensors' own (indexed) device: torch.device("cuda") != torch.device("cuda:0")
         with torch.cuda.device(dev):
@@ -385,6 +395,8 @@ class Line(E.Element):
                     p._chi_key, p._chi_trivial = ckey, bool((chi == 1.0).all())
                 if p._chi_trivial and not _general_kernels:
                     cp.chi = None
+                elif self.radiation is not None:
+                    raise ValueError("radiation: one species only -- every chi must be 1 (set Line.radiation = None)")
             # tallies and monitor storage belong to one state of the line on one device: a line that
             # was edited since (other element count, other monitor layout) gets fresh ones
             bkey = (self._cache.get("generation"), packed.n_elements, packed.monitor_words, dev)
@@ -520,8 +532,9 @@ class Line(E.Element):
             solo = self._cache.get(("solo", i))
             if solo is None or solo.elements[0] is not el:
                 solo = self._cache[("solo", i)] = Line([el], ["e"])
-            if solo.polygon_apertures != self.polygon_apertures:
-                solo.polygon_apertures = self.polygon_apertures
+            for opt in ("polygon_apertures", "radiation", "radiation_seed"):
+                if getattr(solo, opt) != getattr(self, opt):
+                    setattr(solo, opt, getattr(self, opt))
             solo.track(p, _count_turns=False, _element_offset=i)
             out.append(p.copy())
         if end:

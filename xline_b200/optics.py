@@ -150,3 +150,59 @@ def match_tunes(build_line, knobs, qx, qy, tol=1e-10, max_iter=20, step=1e-5):
     else:
         raise ValueError("tune matching did not converge")
     return float(k[0]), float(k[1])
+
+
+def radiation_integrals(line, p0c, mass0, q0=1.0):
+    """Synchrotron radiation integrals of the thin-lens map that ``Line.radiation`` tracks
+    (include/xline_b200.h, DESIGN.md §4.9), from ``twiss``: what to expect of energy loss, damping
+    and the equilibrium beam.  Energies in eV, ``p0c`` and ``mass0`` too.
+
+    Per radiating multipole i (a Multipole of length L_i > 0), with k_i = k0l_i / L_i (curvature of
+    the design orbit; kappa_i = |k_i|), h_i = hxl_i / L_i, and D (dispersion), H = gamma D^2 +
+    2 alpha D D' + beta D'^2 (horizontal) at the element -- the mean of its entrance and exit values,
+    as the two radiating halves sit on either side of the kick:
+      I2 = sum kappa^2 L,  I3 = sum kappa^3 L,  I4 = sum D (h kappa^2 L + 2 k k1l),  I5 = sum H kappa^3 L.
+    I4 follows from the map to first order in x = D delta: the path length of a half grows by
+    hxl x / 2 and kappa^2 by 2 k k1l x / L^2 (for k0l >= 0, k = kappa: the textbook form).  I1 =
+    sum D hxl over all curved multipoles (the momentum compaction times the length).  Then, with
+    C_gamma-free constants K_e = e^2/(4 pi eps0) and hbar c in eV m:
+      U0 = (2/3) q0^2 K_e beta^3 gamma^4 I2  (the mean mode's loss per turn on the design orbit);
+      J_x = 1 - I4/I2, J_y = 1, J_z = 2 + I4/I2;  tau_u = 2 E / (J_u U0) turns;
+      eps_x = C_q gamma^2 I5 / (J_x I2),  sigma_delta^2 = C_q gamma^2 I3 / (J_z I2),
+      C_q = 55 hbar c / (32 sqrt(3) m)  (from <x^2> = 11/27 and the photon rate of the quantum mode).
+    Returns a dict of those (``I1`` .. ``I5``, ``U0``, ``Jx Jy Jz``, ``tau_x tau_y tau_z``,
+    ``eps_x``, ``sigma_delta``, ``gamma``, ``energy``)."""
+    from .lattice import radiation_constants
+
+    ke, hbarc, _ = radiation_constants()
+    tw = twiss(line)
+    energy = math.sqrt(p0c * p0c + mass0 * mass0)
+    gamma, beta = energy / mass0, p0c / energy
+    i1 = i2 = i3 = i4 = i5 = 0.0
+
+    def curly_h(k):
+        b, a, d, dp = tw["betx"][k], tw["alfx"][k], tw["dx"][k], tw["dpx"][k]
+        return ((1 + a * a) / b) * d * d + 2 * a * d * dp + b * dp * dp
+
+    for i, el in enumerate(line.elements):
+        if isinstance(el, E.Multipole) and (el.hxl or el.hyl):
+            i1 += el.hxl * tw["dx"][i]
+        if not (isinstance(el, E.Multipole) and float(el.length) > 0):
+            continue
+        length = float(el.length)
+        knl = list(el.knl) + [0.0, 0.0]
+        k = knl[0] / length
+        kap = abs(k)
+        h = float(el.hxl) / length
+        d = tw["dx"][i]
+        i2 += kap * kap * length
+        i3 += kap ** 3 * length
+        i4 += d * (h * kap * kap * length + 2 * k * knl[1])
+        i5 += 0.5 * (curly_h(i) + curly_h(i + 1)) * kap ** 3 * length
+    u0 = (2.0 / 3.0) * q0 * q0 * ke * beta ** 3 * gamma ** 4 * i2
+    jx, jy, jz = 1 - i4 / i2, 1.0, 2 + i4 / i2
+    cq = 55.0 * hbarc / (32.0 * math.sqrt(3.0) * mass0)
+    return dict(I1=i1, I2=i2, I3=i3, I4=i4, I5=i5, U0=u0, Jx=jx, Jy=jy, Jz=jz,
+                tau_x=2 * energy / (jx * u0), tau_y=2 * energy / (jy * u0), tau_z=2 * energy / (jz * u0),
+                eps_x=cq * gamma ** 2 * i5 / (jx * i2), sigma_delta=math.sqrt(cq * gamma ** 2 * i3 / (jz * i2)),
+                gamma=gamma, energy=energy)

@@ -74,6 +74,7 @@ def track_tangent(line, p, tangent, num_turns=1, threads_per_block=0):
     if p.device.type != "cuda":
         raise RuntimeError("track_tangent needs particles resident on a CUDA device (got %s)" % p.device)
     tangent._check_target(p)
+    _refuse_radiation(line, "track_tangent")
     lib = _cabi.lib()
     dev = p.x.device
     with torch.cuda.device(dev):
@@ -106,6 +107,11 @@ one-turn matrix of the tracked map at ``z``; ``iterations``: Newton steps taken;
 largest |M(z) - z| over the solved coordinates at ``z``."""
 
 
+def _refuse_radiation(line, what):
+    if getattr(line, "radiation", None) is not None:
+        raise ValueError("%s: radiation is not part of the tangent map yet (set Line.radiation = None)" % what)
+
+
 def has_rf(line):
     """True when the line holds an RF element with a voltage (a longitudinal restoring force)."""
     return any(isinstance(el, (E.Cavity, E.SawtoothCavity, E.RFMultipole)) and float(el.voltage) != 0.0
@@ -125,6 +131,7 @@ def closed_orbit(line, particles_like, guess=None, mode="auto", tol=1e-14, max_i
     came within 1e3 ``tol``).  Returns a ``ClosedOrbit``.  Raises ``ValueError`` when the
     particle is lost, when ``M - I`` is singular (no isolated fixed point) or when the iteration
     does not converge within ``max_iter`` steps."""
+    _refuse_radiation(line, "closed_orbit")
     if mode == "auto":
         mode = "6d" if has_rf(line) else "4d"
     if mode not in ("4d", "6d"):
