@@ -47,11 +47,24 @@ def rel_err(a, b):
     return float(np.max(r)) if r.size else 0.0
 
 
+def _finite_pairs(a, b):
+    """The mask of entries finite on both sides, or None when the two finite masks differ."""
+    fa, fb = np.broadcast_arrays(np.isfinite(a), np.isfinite(b))
+    if not np.array_equal(fa, fb):
+        return None
+    return fa
+
+
 def scaled_err(a, b):
-    """max |a-b| / rms(b): error relative to the beam scale of the coordinate."""
+    """max |a-b| / rms(b): error relative to the beam scale of the coordinate.  Entries that are
+    non-finite on both sides are skipped; an entry non-finite on one side only is an infinite
+    error."""
     a = np.asarray(a, dtype=np.float64)
     b = np.asarray(b, dtype=np.float64)
-    ok = np.isfinite(a) & np.isfinite(b)
+    ok = _finite_pairs(a, b)
+    if ok is None:
+        return float("inf")
+    a, b = np.broadcast_arrays(a, b)
     if not ok.any():
         return 0.0
     scale = np.sqrt(np.mean(b[ok] ** 2))
@@ -63,10 +76,14 @@ def scaled_err(a, b):
 def floor_rel_err(a, b, floor=1e-3):
     """max |a-b| / max(|a|, |b|, floor * rms(b)): elementwise relative error with the
     denominator floored at ``floor`` x the beam's r.m.s. of that coordinate, so that values
-    passing through zero are judged against the coordinate's scale, not against themselves."""
+    passing through zero are judged against the coordinate's scale, not against themselves.
+    Non-finite entries as in ``scaled_err``."""
     a = np.asarray(a, dtype=np.float64)
     b = np.asarray(b, dtype=np.float64)
-    ok = np.isfinite(a) & np.isfinite(b)
+    ok = _finite_pairs(a, b)
+    if ok is None:
+        return float("inf")
+    a, b = np.broadcast_arrays(a, b)
     if not ok.any():
         return 0.0
     rms = np.sqrt(np.mean(b[ok] ** 2))

@@ -474,7 +474,7 @@ def test_reference_api_semantics_on_device():
 
 # ------------------------------------------------------------------ beam-field elements
 BF_CASES = sorted(k for k, m in H.manifest().items() if m["type"] in BEAMFIELD_TYPES)
-BF_TOL = 1e-12  # relative to the beam r.m.s. of each coordinate (Faddeeva: 4e-14 of |w|)
+BF_TOL = 1e-12  # relative to the beam r.m.s. of each coordinate (per particle: test_gpu_beamfield_accuracy)
 
 
 @pytest.mark.parametrize("strict", [False, True])
