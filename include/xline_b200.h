@@ -460,6 +460,37 @@ int xlb_track_tangent_device(const xlb_lattice_t *lattice, xlb_particles_t *part
                              const xlb_track_options_t *opts, double *jac /*[n][6][6]*/, int64_t *log2_scale,
                              double *fli, void *stream);
 
+/* Tangent map with radiation (DESIGN.md §4.10): xlb_track_tangent_device, same contract, on a lattice
+ * that may also hold XLB_T_MULTIPOLE_RAD records -- every one of them in mean mode (a quantum record is
+ * XLB_EINVAL naming the element: the random map has no tangent).  The checks on a radiating lattice
+ * are those of xlb_track_device (one species, no beam fields, element indices < 2^24).  A mean-mode
+ * half with kappa == 0 is the identity; otherwise, with W = dE of the half (< 0) as a function of
+ * (x, y, delta) through fl^2 (never fl: smooth where the field vanishes) and l_h:
+ *   J <- J_h J,  J_h = d(add_to_energy(W), then px, py times (1+delta')/(1+delta)) / dz,
+ * so the half is a row update of the delta, zeta, px and py rows.  A lattice without radiating
+ * records gives the results of xlb_track_tangent_device bit for bit.                            */
+int xlb_track_tangent_radiation_device(const xlb_lattice_t *lattice, xlb_particles_t *particles,
+                                       const xlb_track_options_t *opts, double *jac /*[n][6][6]*/,
+                                       int64_t *log2_scale, double *fli, void *stream);
+
+/* Beam envelope (DESIGN.md §4.10): particles tracked as xlb_track_tangent_radiation_device tracks
+ * them (same lattice checks, options, losses and reproducibility), each carrying a 6x6 second moment
+ * Sigma (cov[i*36 + r*6 + c], row-major, symmetric, caller-initialised) and the energy it lost.
+ *   Every element: Sigma <- J_e Sigma J_e^T with J_e the element's Jacobian at the state before it.
+ *   Every radiating half (mean mode, kappa != 0) adds the variance of the quantum mode's loss in
+ *     that half linearised about the mean-mode orbit:  Sigma += V_h g g^T,
+ *     V_h = nbar (11/27) u_c^2 (eV^2; nbar, u_c as in the quantum map of XLB_T_MULTIPOLE_RAD, from the
+ *     record's K_e, hbar_c, alpha), g = dz_after/dW = (0, px' , 0, py', zeta', delta') of the half's
+ *     energy change;  and energy_loss[i] -= W (eV).
+ *   At the end of every turn of a surviving particle Sigma <- (Sigma + Sigma^T)/2.
+ * A lost particle's Sigma and energy_loss are written where it was lost.  On a lattice without
+ * radiating records Sigma is transported without diffusion: J Sigma0 J^T of the same particle's
+ * tangent map.  XLB_EINVAL for the refusals of the tangent map and a null cov / energy_loss with
+ * n > 0.                                                                                          */
+int xlb_track_envelope_device(const xlb_lattice_t *lattice, xlb_particles_t *particles,
+                              const xlb_track_options_t *opts, double *cov /*[n][6][6]*/,
+                              double *energy_loss /*[n]*/, void *stream);
+
 /* Register-resident independent-DFMA-chain microbenchmark: the measured FP64 pipe peak of
  * the current device in FLOP/s (2 flops per DFMA), best of `repeats`.  The roofline
  * denominator of bench.py (MEASURED_PEAKS.json has no FP64 entry). */

@@ -11,11 +11,12 @@ from .elements import *  # noqa: F401,F403
 from .line import Line
 from .moments import BeamMoments, beam_moments
 from .particles import Particles
-from .tangent import ClosedOrbit, TangentMap, closed_orbit
+from .tangent import (ClosedOrbit, Envelope, RadiationEquilibrium, TangentMap, closed_orbit,
+                      radiation_equilibrium)
 from .tunes import monitor_tunes, naff
 
 XlineTestParticles = Particles  # the reference's name (xline/particles.py:4)
 
 __all__ = list(elements.__all__) + ["Line", "Particles", "XlineTestParticles", "elements", "BeamMoments",
                                     "beam_moments", "naff", "monitor_tunes", "TangentMap", "closed_orbit",
-                                    "ClosedOrbit"]
+                                    "ClosedOrbit", "Envelope", "radiation_equilibrium", "RadiationEquilibrium"]

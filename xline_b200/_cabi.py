@@ -25,6 +25,7 @@ EXPORTS = (
     "xlb_measure_fp64_peak", "xlb_measure_dfma_latency", "xlb_kernel_variant_count",
     "xlb_kernel_variant_info", "xlb_selftest_exact_division", "xlb_beam_moments_device",
     "xlb_track_device_moments", "xlb_naff_device", "xlb_track_tangent_device",
+    "xlb_track_tangent_radiation_device", "xlb_track_envelope_device",
 )
 
 
@@ -102,6 +103,11 @@ def lib():
     L.xlb_track_tangent_device.argtypes = [C.POINTER(Lattice), C.POINTER(Particles), C.POINTER(TrackOptions),
                                            C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.xlb_track_tangent_device.restype = C.c_int
+    L.xlb_track_tangent_radiation_device.argtypes = L.xlb_track_tangent_device.argtypes
+    L.xlb_track_tangent_radiation_device.restype = C.c_int
+    L.xlb_track_envelope_device.argtypes = [C.POINTER(Lattice), C.POINTER(Particles), C.POINTER(TrackOptions),
+                                            C.c_void_p, C.c_void_p, C.c_void_p]
+    L.xlb_track_envelope_device.restype = C.c_int
     L.xlb_track_host.argtypes = [C.POINTER(Lattice), C.POINTER(Particles), C.POINTER(TrackOptions)]
     L.xlb_track_host.restype = C.c_int
     L.xlb_get_stats.argtypes = [C.POINTER(TrackStats)]

@@ -940,27 +940,40 @@ int xlb_naff_device(const double *u, const double *pu, int64_t n, int64_t num_tu
   return XLB_OK;
 }
 
-int xlb_track_tangent_device(const xlb_lattice_t *lat, xlb_particles_t *p, const xlb_track_options_t *o,
-                             double *jac, int64_t *log2_scale, double *fli, void *stream) {
-  memset(&g_stats, 0, sizeof(g_stats));
+// The argument checks of the tangent-map entry points (`what` names the call in messages).
+// `radiation`: mean-mode radiating multipoles are allowed.
+static int tangent_checks(const xlb_lattice_t *lat, xlb_particles_t *p, const xlb_track_options_t *o, bool radiation,
+                          const char *what, int *threads) {
   int rc;
   if ((rc = check_call(lat, p, o, nullptr)) != XLB_OK) return rc;
-  if (o->trace) return fail(XLB_EINVAL, "tangent tracking does not combine with a trace");
-  if (lat->flags & XLB_F_RADIATION)
+  char buf[160];
+  if (o->trace) {
+    snprintf(buf, sizeof buf, "%s does not combine with a trace", what);
+    return fail(XLB_EINVAL, buf);
+  }
+  if (!radiation && (lat->flags & XLB_F_RADIATION))
     return fail(XLB_EINVAL, "tangent tracking: radiating multipoles are not in the tangent map");
-  if (lat->flags & XLB_F_STRICT) return fail(XLB_EINVAL, "tangent tracking needs a lattice in the fast encoding");
-  if (lat->n_segments > 0) return fail(XLB_EINVAL, "tangent tracking needs an unsegmented lattice");
-  if (o->particles_per_thread != 0 && o->particles_per_thread != 1)
-    return fail(XLB_EINVAL, "tangent tracking runs one particle per thread");
-  const int threads = o->threads_per_block > 0 ? o->threads_per_block : 128;
-  if (threads % 32 || threads > XLB_TANGENT_MAX_THREADS)
+  if (lat->flags & XLB_F_STRICT) {
+    snprintf(buf, sizeof buf, "%s needs a lattice in the fast encoding", what);
+    return fail(XLB_EINVAL, buf);
+  }
+  if (lat->n_segments > 0) {
+    snprintf(buf, sizeof buf, "%s needs an unsegmented lattice", what);
+    return fail(XLB_EINVAL, buf);
+  }
+  if (o->particles_per_thread != 0 && o->particles_per_thread != 1) {
+    snprintf(buf, sizeof buf, "%s runs one particle per thread", what);
+    return fail(XLB_EINVAL, buf);
+  }
+  *threads = o->threads_per_block > 0 ? o->threads_per_block : 128;
+  if (*threads % 32 || *threads > XLB_TANGENT_MAX_THREADS)
     return fail(XLB_EINVAL, "threads_per_block must be a multiple of 32 and <= XLB_TANGENT_MAX_THREADS");
-  if (p->n == 0 || o->num_turns == 0) return XLB_OK;
-  if (!jac || !log2_scale || !fli) return fail(XLB_EINVAL, "jac, log2_scale and fli must not be null");
-  const cudaStream_t st = static_cast<cudaStream_t>(stream);
-  CallScope call;
-  if ((rc = call.open(st)) != XLB_OK) return rc;
-  // The kernel knows one record per element: refuse the block records and the 6D lens up front.
+  return XLB_OK;
+}
+
+// The kernels know one record per element: refuse the block records and the 6D lens (and, with
+// radiation, quantum-mode radiating multipoles) up front, naming the element.
+static int tangent_scan(const xlb_lattice_t *lat, bool radiation, const char *what, cudaStream_t st) {
   std::vector<uint64_t> w(static_cast<size_t>(lat->n_words));
   XLB_CUDA(cudaMemcpyAsync(w.data(), lat->words, w.size() * 8, cudaMemcpyDefault, st));
   XLB_CUDA(cudaStreamSynchronize(st));
@@ -971,22 +984,77 @@ int xlb_track_tangent_device(const xlb_lattice_t *lat, xlb_particles_t *p, const
       if (tag == XLB_T_END_TURN || tag == XLB_T_END_CHUNK) break;
       if (tag == XLB_T_BEAMBEAM6D || tag >= XLB_T__COUNT) {
         char buf[160];
-        snprintf(buf, sizeof buf, "tangent tracking: element %d is %s", static_cast<int>(hdr >> 32),
+        snprintf(buf, sizeof buf, "%s: element %d is %s", what, static_cast<int>(hdr >> 32),
                  tag == XLB_T_BEAMBEAM6D ? "a BeamBeam6D lens (its Jacobian is not implemented)"
                                          : "a fused block record (pack one record per element)");
+        return fail(XLB_EINVAL, buf);
+      }
+      if (radiation && tag == XLB_T_MULTIPOLE_RAD && static_cast<int64_t>(w[pos + 1]) != XLB_RAD_MEAN) {
+        char buf[160];
+        snprintf(buf, sizeof buf, "%s: element %d radiates in quantum mode (the tangent map and the envelope "
+                 "take mean-mode records)", what, static_cast<int>(hdr >> 32));
         return fail(XLB_EINVAL, buf);
       }
       if (pairs < 1) return fail(XLB_ELATTICE, "record of size 0");
       pos += 2 * static_cast<size_t>(pairs);
     }
   }
-  KArgs a = kernel_args(lat, p, o, call.s->n_lost);
-  a.num_turns = o->num_turns;
-  XLB_CUDA(tangent_launch(a, jac, reinterpret_cast<long long *>(log2_scale), fli, threads, st));
+  return XLB_OK;
+}
+
+static void tangent_stats(const xlb_particles_t *p, int threads) {
   g_stats.kernel_launches = 1;
   g_stats.threads = threads;
   g_stats.blocks = static_cast<int>((p->n + threads - 1) / threads);
   g_stats.n_alive_in = p->n;
+}
+
+static int track_tangent_impl(const xlb_lattice_t *lat, xlb_particles_t *p, const xlb_track_options_t *o,
+                              double *jac, int64_t *log2_scale, double *fli, void *stream, bool radiation) {
+  memset(&g_stats, 0, sizeof(g_stats));
+  int rc, threads;
+  if ((rc = tangent_checks(lat, p, o, radiation, "tangent tracking", &threads)) != XLB_OK) return rc;
+  if (p->n == 0 || o->num_turns == 0) return XLB_OK;
+  if (!jac || !log2_scale || !fli) return fail(XLB_EINVAL, "jac, log2_scale and fli must not be null");
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  CallScope call;
+  if ((rc = call.open(st)) != XLB_OK) return rc;
+  if ((rc = tangent_scan(lat, radiation, "tangent tracking", st)) != XLB_OK) return rc;
+  KArgs a = kernel_args(lat, p, o, call.s->n_lost);
+  a.num_turns = o->num_turns;
+  if (radiation)
+    XLB_CUDA(tangent_radiation_launch(a, jac, reinterpret_cast<long long *>(log2_scale), fli, threads, st));
+  else
+    XLB_CUDA(tangent_launch(a, jac, reinterpret_cast<long long *>(log2_scale), fli, threads, st));
+  tangent_stats(p, threads);
+  return XLB_OK;
+}
+
+int xlb_track_tangent_device(const xlb_lattice_t *lat, xlb_particles_t *p, const xlb_track_options_t *o,
+                             double *jac, int64_t *log2_scale, double *fli, void *stream) {
+  return track_tangent_impl(lat, p, o, jac, log2_scale, fli, stream, false);
+}
+
+int xlb_track_tangent_radiation_device(const xlb_lattice_t *lat, xlb_particles_t *p, const xlb_track_options_t *o,
+                                       double *jac, int64_t *log2_scale, double *fli, void *stream) {
+  return track_tangent_impl(lat, p, o, jac, log2_scale, fli, stream, true);
+}
+
+int xlb_track_envelope_device(const xlb_lattice_t *lat, xlb_particles_t *p, const xlb_track_options_t *o,
+                              double *cov, double *energy_loss, void *stream) {
+  memset(&g_stats, 0, sizeof(g_stats));
+  int rc, threads;
+  if ((rc = tangent_checks(lat, p, o, true, "envelope tracking", &threads)) != XLB_OK) return rc;
+  if (p->n == 0 || o->num_turns == 0) return XLB_OK;
+  if (!cov || !energy_loss) return fail(XLB_EINVAL, "cov and energy_loss must not be null");
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  CallScope call;
+  if ((rc = call.open(st)) != XLB_OK) return rc;
+  if ((rc = tangent_scan(lat, true, "envelope tracking", st)) != XLB_OK) return rc;
+  KArgs a = kernel_args(lat, p, o, call.s->n_lost);
+  a.num_turns = o->num_turns;
+  XLB_CUDA(envelope_launch(a, cov, energy_loss, threads, st));
+  tangent_stats(p, threads);
   return XLB_OK;
 }
 

@@ -77,6 +77,11 @@ cudaError_t naff_launch(const double *u, const double *pu, long long n, int num_
 // all a.num_turns turns in one launch; arguments checked by the caller.
 cudaError_t tangent_launch(const KArgs &a, double *jac, long long *log2_scale, double *fli, int threads,
                            cudaStream_t st);
+// The same with mean-mode radiating multipoles (tangent_kernel_radiation), and the envelope
+// Sigma <- J Sigma J^T + diffusion with the energy lost (envelope_kernel).
+cudaError_t tangent_radiation_launch(const KArgs &a, double *jac, long long *log2_scale, double *fli, int threads,
+                                     cudaStream_t st);
+cudaError_t envelope_launch(const KArgs &a, double *cov, double *energy_loss, int threads, cudaStream_t st);
 
 // variant tables, one per translation unit (kernel family)
 const Variant *fast_lean_variants(int *n);

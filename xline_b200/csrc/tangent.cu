@@ -26,6 +26,37 @@ namespace tangent {
 using Jac = double[6][6];
 enum { X = 0, PX = 1, Y = 2, PY = 3, ZETA = 4, DELTA = 5 };
 
+// What the kernel body carries (include/xline_b200.h, "Tangent map"):
+//   TANGENT   J, no radiating records (tangent_kernel);
+//   TANGENT_R J, with mean-mode MULTIPOLE_RAD records (tangent_kernel_radiation);
+//   ENVELOPE  Sigma <- J_e Sigma J_e^T per element, plus the quantum diffusion of every radiating half
+//             (envelope_kernel).
+enum { TANGENT = 0, TANGENT_R = 1, ENVELOPE = 2 };
+
+__device__ __forceinline__ void transpose(Jac &J) {
+#pragma unroll
+  for (int q = 0; q < 6; ++q)
+#pragma unroll
+    for (int c = q + 1; c < 6; ++c) {
+      const double t = J[q][c];
+      J[q][c] = J[c][q];
+      J[c][q] = t;
+    }
+}
+
+// Applies the row update F(A) = J_e A of an element, a statement on J that reads the state before
+// the element only: once to J, or as F(F(Sigma)^T) = J_e Sigma J_e^T to a symmetric Sigma (the
+// envelope).  A macro rather than a function taking a lambda: the tangent kernel compiles to the
+// same code as it did before the envelope existed.
+#define TAN_ROWS(...)         \
+  do {                        \
+    __VA_ARGS__;              \
+    if (MODE == ENVELOPE) {   \
+      transpose(J);           \
+      __VA_ARGS__;            \
+    }                         \
+  } while (0)
+
 // row r of J += a * row s
 __device__ __forceinline__ void axpy(Jac &J, int r, double a, int s) {
 #pragma unroll
@@ -152,6 +183,7 @@ __device__ __forceinline__ void jac_energy(Jac &J, const Regs<1> &r, double beta
 
 // CAVITY / SAWTOOTH_CAVITY (el_cavity; xline/elements.py:239-263).
 // J and the state (the tracker's el_cavity with sincos_ns for sin).
+template <int MODE>
 __device__ __forceinline__ void tan_cavity(Jac &J, const KArgs &a, Regs<1> &r, const double2 *rec,
                                            double V, bool sawtooth) {
   const double2 c = rec[1];  // k, lag_rad
@@ -173,7 +205,7 @@ __device__ __forceinline__ void tan_cavity(Jac &J, const KArgs &a, Regs<1> &r, c
   const double gz = C * dw * (-c.x / (r.rvv[0] * a.beta0));
   const double gd = C * dw * (c.x * r.zeta[0] * rv1 / (r.rvv[0] * r.rvv[0] * a.beta0));
   const double none[4] = {0.0, 0.0, 0.0, 0.0};
-  jac_energy(J, r, a.beta0, a.energy0, C * w, 0.0, 0.0, gz, gd, none, none);
+  TAN_ROWS(jac_energy(J, r, a.beta0, a.energy0, C * w, 0.0, 0.0, gz, gd, none, none));
   add_to_energy(C * w, a.beta0, a.energy0, r.delta[0], r.rpp[0], r.rvv[0], r.zeta[0]);
 }
 
@@ -183,6 +215,7 @@ __device__ __forceinline__ void tan_cavity(Jac &J, const KArgs &a, Regs<1> &r, c
 //   dptr = Re sum B_i Z_(i+1),       B_i = sn_i kn_i + i ss_i ks_i,
 // dZ_i/dx = Z_(i-1), dZ_i/dy = i Z_(i-1), dA_i/dktau = B_i, dB_i/dktau = -A_i.
 // J and the state (the tracker's el_rfmultipole with sincos_ns for sincos).
+template <int MODE>
 __device__ __forceinline__ void tan_rfmultipole(Jac &J, const KArgs &a, Regs<1> &r, const double2 *rec,
                                                 int order, double V) {
   const double2 c = rec[1];  // k, lag_rad
@@ -229,7 +262,7 @@ __device__ __forceinline__ void tan_rfmultipole(Jac &J, const KArgs &a, Regs<1> 
   const double W = C * (V * sl - a.p0c * c.x * dptr);
   const double dW_dktau = C * (-V * cl + a.p0c * c.x * ar);
   const double gx = -C * a.p0c * c.x * br, gy = C * a.p0c * c.x * bi;
-  jac_energy(J, r, a.beta0, a.energy0, W, gx, gy, dW_dktau * kz, dW_dktau * kd, kxv, kyv);
+  TAN_ROWS(jac_energy(J, r, a.beta0, a.energy0, W, gx, gy, dW_dktau * kz, dW_dktau * kd, kxv, kyv));
   r.px[0] = fma(-chi, dpx, r.px[0]);
   r.py[0] = fma(chi, dpy, r.py[0]);
   add_to_energy(W, a.beta0, a.energy0, r.delta[0], r.rpp[0], r.rvv[0], r.zeta[0]);
@@ -389,14 +422,134 @@ __device__ __forceinline__ void jac_spacecharge(Jac &J, const KArgs &a, const Re
   jac_field_kick(J, g * lam, g * dlz, g * dld, Ex, Ey, exx, exy, eyx, eyy);
 }
 
+template <int MODE>
 __device__ __forceinline__ void tan_drift(Jac &J, Regs<1> &r, double beta0, int aux, double L) {
   if (aux & XLB_AUX_DRIFT_EXACT) {
-    jac_drift_exact(J, r, beta0, L);
+    TAN_ROWS(jac_drift_exact(J, r, beta0, L));
     el_drift_exact<1>(r, L);
   } else {
-    jac_drift(J, r, beta0, L);
+    TAN_ROWS(jac_drift(J, r, beta0, L));
     el_drift<1>(r, L);
   }
+}
+
+// ---------------------------------------------------------------- mean-mode radiation
+// One radiating half of a MULTIPOLE_RAD record in mean mode (the tracker's radiate_half,
+// track_impl.cuh, restated: that function lives behind XLB_RADIATION, which would bring the
+// __constant__ photon table into this unit).  x and y do not change inside the element, so the
+// field size fl and the path length lh of both halves are functions of the state before it; the
+// caller passes fl^2's gradient (f2x, f2y) over (x, y).  With A = -(2/3) q0^2 K_e beta^3 gamma^4 / (L^2
+// (1+delta)^2) the loss is W = A fl^2 lh, whose gradient is taken through fl^2 (smooth where fl = 0,
+// unlike fl itself), and  d ln W / d delta = 1/(1+delta) + P p0c / E^2  (W ~ (1+delta) E).  Then
+// add_to_energy(W) through the chain of jac_energy, and px, py times f = (1+delta')/(1+delta):
+//   row(px) <- f row(px) + px (row(delta') - f row(delta)) / (1+delta),  the same for py.
+// ENVELOPE: Sigma += V_h g g^T with V_h = nbar (11/27) u_c^2, the variance of the quantum mode's
+// loss over the half (nbar, u_c of include/xline_b200.h), and g = dz_after/dW; `eloss` -= W.
+template <int MODE>
+__device__ __forceinline__ void tan_radiate_half(Jac &J, const KArgs &a, Regs<1> &r, const double2 *rec,
+                                                 double fl, double lh, double f2x, double f2y, double hxl,
+                                                 double hyl, double &eloss) {
+  const double2 len = rec[1], ke = rec[2], al = rec[3];  // [L,1/L][K_e,hbar_c][alpha,seed]
+  const double m2 = (a.energy0 - a.p0c) * (a.energy0 + a.p0c);
+  const double opd = 1.0 + r.delta[0];
+  const double P = opd * a.p0c;
+  const double E = sqrt(fma(P, P, m2));
+  const double gamma = E / sqrt(m2);
+  const double kappa = fl * len.y / opd;
+  const double q2 = a.q0 * a.q0;
+  if (kappa == 0.0) return;  // the particle untouched; fl = 0 makes fl^2's gradient 0 as well
+  const double beta = P / E;
+  const double g2 = gamma * gamma;
+  const double dE = -(2.0 / 3.0) * q2 * ke.x * (beta * beta * beta) * (g2 * g2) * (kappa * kappa) * lh;
+  // the gradient of dE over (x, y, delta)
+  const double il = len.y / opd;
+  const double A = -(2.0 / 3.0) * q2 * ke.x * (beta * beta * beta) * (g2 * g2) * (il * il);
+  const double fl2 = fl * fl;
+  const double gx = A * (f2x * lh + fl2 * (0.5 * hxl));
+  const double gy = A * (f2y * lh - fl2 * (0.5 * hyl));
+  const double gd = dE * (1.0 / opd + P * a.p0c / (E * E));
+  // the chain of add_to_energy (jac_energy) with the scaling of px, py
+  const double beta0 = a.beta0, energy0 = a.energy0;
+  const double delta = r.delta[0], rvv = r.rvv[0], zeta = r.zeta[0], px = r.px[0], py = r.py[0];
+  const double Eb = opd / rvv;
+  const double P1 = Eb + dE / energy0;
+  const double ptau = (P1 - 1.0) / beta0;
+  const double opdn = sqrt(ptau * ptau + 2.0 * ptau / beta0 + 1.0);
+  const double rvvn = opdn / P1;
+  const double dd_dP = P1 / (beta0 * beta0 * opdn);
+  const double drvv_dP = dd_dP / P1 - opdn / (P1 * P1);
+  const double rv1 = (1.0 - beta0 * beta0) / (Eb * Eb * Eb);
+  const double px_ = gx / energy0, py_ = gy / energy0;
+  const double pd_ = gd / energy0 + beta0 * beta0 * (1.0 + delta) / Eb;
+  const double zr = zeta / rvv;
+  const double f = opdn / opd, xo = px / opd, yo = py / opd;
+  TAN_ROWS(
+      _Pragma("unroll")
+      for (int c = 0; c < 6; ++c) {
+        const double jx = J[X][c], jy = J[Y][c], jz = J[ZETA][c], jd = J[DELTA][c];
+        const double dP = px_ * jx + py_ * jy + pd_ * jd;
+        const double jdn = dd_dP * dP;
+        J[DELTA][c] = jdn;
+        J[ZETA][c] = (rvvn / rvv) * jz + zr * drvv_dP * dP - zr * (rvvn / rvv) * rv1 * jd;
+        J[PX][c] = f * J[PX][c] + xo * (jdn - f * jd);
+        J[PY][c] = f * J[PY][c] + yo * (jdn - f * jd);
+      });
+  if (MODE == ENVELOPE) {
+    const double nbar = (5.0 / (2.0 * 1.7320508075688772)) * q2 * al.x * gamma * kappa * lh;
+    const double uc = 1.5 * ke.y * (gamma * g2) * kappa;
+    const double V = nbar * (11.0 / 27.0) * (uc * uc);
+    const double gdw = dd_dP / energy0;
+    const double g[6] = {0.0, xo * gdw, 0.0, yo * gdw, zr * drvv_dP / energy0, gdw};
+#pragma unroll
+    for (int q = 0; q < 6; ++q)
+#pragma unroll
+      for (int c = 0; c < 6; ++c) J[q][c] = fma(V * g[q], g[c], J[q][c]);
+    eloss -= dE;
+  }
+  add_to_energy(dE, a.beta0, a.energy0, r.delta[0], r.rpp[0], r.rvv[0], r.zeta[0]);
+  const double fs = (1.0 + r.delta[0]) / opd;
+  r.px[0] = r.px[0] * fs;
+  r.py[0] = r.py[0] * fs;
+}
+
+// MULTIPOLE_RAD in mean mode (el_multipole_rad): radiate, the embedded multipole, radiate.
+template <int MODE>
+__device__ __forceinline__ void tan_multipole_rad(Jac &J, const KArgs &a, Regs<1> &r, const double2 *rec,
+                                                  int order, double &eloss) {
+  const double2 len = rec[1];
+  const double2 *sub = rec + 4;
+  const bool curved = (*reinterpret_cast<const unsigned *>(sub) & 0xffu) == XLB_T_MULTIPOLE_CURVED;
+  const double hxl = curved ? sub[0].y : 0.0;
+  const double hyl = curved ? sub[1].x : 0.0;
+  const double2 *pairs = curved ? sub + 3 : sub + 1;
+  const double x = r.x[0], y = r.y[0];
+  double dpx[1], dpy[1];
+  horner<1>(r, pairs, order, dpx, dpy);  // the tracker's field kick, bit for bit
+  // P' = dr + i di from the Horner sweep of jac_multipole
+  double pr = pairs[0].x, pi = pairs[0].y, dr = 0.0, di = 0.0;
+  for (int m = 1; m <= order; ++m) {
+    const double2 k = pairs[m];
+    const double tr = fma(dr, x, fma(-di, y, pr)), ti = fma(dr, y, fma(di, x, pi));
+    dr = tr;
+    di = ti;
+    const double ur = fma(pr, x, fma(-pi, y, k.x)), ui = fma(pr, y, fma(pi, x, k.y));
+    pr = ur;
+    pi = ui;
+  }
+  // fl^2 = (Re P)^2 + (Im P)^2:  d/dx = 2 (Re P Re P' + Im P Im P'),  d/dy = 2 (Im P Re P' - Re P Im P')
+  const double f2x = 2.0 * (dpx[0] * dr + dpy[0] * di), f2y = 2.0 * (dpy[0] * dr - dpx[0] * di);
+  const double fl = sqrt(fma(dpx[0], dpx[0], dpy[0] * dpy[0]));
+  const double lh = 0.5 * fma(-hyl, y, fma(hxl, x, len.x));
+  if (r.alive(0)) tan_radiate_half<MODE>(J, a, r, rec, fl, lh, f2x, f2y, hxl, hyl, eloss);
+  if (curved) {
+    const double2 c1 = sub[1], c2 = sub[2];  // [hyl, length] [1/length, 0]
+    TAN_ROWS(jac_multipole(J, r, sub + 3, order, true, hxl, c1.x, c2.x));
+    el_multipole_curved<1>(r, sub, order, hxl);
+  } else {
+    TAN_ROWS(jac_multipole(J, r, sub + 1, order, false, 0.0, 0.0, 0.0));
+    el_multipole<1>(r, sub, order);
+  }
+  if (r.alive(0)) tan_radiate_half<MODE>(J, a, r, rec, fl, lh, f2x, f2y, hxl, hyl, eloss);
 }
 
 struct TArgs {
@@ -404,6 +557,12 @@ struct TArgs {
   double *jac;            // [n][6][6]
   long long *log2_scale;  // [n]
   double *fli;            // [n]
+};
+
+// envelope_kernel: t.jac is Sigma [n][6][6]; log2_scale and fli are not used
+struct EArgs {
+  TArgs t;
+  double *energy_loss;  // [n]
 };
 
 __device__ __forceinline__ void store_tangent(const TArgs &t, int i, const Jac &J, long long l2s, double fli) {
@@ -446,13 +605,42 @@ __device__ __forceinline__ void end_turn(Jac &J, long long &l2s, double &fli) {
   fli = fmax(fli, f);
 }
 
-__global__ void __launch_bounds__(256) tangent_kernel(const __grid_constant__ TArgs t) {
+// The envelope's store: Sigma and the energy lost.
+__device__ __forceinline__ void store_envelope(const TArgs &t, double *eloss, int i, const Jac &S, double el) {
+  double *o = t.jac + static_cast<long long>(i) * 36;
+#pragma unroll
+  for (int q = 0; q < 6; ++q)
+#pragma unroll
+    for (int c = 0; c < 6; ++c) o[q * 6 + c] = S[q][c];
+  eloss[i] = el;
+}
+
+template <int MODE>
+__device__ __forceinline__ void store(const TArgs &t, double *eloss, int i, const Jac &J, long long l2s, double fli,
+                                      double el) {
+  if (MODE == ENVELOPE)
+    store_envelope(t, eloss, i, J, el);
+  else
+    store_tangent(t, i, J, l2s, fli);
+}
+
+// End of an envelope turn: Sigma made exactly symmetric (F(F(Sigma)^T) is symmetric up to rounding).
+__device__ __forceinline__ void symmetrize(Jac &S) {
+#pragma unroll
+  for (int q = 0; q < 6; ++q)
+#pragma unroll
+    for (int c = q + 1; c < 6; ++c) S[q][c] = S[c][q] = 0.5 * (S[q][c] + S[c][q]);
+}
+
+template <int MODE>
+__device__ __forceinline__ void tangent_body(const TArgs &t, double *eloss) {
   const KArgs &a = t.k;
   const long long k = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   Regs<1> r;
   Jac J;
   long long l2s = 0;
   double fli = 0.0;
+  double el = 0.0;  // ENVELOPE: energy lost (eV)
   r.slot[0] = -1;
   if (k < a.n) {
     const int i = static_cast<int>(k);
@@ -472,8 +660,12 @@ __global__ void __launch_bounds__(256) tangent_kernel(const __grid_constant__ TA
       for (int q = 0; q < 6; ++q)
 #pragma unroll
         for (int c = 0; c < 6; ++c) J[q][c] = jin[q * 6 + c];
-      l2s = t.log2_scale[i];
-      fli = t.fli[i];
+      if (MODE == ENVELOPE) {
+        el = eloss[i];
+      } else {
+        l2s = t.log2_scale[i];
+        fli = t.fli[i];
+      }
     }
   }
   if (r.slot[0] < 0) {
@@ -509,29 +701,29 @@ __global__ void __launch_bounds__(256) tangent_kernel(const __grid_constant__ TA
       }
       switch (tag) {
         case XLB_T_DRIFT:
-          jac_drift(J, r, a.beta0, p0);
+          TAN_ROWS(jac_drift(J, r, a.beta0, p0));
           el_drift<1>(r, p0);
           break;
         case XLB_T_DRIFT_EXACT:
-          jac_drift_exact(J, r, a.beta0, p0);
+          TAN_ROWS(jac_drift_exact(J, r, a.beta0, p0));
           el_drift_exact<1>(r, p0);
           break;
         case XLB_T_MULTIPOLE:
-          jac_multipole(J, r, cur + 1, aux, false, 0.0, 0.0, 0.0);
+          TAN_ROWS(jac_multipole(J, r, cur + 1, aux, false, 0.0, 0.0, 0.0));
           el_multipole<1>(r, cur, aux);
           break;
         case XLB_T_MULTIPOLE_CURVED: {
           const double2 c1 = cur[1], c2 = cur[2];  // [hyl, length] [1/length, 0]
-          jac_multipole(J, r, cur + 3, aux, true, p0, c1.x, c2.x);
+          TAN_ROWS(jac_multipole(J, r, cur + 3, aux, true, p0, c1.x, c2.x));
           el_multipole_curved<1>(r, cur, aux, p0);
           break;
         }
         case XLB_T_CAVITY:
         case XLB_T_SAWTOOTH_CAVITY:
-          tan_cavity(J, a, r, cur, p0, tag == XLB_T_SAWTOOTH_CAVITY);
+          tan_cavity<MODE>(J, a, r, cur, p0, tag == XLB_T_SAWTOOTH_CAVITY);
           break;
         case XLB_T_RFMULTIPOLE:
-          tan_rfmultipole(J, a, r, cur, aux, p0);
+          tan_rfmultipole<MODE>(J, a, r, cur, aux, p0);
           break;
         case XLB_T_XYSHIFT:  // xline/elements.py:274-276: J unchanged
           r.x[0] = r.x[0] - p0;
@@ -539,14 +731,15 @@ __global__ void __launch_bounds__(256) tangent_kernel(const __grid_constant__ TA
           break;
         case XLB_T_SROTATION: {  // xline/elements.py:379-390: the same rotation of the rows
           const double cz = p0, sz = cur[1].x;
-#pragma unroll
-          for (int c = 0; c < 6; ++c) {
-            const double jx = J[X][c], jy = J[Y][c], jpx = J[PX][c], jpy = J[PY][c];
-            J[X][c] = fma(cz, jx, sz * jy);
-            J[Y][c] = fma(-sz, jx, cz * jy);
-            J[PX][c] = fma(cz, jpx, sz * jpy);
-            J[PY][c] = fma(-sz, jpx, cz * jpy);
-          }
+          TAN_ROWS(
+              _Pragma("unroll")
+              for (int c = 0; c < 6; ++c) {
+                const double jx = J[X][c], jy = J[Y][c], jpx = J[PX][c], jpy = J[PY][c];
+                J[X][c] = fma(cz, jx, sz * jy);
+                J[Y][c] = fma(-sz, jx, cz * jy);
+                J[PX][c] = fma(cz, jpx, sz * jpy);
+                J[PY][c] = fma(-sz, jpx, cz * jpy);
+              });
           const double xn = fma(cz, r.x[0], sz * r.y[0]), yn = fma(-sz, r.x[0], cz * r.y[0]);
           const double pxn = fma(cz, r.px[0], sz * r.py[0]), pyn = fma(-sz, r.px[0], cz * r.py[0]);
           r.x[0] = xn;
@@ -557,8 +750,7 @@ __global__ void __launch_bounds__(256) tangent_kernel(const __grid_constant__ TA
         }
         case XLB_T_DIPOLE_EDGE: {  // xline/elements.py:538-548
           const double r43 = cur[1].x;
-          axpy(J, PX, p0, X);
-          axpy(J, PY, r43, Y);
+          TAN_ROWS(axpy(J, PX, p0, X); axpy(J, PY, r43, Y));
           r.px[0] = r.px[0] + p0 * r.x[0];
           r.py[0] = r.py[0] + r43 * r.y[0];
           break;
@@ -572,7 +764,7 @@ __global__ void __launch_bounds__(256) tangent_kernel(const __grid_constant__ TA
             in = (r.x[0] >= p0) & (r.x[0] <= c1.x) & (r.y[0] >= c1.y) & (r.y[0] <= c2.x);
           const bool lost[1] = {r.alive(0) && !in};
           apply_losses<1>(a, r, lost, cur, 1, 5);
-          if (aux & XLB_AUX_DRIFT) tan_drift(J, r, a.beta0, aux, cur[3].x);
+          if (aux & XLB_AUX_DRIFT) tan_drift<MODE>(J, r, a.beta0, aux, cur[3].x);
           break;
         }
         case XLB_T_LIMIT_ELLIPSE: {
@@ -580,7 +772,7 @@ __global__ void __launch_bounds__(256) tangent_kernel(const __grid_constant__ TA
           const double q = fma(r.x[0] * r.x[0], c1.y, (r.y[0] * r.y[0]) * c2.x);
           const bool lost[1] = {r.alive(0) && !(q <= 1.0)};
           apply_losses<1>(a, r, lost, cur, 1, 5);
-          if (aux & XLB_AUX_DRIFT) tan_drift(J, r, a.beta0, aux, cur[3].x);
+          if (aux & XLB_AUX_DRIFT) tan_drift<MODE>(J, r, a.beta0, aux, cur[3].x);
           break;
         }
         case XLB_T_LIMIT_RECT_ELLIPSE: {
@@ -590,7 +782,7 @@ __global__ void __launch_bounds__(256) tangent_kernel(const __grid_constant__ TA
           const bool in = (r.x[0] >= -mx) & (r.x[0] <= mx) & (r.y[0] >= -c1.x) & (r.y[0] <= c1.x) & (q <= 1.0);
           const bool lost[1] = {r.alive(0) && !in};
           apply_losses<1>(a, r, lost, cur, 1, 7);
-          if (aux & XLB_AUX_DRIFT) tan_drift(J, r, a.beta0, aux, cur[4].x);
+          if (aux & XLB_AUX_DRIFT) tan_drift<MODE>(J, r, a.beta0, aux, cur[4].x);
           break;
         }
         case XLB_T_LIMIT_POLYGON: {
@@ -600,24 +792,30 @@ __global__ void __launch_bounds__(256) tangent_kernel(const __grid_constant__ TA
           for (int q = 0; q < n_edges; ++q, e += 2) odd ^= polygon_edge_crossed(r.x[0], r.y[0], e[0], e[1]);
           const bool lost[1] = {r.alive(0) && !odd};
           apply_losses<1>(a, r, lost, cur, 1, 2);
-          if (aux & XLB_AUX_DRIFT) tan_drift(J, r, a.beta0, aux, cur[1].y);
+          if (aux & XLB_AUX_DRIFT) tan_drift<MODE>(J, r, a.beta0, aux, cur[1].y);
           break;
         }
         case XLB_T_BEAMBEAM4D:
-          jac_beambeam4d(J, a, r, cur);
+          TAN_ROWS(jac_beambeam4d(J, a, r, cur));
           bf::beambeam4d<1>(a, r, cur);
           break;
         case XLB_T_SPACECHARGE:
-          jac_spacecharge(J, a, r, cur, aux & 0xf);
+          TAN_ROWS(jac_spacecharge(J, a, r, cur, aux & 0xf));
           bf::spacecharge<1>(a, r, cur, aux & 0xf);
-          if (aux & XLB_AUX_DRIFT) tan_drift(J, r, a.beta0, aux, p0);
+          if (aux & XLB_AUX_DRIFT) tan_drift<MODE>(J, r, a.beta0, aux, p0);
           break;
         default:  // XLB_T_MONITOR: the identity, nothing stored.  The host refuses every other tag.
+          if (MODE != TANGENT && tag == XLB_T_MULTIPOLE_RAD) tan_multipole_rad<MODE>(J, a, r, cur, aux, el);
           break;
       }
-      if (was_alive && !r.alive(0)) store_tangent(t, static_cast<int>(k), J, l2s, fli);  // frozen where lost
+      if (was_alive && !r.alive(0)) store<MODE>(t, eloss, static_cast<int>(k), J, l2s, fli, el);  // frozen where lost
     }
-    if (r.alive(0)) end_turn(J, l2s, fli);
+    if (r.alive(0)) {
+      if (MODE == ENVELOPE)
+        symmetrize(J);
+      else
+        end_turn(J, l2s, fli);
+    }
     r.turns_done += a.count_turns;
   }
   if (r.alive(0)) {
@@ -633,8 +831,20 @@ __global__ void __launch_bounds__(256) tangent_kernel(const __grid_constant__ TA
     a.s[i] = a.s[i] + r.s_acc;
     a.at_turn[i] = a.at_turn[i] + r.turns_done;
     a.at_element[i] = 0;
-    store_tangent(t, i, J, l2s, fli);
+    store<MODE>(t, eloss, i, J, l2s, fli, el);
   }
+}
+
+__global__ void __launch_bounds__(256) tangent_kernel(const __grid_constant__ TArgs t) {
+  tangent_body<TANGENT>(t, nullptr);
+}
+
+__global__ void __launch_bounds__(256) tangent_kernel_radiation(const __grid_constant__ TArgs t) {
+  tangent_body<TANGENT_R>(t, nullptr);
+}
+
+__global__ void __launch_bounds__(256) envelope_kernel(const __grid_constant__ EArgs e) {
+  tangent_body<ENVELOPE>(e.t, e.energy_loss);
 }
 
 }  // namespace tangent
@@ -648,6 +858,30 @@ cudaError_t tangent_launch(const KArgs &a, double *jac, long long *log2_scale, d
   t.fli = fli;
   const long long blocks = (a.n + threads - 1) / threads;
   tangent::tangent_kernel<<<static_cast<unsigned>(blocks), threads, 0, st>>>(t);
+  return cudaGetLastError();
+}
+
+cudaError_t tangent_radiation_launch(const KArgs &a, double *jac, long long *log2_scale, double *fli, int threads,
+                                     cudaStream_t st) {
+  tangent::TArgs t;
+  t.k = a;
+  t.jac = jac;
+  t.log2_scale = log2_scale;
+  t.fli = fli;
+  const long long blocks = (a.n + threads - 1) / threads;
+  tangent::tangent_kernel_radiation<<<static_cast<unsigned>(blocks), threads, 0, st>>>(t);
+  return cudaGetLastError();
+}
+
+cudaError_t envelope_launch(const KArgs &a, double *cov, double *energy_loss, int threads, cudaStream_t st) {
+  tangent::EArgs e;
+  e.t.k = a;
+  e.t.jac = cov;
+  e.t.log2_scale = nullptr;
+  e.t.fli = nullptr;
+  e.energy_loss = energy_loss;
+  const long long blocks = (a.n + threads - 1) / threads;
+  tangent::envelope_kernel<<<static_cast<unsigned>(blocks), threads, 0, st>>>(e);
   return cudaGetLastError();
 }
 

@@ -492,34 +492,54 @@ class Line(E.Element):
                 object.__setattr__(self, k, v)
         return trace
 
-    def _tangent_lattice(self, device):
+    def _tangent_lattice(self, device, radiation=False):
         """The element-by-element packing of ``trace_elem_by_elem`` (one record per element: no
         record fusing, no merging, no split lenses, no-ops kept) in the fast encoding, with a cache
-        entry of its own, and its copy on ``device``."""
+        entry of its own, and its copy on ``device``.  ``radiation=True``: the same packing with every
+        Multipole of length > 0 a mean-mode radiating record, whatever ``self.radiation`` is (the
+        tangent map and the envelope linearise about the mean-mode orbit), under a key of its own."""
         self._current_stamp()
-        key = ("tangent", self.chunk_words, self.flag_horizontal_bends, self.polygon_apertures, str(device))
-        hit = self._cache.get("tangent")
+        name = "tangent_rad" if radiation else "tangent"
+        key = (name, self.chunk_words, self.flag_horizontal_bends, self.polygon_apertures, str(device))
+        hit = self._cache.get(name)
         if hit is not None and hit[0] == key:
             return hit[1], hit[2]
         kw = {} if self.chunk_words is None else {"chunk_words": self.chunk_words}
+        if radiation:
+            kw["radiation"] = "mean"
         packed = pack_line(self.elements, strict=False, fuse=False, merge=False, split_lenses=False,
                            hx_only=self.flag_horizontal_bends, polygons=self.polygon_apertures,
                            drop_noops=False, **kw)
         _cabi.check(_cabi.lib().xlb_lattice_validate(C.byref(packed.c_lattice())))
         words = torch.from_numpy(packed.words.view(np.int64)).to(device)
-        self._cache["tangent"] = (key, packed, words)
+        self._cache[name] = (key, packed, words)
         return packed, words
 
-    def track_tangent(self, p, tangent, num_turns=1, threads_per_block=0):
+    def track_tangent(self, p, tangent, num_turns=1, threads_per_block=0, radiation=False):
         """Track ``p`` as ``track`` would, ``num_turns`` turns, and carry the Jacobian of every
         particle in ``tangent`` (a ``TangentMap`` of ``len(p)`` particles): both are updated in
         place, and a second call continues where the first stopped.  Returns ``None``.  Losses,
         ``at_element``, ``at_turn`` and ``loss_tally`` behave as in ``track``; a lost particle's
         Jacobian and FLI are frozen where it was lost.  Monitors store nothing here.  BeamBeam6D
-        lenses are refused (``ValueError``).  See ``xline_b200.tangent``."""
+        lenses are refused (``ValueError``).  A radiating line is refused unless ``radiation=True``,
+        which differentiates the mean-mode radiation too (a ``"quantum"`` line is refused: the random
+        map has no tangent); on a line without radiation ``radiation=True`` changes nothing.  See
+        ``xline_b200.tangent``."""
         from .tangent import track_tangent
 
-        return track_tangent(self, p, tangent, num_turns=num_turns, threads_per_block=threads_per_block)
+        return track_tangent(self, p, tangent, num_turns=num_turns, threads_per_block=threads_per_block,
+                             radiation=radiation)
+
+    def track_envelope(self, p, envelope, num_turns=1, threads_per_block=0):
+        """Track ``p`` as ``track_tangent`` would and carry, per particle, the second moment ``Sigma``
+        of a beam around it in ``envelope`` (an ``Envelope`` of ``len(p)`` particles): every element
+        maps ``Sigma -> J Sigma J^T``; on a radiating line (``"mean"`` or ``"quantum"``) the particle
+        follows the mean-mode map and every radiating half adds the variance of the quantum mode's
+        energy loss, and ``envelope.energy_loss`` accumulates the energy radiated (eV).  Both are
+        updated in place.  See ``xline_b200.tangent``."""
+        from .tangent import track_envelope
+
+        return track_envelope(self, p, envelope, num_turns=num_turns, threads_per_block=threads_per_block)
 
     def track_elem_by_elem(self, p, start=True, end=False):
         """Debug path (xline/line.py:97-108): one single-element launch per element,
