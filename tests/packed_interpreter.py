@@ -9,14 +9,18 @@ here must reproduce the oracle bit for bit (NumPy has no FMA contraction, and th
 encoding keeps the reference's operation order), the *fast* encoding to rounding.
 
 Everything but the BeamBeam6D record (covered by the GPU parity tests); the Faddeeva function of
-the Gaussian-field records is scipy's.  Nothing in the product imports this file.
+the Gaussian-field records is scipy's, and a MULTIPOLE_RAD record radiates through
+``tests/radiation_oracle.py`` with the mode, constants and seed it reads from the record.  Nothing
+in the product imports this file.
 """
 import numpy as np
+
+from tests import radiation_oracle as RO
 
 T_END_TURN, T_END_CHUNK, T_DRIFT, T_DRIFT_EXACT, T_MULTIPOLE, T_MULTIPOLE_CURVED = range(6)
 T_CAVITY, T_RFMULTIPOLE, T_XYSHIFT, T_SROTATION, T_DIPOLE_EDGE = range(6, 11)
 T_LIMIT_RECT, T_LIMIT_ELLIPSE, T_LIMIT_RECT_ELLIPSE, T_MONITOR, T_SAWTOOTH_CAVITY = range(11, 16)
-T_BEAMBEAM4D, T_SPACECHARGE, T_BEAMBEAM6D = 16, 17, 18
+T_BEAMBEAM4D, T_SPACECHARGE, T_BEAMBEAM6D, T_LIMIT_POLYGON, T_MULTIPOLE_RAD = 16, 17, 18, 19, 20
 AP_NONE, AP_RECT_SYM, AP_RECT, AP_ELLIPSE = range(4)
 COORDS = ("x", "px", "y", "py", "zeta", "delta", "rpp", "rvv")
 
@@ -170,6 +174,62 @@ def _kick(p, dpx, dpy, curved, strict, k0=None):
     return p.px + ddx, p.py + ddy, zeta
 
 
+def _multipole(p, f64, w, tag, aux, strict):
+    """The MULTIPOLE / MULTIPOLE_CURVED record at word ``w``: the kick applied to ``p``."""
+    if tag == T_MULTIPOLE:
+        pairs = f64[w + 2: w + 2 + 2 * (aux + 1)].reshape(aux + 1, 2)
+        curved = None
+    else:
+        pairs = f64[w + 6: w + 6 + 2 * (aux + 1)].reshape(aux + 1, 2)
+        curved = (f64[w + 1], f64[w + 2], f64[w + 3], f64[w + 4])
+    dpx, dpy = _horner(p, pairs, aux, strict)
+    p.px, p.py, p.zeta = _kick(p, dpx, dpy, curved, strict, k0=pairs[aux])
+
+
+class _Rad:
+    """The live particles as the radiation oracle's map sees them."""
+
+    def __init__(self, live, beam):
+        self.live, self.beam = live, beam
+        self.q0, self.p0c, self.energy0 = beam.q0, beam.p0c, beam.energy0
+        self.particle_id = beam.particle_id[live.idx]
+        self.at_turn = beam.at_turn[live.idx]
+
+    def __getattr__(self, k):
+        return getattr(self.live, k)
+
+    def __setattr__(self, k, v):
+        if k in COORDS:
+            setattr(self.live, k, v)
+        else:
+            object.__setattr__(self, k, v)
+
+    def add_to_energy(self, energy):
+        _add_to_energy(self.live, self.beam, energy)
+
+
+def _multipole_rad(p, beam, words, f64, i64, w, aux, elem, strict):
+    """The MULTIPOLE_RAD record at word ``w``: radiate, the embedded multipole, radiate."""
+    mode = {1: "mean", 2: "quantum"}[int(i64[w + 1])]
+    length = f64[w + 2]
+    consts = (f64[w + 4], f64[w + 5], f64[w + 6])
+    seed = int(words[w + 7])
+    sub = w + 8
+    tag = int(words[sub]) & 0xFF
+    if tag == T_MULTIPOLE:
+        pairs = f64[sub + 2: sub + 2 + 2 * (aux + 1)].reshape(aux + 1, 2)
+        hxl = hyl = 0.0
+    else:
+        pairs = f64[sub + 6: sub + 6 + 2 * (aux + 1)].reshape(aux + 1, 2)
+        hxl, hyl = f64[sub + 1], f64[sub + 2]
+    dpx, dpy = _horner(p, pairs, aux, strict)
+    fl = np.sqrt(dpx * dpx + dpy * dpy)
+    lh = 0.5 * (length + hxl * p.x - hyl * p.y)
+    RO.radiate_half(_Rad(p, beam), fl, lh, length, mode, seed, elem, 0, consts=consts)
+    _multipole(p, f64, sub, tag, aux, strict)
+    RO.radiate_half(_Rad(p, beam), fl, lh, length, mode, seed, elem, 1, consts=consts)
+
+
 def _inside(kind, x, y, lim, strict):
     if kind == AP_RECT_SYM:
         return (np.abs(x) <= lim[1]) & (np.abs(y) <= lim[3])
@@ -178,6 +238,17 @@ def _inside(kind, x, y, lim, strict):
     if strict:
         return x * x / lim[0] + y * y / lim[1] <= 1.0
     return x * x * lim[2] + y * y * lim[3] <= 1.0
+
+
+def polygon_inside(f64, i64, w, x, y):
+    """LIMIT_POLYGON at word ``w``: [hdr,n_edges][s_here,drift] then [y_lo,y_hi][x_lo,slope] per edge."""
+    n_edges = int(i64[w + 1])
+    odd = np.zeros(len(x), dtype=bool)
+    for y_lo, y_hi, x_lo, slope in f64[w + 4: w + 4 + 4 * n_edges].reshape(-1, 4):
+        assert y_lo < y_hi
+        with np.errstate(invalid="ignore"):  # inf * 0 for an infinite y at a vertical edge
+            odd ^= (y >= y_lo) & (y < y_hi) & (x < x_lo + (y - y_lo) * slope)
+    return odd
 
 
 def _gauss_field(f64, i64, w, x, y, strict):
@@ -229,6 +300,8 @@ def _path_length_words(tag, aux, w, f64, i64):
         return w + 5, (f64[w + 6] if aux & 0x10 else 0.0)
     if tag == T_LIMIT_RECT_ELLIPSE:
         return w + 7, (f64[w + 8] if aux & 0x10 else 0.0)
+    if tag == T_LIMIT_POLYGON:
+        return w + 2, (f64[w + 3] if aux & 0x10 else 0.0)
     if tag == T_SPACECHARGE:
         return None, (f64[w + 1] if aux & 0x10 else 0.0)
     if (tag & 0xC0) == 0xC0:  # dipole edge -> [drift]
@@ -342,15 +415,10 @@ def track(packed, cols, p0c, mass0, num_turns=1, monitor=None):
                     _drift(p, p0)
                 elif tag == T_DRIFT_EXACT:
                     _drift_exact(p, p0)
-                elif tag == T_MULTIPOLE:
-                    pairs = f64[w + 2: w + 2 + 2 * (aux + 1)].reshape(aux + 1, 2)
-                    dpx, dpy = _horner(p, pairs, aux, strict)
-                    p.px, p.py, p.zeta = _kick(p, dpx, dpy, None, strict)
-                elif tag == T_MULTIPOLE_CURVED:
-                    pairs = f64[w + 6: w + 6 + 2 * (aux + 1)].reshape(aux + 1, 2)
-                    dpx, dpy = _horner(p, pairs, aux, strict)
-                    curved = (p0, pair(1)[0], pair(1)[1], pair(2)[0])
-                    p.px, p.py, p.zeta = _kick(p, dpx, dpy, curved, strict, k0=pairs[aux])
+                elif tag in (T_MULTIPOLE, T_MULTIPOLE_CURVED):
+                    _multipole(p, f64, w, tag, aux, strict)
+                elif tag == T_MULTIPOLE_RAD:
+                    _multipole_rad(p, beam, words, f64, i64, w, aux, elem, strict)
                 elif tag in (T_CAVITY, T_SAWTOOTH_CAVITY):
                     k, lag = pair(1)
                     tau = p.zeta / p.rvv / beam.beta0
@@ -392,6 +460,10 @@ def track(packed, cols, p0c, mass0, num_turns=1, monitor=None):
                     p.lose(~inside, elem, turn)
                     if aux & 0x10:
                         (_drift_exact if aux & 0x20 else _drift)(p, pair(4)[0])
+                elif tag == T_LIMIT_POLYGON:
+                    p.lose(~polygon_inside(f64, i64, w, p.x, p.y), elem, turn)
+                    if aux & 0x10:
+                        (_drift_exact if aux & 0x20 else _drift)(p, f64[w + 3])
                 elif tag == T_RFMULTIPOLE:  # [hdr,V][k,lag] then per order [knl,ksl][pn,ps]
                     k, lag = pair(1)
                     ktau = k * (p.zeta / p.rvv / beam.beta0)

@@ -2,9 +2,12 @@
 ("Tangent map"): one particle walked through the element-by-element packing of a line (fast
 encoding, ``Line._tangent_lattice``), the coordinates advanced with the maps of
 ``tests/packed_interpreter.py`` and ``J <- M(z before) . J`` with each element's 6x6 Jacobian M
-written out densely from the element definitions.  Everything but BeamBeam6D.
+written out densely from the element definitions.  Everything but BeamBeam6D.  A mean-mode
+MULTIPOLE_RAD record's Jacobian and diffusion come from ``tests/tangent_radiation_oracle.py``,
+and the walk carries the envelope Sigma <- M Sigma M^T + D along with J.
 """
 import math
+import types
 
 import numpy as np
 from scipy.special import wofz
@@ -238,44 +241,37 @@ def element_jacobian(words, w, s, b, chi=1.0, qr=1.0):
     return M  # XYSHIFT, LIMIT_*, MONITOR: the identity
 
 
-def _advance(words, w, part, n_words_rec):
-    """Advance ``part`` through the record at word ``w`` with the packed interpreter: a one-record
-    copy of the lattice, closed by END_TURN."""
-    import types
-
-    rec = np.zeros(2 * n_words_rec + 2, dtype=np.uint64)
-    rec[: 2 * n_words_rec] = words[w: w + 2 * n_words_rec]
-    f64 = rec.view(np.float64)
-    hdr = int(rec[0])
-    tag, aux = hdr & 0xFF, (hdr >> 8) & 0xFF
-    s_adv = f64[1] if tag in (PI.T_DRIFT, PI.T_DRIFT_EXACT) else 0.0
-    rec[2 * n_words_rec] = np.uint64(0)  # END_TURN
-    f64[2 * n_words_rec + 1] = s_adv
-    # records with an s_here word expect 0.0 there: a one-record pass starts at s = 0
-    if tag in (PI.T_LIMIT_RECT, PI.T_LIMIT_ELLIPSE):
-        f64[5] = 0.0
-    elif tag == PI.T_LIMIT_RECT_ELLIPSE:
-        f64[7] = 0.0
-    packed = types.SimpleNamespace(words=rec, chunk_words=len(rec), n_chunks=1, strict=False, segments=None)
-    cols = {k: getattr(part.p, k) for k in COORDS}
-    out = PI.track(packed, cols, part.beam.p0c, part.beam.mass0, 1)
-    return out
-
-
 def element_map(words, w, z, p0c, mass0, q0=1.0):
-    """z after the record at word ``w`` (packed interpreter), and whether the particle survived."""
-    hdr = int(words[w])
+    """z after the record at word ``w`` (packed interpreter), and whether the particle survived: the
+    interpreter runs a one-record copy of the lattice, closed by END_TURN."""
+    size = (int(words[w]) >> 16) & 0x3FFF
+    rec = np.zeros(2 * size + 2, dtype=np.uint64)
+    rec[: 2 * size] = words[w: w + 2 * size]
+    f64, i64 = rec.view(np.float64), rec.view(np.int64)
+    hdr = int(rec[0])
+    # a one-record pass starts at s = 0: the s_here word, if any, holds 0.0 and END_TURN the advance
+    s_at, adv = PI._path_length_words(hdr & 0xFF, (hdr >> 8) & 0xFF, 0, f64, i64)
+    if s_at is not None:
+        f64[s_at] = 0.0
+    rec[2 * size] = np.uint64(PI.T_END_TURN)
+    f64[2 * size + 1] = adv
+    packed = types.SimpleNamespace(words=rec, chunk_words=len(rec), n_chunks=1, strict=False, segments=None)
     part = Particle(z, p0c, mass0, q0)
-    out = _advance(words, w, part, (hdr >> 16) & 0x3FFF)
+    out = PI.track(packed, {k: getattr(part.p, k) for k in COORDS}, p0c, mass0, 1)
     return np.array([out[k][0] for k in COORDS]), bool(out["state"][0] == 1)
 
 
-def track(packed, z, p0c, mass0, q0=1.0, num_turns=1):
-    """(z after ``num_turns`` turns, J) of one particle through ``packed`` (element-by-element
-    packing, fast encoding).  Tagging records it cannot follow raises."""
+def track(packed, z, p0c, mass0, q0=1.0, num_turns=1, cov=None):
+    """(z, J, Sigma, energy lost, alive) of one particle after ``num_turns`` turns of ``packed``
+    (element-by-element packing, fast encoding, mean-mode radiating records included); Sigma starts
+    at ``cov`` (default 0).  Tagging records it cannot follow raises."""
+    from tests import tangent_radiation_oracle as TRO
+
     words = np.ascontiguousarray(packed.words, dtype=np.uint64)
     z = np.array(z, dtype=np.float64)
     J = np.eye(6)
+    S = np.zeros((6, 6)) if cov is None else np.array(cov, dtype=np.float64)
+    lost = 0.0
     b = Particle(z, p0c, mass0, q0).beam
     for _ in range(num_turns):
         for ch in range(packed.n_chunks):
@@ -289,16 +285,22 @@ def track(packed, z, p0c, mass0, q0=1.0, num_turns=1):
                 if tag == PI.T_END_TURN:
                     end = True
                     break
-                part = Particle(z, p0c, mass0, q0)
-                s = [float(getattr(part.p, k)[0]) for k in COORDS + ("rpp", "rvv")]
-                J = element_jacobian(words, w, s, b) @ J
+                if tag == PI.T_MULTIPOLE_RAD:
+                    M, D, e, _ = TRO.rad_record(words, w, z, b)
+                    lost += e
+                else:
+                    part = Particle(z, p0c, mass0, q0)
+                    s = [float(getattr(part.p, k)[0]) for k in COORDS + ("rpp", "rvv")]
+                    M, D = element_jacobian(words, w, s, b), 0.0
+                J = M @ J
+                S = M @ S @ M.T + D
                 z, alive = element_map(words, w, z, p0c, mass0, q0)
                 if not alive:
-                    return z, J, False
+                    return z, J, S, lost, False
                 w += 2 * size
             if end:
                 break
-    return z, J, True
+    return z, J, S, lost, True
 
 
 P0C, MASS0 = 6.5e12, 938.27208816e6  # LHC protons: beta0 close to 1
@@ -347,16 +349,18 @@ def element_cases():
     ]
 
 
-def pack_one(element):
-    """The element-by-element packing ``Line.track_tangent`` uses, of a one-element line."""
+def pack_one(element, radiation=None):
+    """The element-by-element packing ``Line.track_tangent`` uses, of a one-element line
+    (``radiation="mean"``: that of ``Line.track_tangent(..., radiation=True)``)."""
     from xline_b200.lattice import pack_line
 
-    return pack_line([element], strict=False, fuse=False, merge=False, split_lenses=False, drop_noops=False)
+    return pack_line([element], strict=False, fuse=False, merge=False, split_lenses=False, drop_noops=False,
+                     radiation=radiation)
 
 
-def fd_jacobian(element, z, p0c, rel=1e-3):
-    """Central differences of the packed interpreter's map, Richardson-extrapolated (h, h/2)."""
-    packed = pack_one(element)
+def fd_jacobian(packed, z, p0c, mass0=MASS0, rel=1e-3, w=0):
+    """Central differences of the packed interpreter's map of the record at word ``w``,
+    Richardson-extrapolated (h, h/2)."""
     words = np.ascontiguousarray(packed.words, dtype=np.uint64)
     # delta steps are the largest: rvv and rpp are recomputed from delta with an error of ~1e-16 each
     scale = np.array([1e-3, 1e-4, 1e-3, 1e-4, 1e-2, 1e-3])
@@ -368,7 +372,7 @@ def fd_jacobian(element, z, p0c, rel=1e-3):
             zp, zm = z.copy(), z.copy()
             zp[c] += hh
             zm[c] -= hh
-            return (element_map(words, 0, zp, p0c, MASS0)[0] - element_map(words, 0, zm, p0c, MASS0)[0]) / (2 * hh)
+            return (element_map(words, w, zp, p0c, mass0)[0] - element_map(words, w, zm, p0c, mass0)[0]) / (2 * hh)
 
         out[:, c] = (4 * d(h / 2) - d(h)) / 3
     return out
@@ -376,6 +380,6 @@ def fd_jacobian(element, z, p0c, rel=1e-3):
 
 def oracle_jacobian(element, z, p0c):
     packed = pack_one(element)
-    zz, J, alive = track(packed, z, p0c, MASS0)
+    zz, J, _, _, alive = track(packed, z, p0c, MASS0)
     assert alive
     return J

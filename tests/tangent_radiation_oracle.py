@@ -1,34 +1,20 @@
-"""TEST INFRASTRUCTURE -- a NumPy statement of the tangent map and the envelope of lines with
-mean-mode radiating multipoles (include/xline_b200.h, xlb_track_tangent_radiation_device and
-xlb_track_envelope_device; DESIGN.md §4.10).
+"""TEST INFRASTRUCTURE -- a NumPy statement of the Jacobian and the diffusion of a mean-mode
+MULTIPOLE_RAD record (include/xline_b200.h, xlb_track_tangent_radiation_device and
+xlb_track_envelope_device; DESIGN.md §4.10), for the walk of ``tests/tangent_oracle.py``.
 
-One particle is walked through the element-by-element packing with radiation
-(``Line._tangent_lattice(..., radiation=True)``): the coordinates advance with
-``tests/radiation_interpreter.py`` (the packed maps), every other record's Jacobian comes from
-``tests/tangent_oracle.py``, and a MULTIPOLE_RAD record's Jacobian is written out densely here as
-half . kick . half, each half the chain of add_to_energy and the scaling of px, py.  The envelope
-adds, per radiating half, V_h g g^T with V_h = nbar (11/27) u_c^2 and g = dz_after/dW.
+The record's Jacobian is written out densely as half . kick . half, each half the chain of
+add_to_energy and the scaling of px, py.  The envelope adds, per radiating half, V_h g g^T with
+V_h = nbar (11/27) u_c^2 and g = dz_after/dW.  ``b`` is the beam of ``tangent_oracle.Particle``.
 """
 import math
-import types
 
 import numpy as np
 
 from tests import packed_interpreter as PI
-from tests import radiation_interpreter as RI
 from tests import tangent_oracle as TO
 
 X, PX, Y, PY, ZETA, DELTA = range(6)
-COORDS = TO.COORDS
-T_MULTIPOLE_RAD = RI.T_MULTIPOLE_RAD
 X2_MEAN = 11.0 / 27.0  # <x^2> of the photon-number spectrum (x = photon energy / u_c)
-
-
-class Beam:
-    def __init__(self, p0c, mass0, q0=1.0):
-        self.p0c, self.mass0, self.q0 = float(p0c), float(mass0), float(q0)
-        self.energy0 = math.sqrt(self.p0c ** 2 + self.mass0 ** 2)
-        self.beta0 = self.p0c / self.energy0
 
 
 def _energy(b, d):
@@ -138,88 +124,3 @@ def rad_record(words, w, z, b):
     T = M2 @ K
     D = V1 * np.outer(T @ g1, T @ g1) + V2 * np.outer(g2, g2)
     return M2 @ K @ M1, D, -(e1 + e2), z3
-
-
-def _one_record(words, w, size):
-    rec = np.zeros(2 * size + 2, dtype=np.uint64)
-    rec[: 2 * size] = words[w: w + 2 * size]
-    f64 = rec.view(np.float64)
-    tag = int(rec[0]) & 0xFF
-    f64[2 * size + 1] = f64[1] if tag in (PI.T_DRIFT, PI.T_DRIFT_EXACT) else 0.0  # END_TURN
-    if tag in (PI.T_LIMIT_RECT, PI.T_LIMIT_ELLIPSE):
-        f64[5] = 0.0
-    return types.SimpleNamespace(words=rec, chunk_words=len(rec), n_chunks=1, strict=False, segments=None)
-
-
-def element_map(words, w, z, p0c, mass0):
-    """z after the record at word ``w`` (radiation interpreter), and whether the particle survived."""
-    size = (int(words[w]) >> 16) & 0x3FFF
-    out = RI.track(_one_record(words, w, size), {k: [float(v)] for k, v in zip(COORDS, z)}, p0c, mass0, 1)
-    return np.array([out[k][0] for k in COORDS]), bool(out["state"][0] == 1)
-
-
-def track(packed, z, p0c, mass0, num_turns=1, cov=None):
-    """(z, J, Sigma, energy lost, alive) of one particle after ``num_turns`` turns of ``packed``
-    (element-by-element packing with mean-mode radiating records); Sigma starts at ``cov``
-    (default 0)."""
-    words = np.ascontiguousarray(packed.words, dtype=np.uint64)
-    z = np.array(z, dtype=np.float64)
-    J = np.eye(6)
-    S = np.zeros((6, 6)) if cov is None else np.array(cov, dtype=np.float64)
-    b = Beam(p0c, mass0)
-    lost = 0.0
-    for _ in range(num_turns):
-        for ch in range(packed.n_chunks):
-            w = ch * packed.chunk_words
-            end = False
-            while True:
-                hdr = int(words[w])
-                tag, size = hdr & 0xFF, (hdr >> 16) & 0x3FFF
-                if tag == PI.T_END_CHUNK:
-                    break
-                if tag == PI.T_END_TURN:
-                    end = True
-                    break
-                if tag == T_MULTIPOLE_RAD:
-                    M, D, e, _ = rad_record(words, w, z, b)
-                    lost += e
-                else:
-                    rvv, _ = _energy(b, z[DELTA])
-                    M = TO.element_jacobian(words, w, list(z) + [1 / (1 + z[DELTA]), rvv], b)
-                    D = 0.0
-                J = M @ J
-                S = M @ S @ M.T + D
-                z, alive = element_map(words, w, z, p0c, mass0)
-                if not alive:
-                    return z, J, S, lost, False
-                w += 2 * size
-            if end:
-                break
-    return z, J, S, lost, True
-
-
-def pack_one(element):
-    """The packing ``Line.track_tangent(..., radiation=True)`` uses, of a one-element line."""
-    from xline_b200.lattice import pack_line
-
-    return pack_line([element], strict=False, fuse=False, merge=False, split_lenses=False, drop_noops=False,
-                     radiation="mean")
-
-
-def fd_jacobian(packed, z, p0c, mass0, rel=1e-3, w=0):
-    """Central differences of the radiation interpreter's map of the record at word ``w``,
-    Richardson-extrapolated (h, h/2)."""
-    words = np.ascontiguousarray(packed.words, dtype=np.uint64)
-    scale = np.array([1e-3, 1e-4, 1e-3, 1e-4, 1e-2, 1e-3])
-    out = np.zeros((6, 6))
-    for c in range(6):
-        h = rel * scale[c]
-
-        def d(hh):
-            zp, zm = z.copy(), z.copy()
-            zp[c] += hh
-            zm[c] -= hh
-            return (element_map(words, w, zp, p0c, mass0)[0] - element_map(words, w, zm, p0c, mass0)[0]) / (2 * hh)
-
-        out[:, c] = (4 * d(h / 2) - d(h)) / 3
-    return out

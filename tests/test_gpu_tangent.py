@@ -119,7 +119,7 @@ def test_lattice_jacobian_matches_oracle_on_fodo_and_psb():
         p, t = _tangent(line, z, p0c, m0)
         J = t.matrix()[0].cpu().numpy()
         packed, _ = line._tangent_lattice(DEV)
-        zz, ref, alive = TO.track(packed, z, p0c, m0)
+        zz, ref, _, _, alive = TO.track(packed, z, p0c, m0)
         assert alive
         scale = np.maximum(np.max(np.abs(ref), axis=0), 1e-300)
         err = np.max(np.abs(J - ref) / scale)

@@ -13,7 +13,7 @@ import pytest
 import torch
 
 import xline_b200 as xl
-from tests import tangent_radiation_oracle as TRO
+from tests import tangent_oracle as TO
 from tests.test_gpu_radiation import _damping_ring, _planes, _ring
 from xline_b200 import build, configs, lattice, optics, tangent
 
@@ -70,7 +70,7 @@ def test_jacobian_against_oracle_and_coordinates_against_track(which):
         worst_z = max(worst_z, float(np.max(np.abs(got - ref) / scale)))
         packed, _ = line._tangent_lattice(torch.device("cuda", torch.cuda.current_device()), radiation=True)
         for i, z in enumerate(Z0):
-            zz, J, _, _, alive = TRO.track(packed, z, P0C, ELECTRON)
+            zz, J, _, _, alive = TO.track(packed, z, P0C, ELECTRON)
             assert alive
             worst_j = max(worst_j, _jac_err(t.matrix()[i].cpu().numpy(), J))
     print("tangent with radiation (%s): J vs oracle %.3g, z vs Line.track %.3g" % (which, worst_j, worst_z))
@@ -114,7 +114,7 @@ def test_envelope_on_the_radiating_ring_against_oracle():
     packed, _ = line._tangent_lattice(torch.device("cuda", torch.cuda.current_device()), radiation=True)
     worst_s = worst_d = worst_u = 0.0
     for i, z in enumerate(Z0):
-        _, J, S, lost, _ = TRO.track(packed, z, P0C, ELECTRON, cov=s0)
+        _, J, S, lost, _ = TO.track(packed, z, P0C, ELECTRON, cov=s0)
         got = env.cov[i].cpu().numpy()
         worst_s = max(worst_s, float(np.max(np.abs(got - S)) / np.max(np.abs(S))))
         worst_u = max(worst_u, abs(float(env.energy_loss[i]) / lost - 1))
@@ -122,7 +122,7 @@ def test_envelope_on_the_radiating_ring_against_oracle():
     env0 = xl.Envelope(len(Z0), device="cuda")
     line.track_envelope(_particles(Z0), env0)
     for i, z in enumerate(Z0):
-        D = TRO.track(packed, z, P0C, ELECTRON)[2]
+        D = TO.track(packed, z, P0C, ELECTRON)[2]
         worst_d = max(worst_d, float(np.max(np.abs(env0.cov[i].cpu().numpy() - D)) / np.max(np.abs(D))))
     print("envelope vs oracle: Sigma %.3g, D %.3g, energy loss %.3g" % (worst_s, worst_d, worst_u))
     # measured on a B200: 2.2e-15, 7.1e-16, 2.2e-16
@@ -159,7 +159,7 @@ def test_damping_ring_equilibrium():
     assert abs(robinson - 4) < 7e-5
     # the oracle's one-turn matrix on the GPU's orbit: the same eigenvalues
     packed, _ = line._tangent_lattice(torch.device("cuda", torch.cuda.current_device()), radiation=True)
-    zz, J, D, U, alive = TRO.track(packed, eq.orbit, p0c, m0)
+    zz, J, D, U, alive = TO.track(packed, eq.orbit, p0c, m0)
     assert alive
     assert np.max(np.abs(zz - eq.orbit)) < 1e-12
     lam, _ = tangent._symplectic_modes(J)

@@ -11,7 +11,7 @@ import xline_b200 as xl
 from oracle import xline_oracle as xo
 from tests import helpers as H
 from tests import polygon_cases as PC
-from tests import polygon_interpreter as PI
+from tests import packed_interpreter as PI
 from tests import polygon_oracle as PO
 from xline_b200 import _cabi, lattice
 

@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 
 import xline_b200 as xl
-from tests import radiation_interpreter as RI
+from tests import packed_interpreter as PI
 from tests import radiation_oracle as RO
 from xline_b200 import lattice, optics
 
@@ -195,7 +195,7 @@ def test_interpreter_against_oracle_on_random_lines(mode):
         cols = dict(x=rng.normal(0, 1e-3, n), px=rng.normal(0, 1e-4, n), y=rng.normal(0, 1e-3, n),
                     py=rng.normal(0, 1e-4, n), zeta=rng.normal(0, 1e-3, n), delta=rng.normal(0, 1e-3, n))
         pk = lattice.pack_line(els, radiation=mode, radiation_seed=trial + 17, merge=False)
-        got = RI.track(pk, cols, P0C, ELECTRON, num_turns=3)
+        got = PI.track(pk, cols, P0C, ELECTRON, num_turns=3)
         want = RO.run_oracle(lattice.element_specs(els), cols, P0C, ELECTRON, num_turns=3, radiation=mode,
                              seed=trial + 17)
         np.testing.assert_array_equal(got["state"], want["state"])

@@ -19,7 +19,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 def test_oracle_jacobian_matches_finite_differences(case):
     name, el, p0c, z = case
     J = TO.oracle_jacobian(el, z, p0c)
-    fd = TO.fd_jacobian(el, z, p0c)
+    fd = TO.fd_jacobian(TO.pack_one(el), z, p0c)
     # per column: the error of a Richardson-extrapolated difference is relative to the column's size
     scale = np.maximum(np.max(np.abs(J), axis=0), 1e-300)
     err = np.max(np.abs(J - fd) / scale)

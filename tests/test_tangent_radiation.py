@@ -1,6 +1,6 @@
 """Radiation in the tangent map without a GPU: the NumPy statement of the radiating record's Jacobian
 and diffusion (tests/tangent_radiation_oracle.py) against Richardson-extrapolated central differences
-of the radiation interpreter's map, V_h against the photon statistics of the committed table, the
+of the packed interpreter's map, V_h against the photon statistics of the committed table, the
 header and the refusals that need no device."""
 import math
 import os
@@ -11,6 +11,7 @@ import pytest
 
 import xline_b200 as xl
 from tests import radiation_oracle as RO
+from tests import tangent_oracle as TO
 from tests import tangent_radiation_oracle as TRO
 from xline_b200 import _cabi, configs
 
@@ -32,7 +33,7 @@ CASES = [
 def _boosted(el, boost):
     """The element's radiating packing with K_e and alpha multiplied by ``boost``: the radiation terms of
     J then stand out of its radiation-free part, so the differences test them, not just the kick."""
-    packed = TRO.pack_one(el)
+    packed = TO.pack_one(el, radiation="mean")
     f64 = packed.words.view(np.float64)
     f64[4] *= boost
     f64[6] *= boost
@@ -44,20 +45,20 @@ def _boosted(el, boost):
 def test_oracle_jacobian_matches_finite_differences(case, boost):
     name, el, z = case
     packed = _boosted(el, boost)
-    _, J, _, _, alive = TRO.track(packed, z, P0C, ELECTRON)
+    _, J, _, _, alive = TO.track(packed, z, P0C, ELECTRON)
     assert alive
-    fd = TRO.fd_jacobian(packed, z, P0C, ELECTRON)
+    fd = TO.fd_jacobian(packed, z, P0C, ELECTRON)
     scale = np.maximum(np.max(np.abs(J), axis=0), 1e-300)
     err = np.max(np.abs(J - fd) / scale)
     assert err <= 1e-8, (name, err, J, fd)
     # the radiation part itself, against the differences of the map without radiation
     if boost > 1 and name != "quadrupole_on_axis":
-        bare = TRO.pack_one(el)
+        bare = TO.pack_one(el, radiation="mean")
         bare.words.view(np.float64)[4] = 0.0
-        J0 = TRO.track(bare, z, P0C, ELECTRON)[1]
+        J0 = TO.track(bare, z, P0C, ELECTRON)[1]
         rad = J - J0
         assert np.max(np.abs(rad)) > 1e-4 * np.max(np.abs(J))
-        fd0 = TRO.fd_jacobian(bare, z, P0C, ELECTRON)
+        fd0 = TO.fd_jacobian(bare, z, P0C, ELECTRON)
         err = np.max(np.abs(rad - (fd - fd0))) / np.max(np.abs(rad))
         assert err <= 1e-6, (name, err)
 
@@ -65,8 +66,8 @@ def test_oracle_jacobian_matches_finite_differences(case, boost):
 def test_on_axis_quadrupole_radiates_nothing():
     el = CASES[-1][1]
     z = CASES[-1][2]
-    packed = TRO.pack_one(el)
-    zz, J, S, lost, alive = TRO.track(packed, z, P0C, ELECTRON)
+    packed = TO.pack_one(el, radiation="mean")
+    zz, J, S, lost, alive = TO.track(packed, z, P0C, ELECTRON)
     assert lost == 0.0 and not S.any()
 
 
@@ -76,9 +77,9 @@ def test_diffusion_matches_difference_jacobians_and_vh(case):
     g_h = dz_after/dW of a half is the difference of the map under a shift of the half's loss, taken
     here by a shift of K_e in that half alone (W is proportional to K_e)."""
     name, el, z = case
-    packed = TRO.pack_one(el)
+    packed = TO.pack_one(el, radiation="mean")
     words = np.ascontiguousarray(packed.words)
-    b = TRO.Beam(P0C, ELECTRON)
+    b = TO.Particle(z, P0C, ELECTRON).beam
     J, D, lost, zout = TRO.rad_record(words, 0, z, b)
     f64 = words.view(np.float64)
     rec = (f64[2], f64[3], f64[4], f64[5], f64[6])
@@ -162,10 +163,10 @@ def test_vh_matches_the_photon_statistics_of_the_table():
 
 def test_oracle_record_matches_the_interpreter_state():
     for name, el, z in CASES:
-        packed = TRO.pack_one(el)
+        packed = TO.pack_one(el, radiation="mean")
         words = np.ascontiguousarray(packed.words)
-        zout = TRO.rad_record(words, 0, z, TRO.Beam(P0C, ELECTRON))[3]
-        ref, alive = TRO.element_map(words, 0, z, P0C, ELECTRON)
+        zout = TRO.rad_record(words, 0, z, TO.Particle(z, P0C, ELECTRON).beam)[3]
+        ref, alive = TO.element_map(words, 0, z, P0C, ELECTRON)
         assert alive
         np.testing.assert_allclose(zout, ref, rtol=1e-13, atol=1e-19, err_msg=name)
 

@@ -1002,60 +1002,47 @@ static int tangent_scan(const xlb_lattice_t *lat, bool radiation, const char *wh
   return XLB_OK;
 }
 
-static void tangent_stats(const xlb_particles_t *p, int threads) {
+// The three tangent-map entry points: the kernel of `mode` over the particles of p.  `jac` is J, or
+// Sigma for the envelope; log2_scale and fli go with J, energy_loss with Sigma.
+static int track_tangent_impl(const xlb_lattice_t *lat, xlb_particles_t *p, const xlb_track_options_t *o,
+                              tangent::Mode mode, double *jac, int64_t *log2_scale, double *fli,
+                              double *energy_loss, void *stream) {
+  memset(&g_stats, 0, sizeof(g_stats));
+  const bool envelope = mode == tangent::ENVELOPE, radiation = mode != tangent::TANGENT;
+  const char *what = envelope ? "envelope tracking" : "tangent tracking";
+  int rc, threads;
+  if ((rc = tangent_checks(lat, p, o, radiation, what, &threads)) != XLB_OK) return rc;
+  if (p->n == 0 || o->num_turns == 0) return XLB_OK;
+  if (envelope && (!jac || !energy_loss)) return fail(XLB_EINVAL, "cov and energy_loss must not be null");
+  if (!envelope && (!jac || !log2_scale || !fli))
+    return fail(XLB_EINVAL, "jac, log2_scale and fli must not be null");
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  CallScope call;
+  if ((rc = call.open(st)) != XLB_OK) return rc;
+  if ((rc = tangent_scan(lat, radiation, what, st)) != XLB_OK) return rc;
+  KArgs a = kernel_args(lat, p, o, call.s->n_lost);
+  a.num_turns = o->num_turns;
+  XLB_CUDA(tangent_launch(mode, a, jac, reinterpret_cast<long long *>(log2_scale), fli, energy_loss, threads, st));
   g_stats.kernel_launches = 1;
   g_stats.threads = threads;
   g_stats.blocks = static_cast<int>((p->n + threads - 1) / threads);
   g_stats.n_alive_in = p->n;
-}
-
-static int track_tangent_impl(const xlb_lattice_t *lat, xlb_particles_t *p, const xlb_track_options_t *o,
-                              double *jac, int64_t *log2_scale, double *fli, void *stream, bool radiation) {
-  memset(&g_stats, 0, sizeof(g_stats));
-  int rc, threads;
-  if ((rc = tangent_checks(lat, p, o, radiation, "tangent tracking", &threads)) != XLB_OK) return rc;
-  if (p->n == 0 || o->num_turns == 0) return XLB_OK;
-  if (!jac || !log2_scale || !fli) return fail(XLB_EINVAL, "jac, log2_scale and fli must not be null");
-  const cudaStream_t st = static_cast<cudaStream_t>(stream);
-  CallScope call;
-  if ((rc = call.open(st)) != XLB_OK) return rc;
-  if ((rc = tangent_scan(lat, radiation, "tangent tracking", st)) != XLB_OK) return rc;
-  KArgs a = kernel_args(lat, p, o, call.s->n_lost);
-  a.num_turns = o->num_turns;
-  if (radiation)
-    XLB_CUDA(tangent_radiation_launch(a, jac, reinterpret_cast<long long *>(log2_scale), fli, threads, st));
-  else
-    XLB_CUDA(tangent_launch(a, jac, reinterpret_cast<long long *>(log2_scale), fli, threads, st));
-  tangent_stats(p, threads);
   return XLB_OK;
 }
 
 int xlb_track_tangent_device(const xlb_lattice_t *lat, xlb_particles_t *p, const xlb_track_options_t *o,
                              double *jac, int64_t *log2_scale, double *fli, void *stream) {
-  return track_tangent_impl(lat, p, o, jac, log2_scale, fli, stream, false);
+  return track_tangent_impl(lat, p, o, tangent::TANGENT, jac, log2_scale, fli, nullptr, stream);
 }
 
 int xlb_track_tangent_radiation_device(const xlb_lattice_t *lat, xlb_particles_t *p, const xlb_track_options_t *o,
                                        double *jac, int64_t *log2_scale, double *fli, void *stream) {
-  return track_tangent_impl(lat, p, o, jac, log2_scale, fli, stream, true);
+  return track_tangent_impl(lat, p, o, tangent::TANGENT_R, jac, log2_scale, fli, nullptr, stream);
 }
 
 int xlb_track_envelope_device(const xlb_lattice_t *lat, xlb_particles_t *p, const xlb_track_options_t *o,
                               double *cov, double *energy_loss, void *stream) {
-  memset(&g_stats, 0, sizeof(g_stats));
-  int rc, threads;
-  if ((rc = tangent_checks(lat, p, o, true, "envelope tracking", &threads)) != XLB_OK) return rc;
-  if (p->n == 0 || o->num_turns == 0) return XLB_OK;
-  if (!cov || !energy_loss) return fail(XLB_EINVAL, "cov and energy_loss must not be null");
-  const cudaStream_t st = static_cast<cudaStream_t>(stream);
-  CallScope call;
-  if ((rc = call.open(st)) != XLB_OK) return rc;
-  if ((rc = tangent_scan(lat, true, "envelope tracking", st)) != XLB_OK) return rc;
-  KArgs a = kernel_args(lat, p, o, call.s->n_lost);
-  a.num_turns = o->num_turns;
-  XLB_CUDA(envelope_launch(a, cov, energy_loss, threads, st));
-  tangent_stats(p, threads);
-  return XLB_OK;
+  return track_tangent_impl(lat, p, o, tangent::ENVELOPE, cov, nullptr, nullptr, energy_loss, stream);
 }
 
 int xlb_compact_alive_device(const int64_t *state, int64_t n, int32_t *idx_out, int32_t *n_out,

@@ -73,15 +73,21 @@ cudaError_t beam_moments_launch(const double *x, const double *px, const double 
 cudaError_t naff_launch(const double *u, const double *pu, long long n, int num_turns, long long stride,
                         double beta, double alpha, double *tune, double *amplitude, cudaStream_t st);
 
-// Tangent-map tracking of the a.n particles (tangent.cu): one particle per thread, `threads` per CTA,
-// all a.num_turns turns in one launch; arguments checked by the caller.
-cudaError_t tangent_launch(const KArgs &a, double *jac, long long *log2_scale, double *fli, int threads,
-                           cudaStream_t st);
-// The same with mean-mode radiating multipoles (tangent_kernel_radiation), and the envelope
-// Sigma <- J Sigma J^T + diffusion with the energy lost (envelope_kernel).
-cudaError_t tangent_radiation_launch(const KArgs &a, double *jac, long long *log2_scale, double *fli, int threads,
-                                     cudaStream_t st);
-cudaError_t envelope_launch(const KArgs &a, double *cov, double *energy_loss, int threads, cudaStream_t st);
+namespace tangent {
+// What the tangent-map kernel body carries (tangent.cu; include/xline_b200.h, "Tangent map"):
+//   TANGENT   J, no radiating records (tangent_kernel);
+//   TANGENT_R J, with mean-mode MULTIPOLE_RAD records (tangent_kernel_radiation);
+//   ENVELOPE  Sigma <- J_e Sigma J_e^T per element, plus the quantum diffusion of every radiating half
+//             (envelope_kernel).
+enum Mode { TANGENT = 0, TANGENT_R = 1, ENVELOPE = 2 };
+}  // namespace tangent
+
+// Tangent-map tracking of the a.n particles (tangent.cu) in the kernel of `mode`: one particle per
+// thread, `threads` per CTA, all a.num_turns turns in one launch; arguments checked by the caller.
+// `jac` is J, or Sigma for ENVELOPE, [n][6][6]; log2_scale and fli are used by the tangent kernels,
+// energy_loss by the envelope (the others may be null).
+cudaError_t tangent_launch(tangent::Mode mode, const KArgs &a, double *jac, long long *log2_scale, double *fli,
+                           double *energy_loss, int threads, cudaStream_t st);
 
 // variant tables, one per translation unit (kernel family)
 const Variant *fast_lean_variants(int *n);

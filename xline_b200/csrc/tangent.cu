@@ -26,12 +26,7 @@ namespace tangent {
 using Jac = double[6][6];
 enum { X = 0, PX = 1, Y = 2, PY = 3, ZETA = 4, DELTA = 5 };
 
-// What the kernel body carries (include/xline_b200.h, "Tangent map"):
-//   TANGENT   J, no radiating records (tangent_kernel);
-//   TANGENT_R J, with mean-mode MULTIPOLE_RAD records (tangent_kernel_radiation);
-//   ENVELOPE  Sigma <- J_e Sigma J_e^T per element, plus the quantum diffusion of every radiating half
-//             (envelope_kernel).
-enum { TANGENT = 0, TANGENT_R = 1, ENVELOPE = 2 };
+// The kernel body is a template over what it carries, MODE (kargs.h: TANGENT, TANGENT_R, ENVELOPE).
 
 __device__ __forceinline__ void transpose(Jac &J) {
 #pragma unroll
@@ -113,22 +108,31 @@ __device__ __forceinline__ void jac_drift_exact(Jac &J, const Regs<1> &r, double
   }
 }
 
-// Thin multipole, straight or curved (el_multipole, el_multipole_curved; xline/elements.py:120-156).
-// pairs[m] = (kn, ks)[order - m] / (order - m)!: P(z) = sum (kn_i + i ks_i) z^i / i!, and
-// dpx = -chi Re P, dpy = chi Im P; P' comes from the same Horner sweep.
-__device__ __forceinline__ void jac_multipole(Jac &J, const Regs<1> &r, const double2 *pairs, int order,
-                                              bool curved, double hxl, double hyl, double inv_len) {
-  const double x = r.x[0], y = r.y[0], chi = r.chi[0];
-  double pr = pairs[0].x, pi = pairs[0].y, dr = 0.0, di = 0.0;
+// P' = dr + i di at z = x + i y of P(z) = sum (kn_i + i ks_i) z^i / i!, pairs[m] = (kn, ks)[order - m]
+// / (order - m)!: the Horner sweep of P carrying its derivative along.
+__device__ __forceinline__ void horner_prime(const double2 *pairs, int order, double x, double y, double &dr,
+                                             double &di) {
+  double pr = pairs[0].x, pi = pairs[0].y, qr = 0.0, qi = 0.0;
   for (int m = 1; m <= order; ++m) {
     const double2 k = pairs[m];
-    const double tr = fma(dr, x, fma(-di, y, pr)), ti = fma(dr, y, fma(di, x, pi));
-    dr = tr;
-    di = ti;
+    const double tr = fma(qr, x, fma(-qi, y, pr)), ti = fma(qr, y, fma(qi, x, pi));
+    qr = tr;
+    qi = ti;
     const double ur = fma(pr, x, fma(-pi, y, k.x)), ui = fma(pr, y, fma(pi, x, k.y));
     pr = ur;
     pi = ui;
   }
+  dr = qr;
+  di = qi;
+}
+
+// Thin multipole, straight or curved (el_multipole, el_multipole_curved; xline/elements.py:120-156):
+// dpx = -chi Re P, dpy = chi Im P.
+__device__ __forceinline__ void jac_multipole(Jac &J, const Regs<1> &r, const double2 *pairs, int order,
+                                              bool curved, double hxl, double hyl, double inv_len) {
+  const double x = r.x[0], y = r.y[0], chi = r.chi[0];
+  double dr, di;
+  horner_prime(pairs, order, x, y, dr, di);
   // d(-chi Re P)/dx = -chi Re P', /dy = chi Im P';  d(chi Im P)/dx = chi Im P', /dy = chi Re P'
   double axx = -chi * dr, axy = chi * di, ayx = chi * di, ayy = chi * dr, axd = 0.0, ayd = 0.0;
   double zx = 0.0, zy = 0.0;
@@ -151,33 +155,63 @@ __device__ __forceinline__ void jac_multipole(Jac &J, const Regs<1> &r, const do
 }
 
 // The chain through Pyparticles.add_to_energy (track_impl.cuh) of an energy change W whose
-// gradient over (x, y, zeta, delta) is (gx, gy, gz, gd); plus the px, py rows of a kick applied
-// before it (kx*, ky*: gradients of the px and py increments over x, y, zeta, delta).  Old rows
-// are read before any row is written.
-__device__ __forceinline__ void jac_energy(Jac &J, const Regs<1> &r, double beta0, double energy0, double W,
-                                           double gx, double gy, double gz, double gd, const double (&kx)[4],
+// gradient over (x, y, zeta, delta) is (gx, gy, gz, gd).  delta and rvv after it are functions of
+// P1 = 1 + ptau*beta0 after; zeta' = zeta rvv'/rvv.
+struct EnergyChain {
+  double opdn;                  // 1 + delta after
+  double dd_dP, drvv_dP;        // d delta' / d P1, d rvv' / d P1
+  double rr, zr, rv1;           // rvv'/rvv, zeta/rvv, d rvv / d delta before
+  double px_, py_, pz_, pd_;    // gradient of P1 over (x, y, zeta, delta)
+
+  __device__ __forceinline__ EnergyChain(const Regs<1> &r, double beta0, double energy0, double W, double gx,
+                                         double gy, double gz, double gd) {
+    const double delta = r.delta[0], rvv = r.rvv[0];
+    const double E = (1.0 + delta) / rvv;               // 1 + ptau*beta0 before
+    const double P1 = E + W / energy0;                  // 1 + ptau*beta0 after
+    const double ptau = (P1 - 1.0) / beta0;
+    opdn = sqrt(ptau * ptau + 2.0 * ptau / beta0 + 1.0);
+    const double rvvn = opdn / P1;                      // rvv after
+    dd_dP = P1 / (beta0 * beta0 * opdn);
+    drvv_dP = dd_dP / P1 - opdn / (P1 * P1);
+    rv1 = (1.0 - beta0 * beta0) / (E * E * E);
+    px_ = gx / energy0;
+    py_ = gy / energy0;
+    pz_ = gz / energy0;
+    pd_ = gd / energy0 + beta0 * beta0 * (1.0 + delta) / E;
+    zr = r.zeta[0] / rvv;
+    rr = rvvn / rvv;
+  }
+
+  // P1's entry in a column of J from the column's x, y, zeta, delta entries.  ZGRAD: W depends on
+  // zeta.  Without it the term is absent, not multiplied by 0 (which would turn an infinite jz
+  // into NaN).
+  template <bool ZGRAD>
+  __device__ __forceinline__ double dP(double jx, double jy, double jz, double jd) const {
+    return ZGRAD ? px_ * jx + py_ * jy + pz_ * jz + pd_ * jd : px_ * jx + py_ * jy + pd_ * jd;
+  }
+
+  // The delta and zeta entries of column c after the change, from P1's entry dP and the old zeta
+  // and delta entries; returns the new delta entry.
+  __device__ __forceinline__ double rows(Jac &J, int c, double dP, double jz, double jd) const {
+    const double jdn = dd_dP * dP;
+    J[DELTA][c] = jdn;
+    J[ZETA][c] = rr * jz + zr * drvv_dP * dP - zr * rr * rv1 * jd;
+    return jdn;
+  }
+};
+
+// The chain of an energy change, plus the px, py rows of a kick applied before it (kx*, ky*:
+// gradients of the px and py increments over x, y, zeta, delta).  Old rows are read before any
+// row is written.
+__device__ __forceinline__ void jac_energy(Jac &J, const EnergyChain &e, const double (&kx)[4],
                                            const double (&ky)[4]) {
-  const double delta = r.delta[0], rvv = r.rvv[0], zeta = r.zeta[0];
-  const double E = (1.0 + delta) / rvv;               // 1 + ptau*beta0 before
-  const double P1 = E + W / energy0;                  // 1 + ptau*beta0 after
-  const double ptau = (P1 - 1.0) / beta0;
-  const double opdn = sqrt(ptau * ptau + 2.0 * ptau / beta0 + 1.0);  // 1 + delta after
-  const double rvvn = opdn / P1;
-  const double dd_dP = P1 / (beta0 * beta0 * opdn);
-  const double drvv_dP = dd_dP / P1 - opdn / (P1 * P1);
-  const double rv1 = (1.0 - beta0 * beta0) / (E * E * E);
-  // gradient of P1 over (x, y, zeta, delta)
-  const double px_ = gx / energy0, py_ = gy / energy0, pz_ = gz / energy0;
-  const double pd_ = gd / energy0 + beta0 * beta0 * (1.0 + delta) / E;
-  const double zr = zeta / rvv;
 #pragma unroll
   for (int c = 0; c < 6; ++c) {
     const double jx = J[X][c], jy = J[Y][c], jz = J[ZETA][c], jd = J[DELTA][c];
-    const double dP = px_ * jx + py_ * jy + pz_ * jz + pd_ * jd;
+    const double dP = e.dP<true>(jx, jy, jz, jd);
     J[PX][c] += kx[0] * jx + kx[1] * jy + kx[2] * jz + kx[3] * jd;
     J[PY][c] += ky[0] * jx + ky[1] * jy + ky[2] * jz + ky[3] * jd;
-    J[DELTA][c] = dd_dP * dP;
-    J[ZETA][c] = (rvvn / rvv) * jz + zr * drvv_dP * dP - zr * (rvvn / rvv) * rv1 * jd;
+    e.rows(J, c, dP, jz, jd);
   }
 }
 
@@ -205,7 +239,8 @@ __device__ __forceinline__ void tan_cavity(Jac &J, const KArgs &a, Regs<1> &r, c
   const double gz = C * dw * (-c.x / (r.rvv[0] * a.beta0));
   const double gd = C * dw * (c.x * r.zeta[0] * rv1 / (r.rvv[0] * r.rvv[0] * a.beta0));
   const double none[4] = {0.0, 0.0, 0.0, 0.0};
-  TAN_ROWS(jac_energy(J, r, a.beta0, a.energy0, C * w, 0.0, 0.0, gz, gd, none, none));
+  const EnergyChain e(r, a.beta0, a.energy0, C * w, 0.0, 0.0, gz, gd);
+  TAN_ROWS(jac_energy(J, e, none, none));
   add_to_energy(C * w, a.beta0, a.energy0, r.delta[0], r.rpp[0], r.rvv[0], r.zeta[0]);
 }
 
@@ -262,7 +297,8 @@ __device__ __forceinline__ void tan_rfmultipole(Jac &J, const KArgs &a, Regs<1> 
   const double W = C * (V * sl - a.p0c * c.x * dptr);
   const double dW_dktau = C * (-V * cl + a.p0c * c.x * ar);
   const double gx = -C * a.p0c * c.x * br, gy = C * a.p0c * c.x * bi;
-  TAN_ROWS(jac_energy(J, r, a.beta0, a.energy0, W, gx, gy, dW_dktau * kz, dW_dktau * kd, kxv, kyv));
+  const EnergyChain e(r, a.beta0, a.energy0, W, gx, gy, dW_dktau * kz, dW_dktau * kd);
+  TAN_ROWS(jac_energy(J, e, kxv, kyv));
   r.px[0] = fma(-chi, dpx, r.px[0]);
   r.py[0] = fma(chi, dpy, r.py[0]);
   add_to_energy(W, a.beta0, a.energy0, r.delta[0], r.rpp[0], r.rvv[0], r.zeta[0]);
@@ -422,15 +458,27 @@ __device__ __forceinline__ void jac_spacecharge(Jac &J, const KArgs &a, const Re
   jac_field_kick(J, g * lam, g * dlz, g * dld, Ex, Ey, exx, exy, eyx, eyy);
 }
 
+// DRIFT / DRIFT_EXACT, and the drift fused into an aperture or space-charge record.
 template <int MODE>
-__device__ __forceinline__ void tan_drift(Jac &J, Regs<1> &r, double beta0, int aux, double L) {
-  if (aux & XLB_AUX_DRIFT_EXACT) {
+__device__ __forceinline__ void tan_drift(Jac &J, Regs<1> &r, double beta0, bool exact, double L) {
+  if (exact) {
     TAN_ROWS(jac_drift_exact(J, r, beta0, L));
     el_drift_exact<1>(r, L);
   } else {
     TAN_ROWS(jac_drift(J, r, beta0, L));
     el_drift<1>(r, L);
   }
+}
+
+// The end of an aperture record (LIMIT_*; the inside-tests are the tracker's, run_chunk): the
+// particle is lost unless `in`, with the s-word at cur[s_word] (apply_losses), then the record's
+// fused drift of length L, if any.  J is unchanged by the test.
+template <int MODE>
+__device__ __forceinline__ void tan_limit(Jac &J, const KArgs &a, Regs<1> &r, const double2 *cur, int aux,
+                                          bool in, int s_word, const double &L) {
+  const bool lost[1] = {r.alive(0) && !in};
+  apply_losses<1>(a, r, lost, cur, 1, s_word);
+  if (aux & XLB_AUX_DRIFT) tan_drift<MODE>(J, r, a.beta0, aux & XLB_AUX_DRIFT_EXACT, L);
 }
 
 // ---------------------------------------------------------------- mean-mode radiation
@@ -441,7 +489,7 @@ __device__ __forceinline__ void tan_drift(Jac &J, Regs<1> &r, double beta0, int 
 // caller passes fl^2's gradient (f2x, f2y) over (x, y).  With A = -(2/3) q0^2 K_e beta^3 gamma^4 / (L^2
 // (1+delta)^2) the loss is W = A fl^2 lh, whose gradient is taken through fl^2 (smooth where fl = 0,
 // unlike fl itself), and  d ln W / d delta = 1/(1+delta) + P p0c / E^2  (W ~ (1+delta) E).  Then
-// add_to_energy(W) through the chain of jac_energy, and px, py times f = (1+delta')/(1+delta):
+// add_to_energy(W) through EnergyChain, and px, py times f = (1+delta')/(1+delta):
 //   row(px) <- f row(px) + px (row(delta') - f row(delta)) / (1+delta),  the same for py.
 // ENVELOPE: Sigma += V_h g g^T with V_h = nbar (11/27) u_c^2, the variance of the quantum mode's
 // loss over the half (nbar, u_c of include/xline_b200.h), and g = dz_after/dW; `eloss` -= W.
@@ -468,29 +516,14 @@ __device__ __forceinline__ void tan_radiate_half(Jac &J, const KArgs &a, Regs<1>
   const double gx = A * (f2x * lh + fl2 * (0.5 * hxl));
   const double gy = A * (f2y * lh - fl2 * (0.5 * hyl));
   const double gd = dE * (1.0 / opd + P * a.p0c / (E * E));
-  // the chain of add_to_energy (jac_energy) with the scaling of px, py
-  const double beta0 = a.beta0, energy0 = a.energy0;
-  const double delta = r.delta[0], rvv = r.rvv[0], zeta = r.zeta[0], px = r.px[0], py = r.py[0];
-  const double Eb = opd / rvv;
-  const double P1 = Eb + dE / energy0;
-  const double ptau = (P1 - 1.0) / beta0;
-  const double opdn = sqrt(ptau * ptau + 2.0 * ptau / beta0 + 1.0);
-  const double rvvn = opdn / P1;
-  const double dd_dP = P1 / (beta0 * beta0 * opdn);
-  const double drvv_dP = dd_dP / P1 - opdn / (P1 * P1);
-  const double rv1 = (1.0 - beta0 * beta0) / (Eb * Eb * Eb);
-  const double px_ = gx / energy0, py_ = gy / energy0;
-  const double pd_ = gd / energy0 + beta0 * beta0 * (1.0 + delta) / Eb;
-  const double zr = zeta / rvv;
-  const double f = opdn / opd, xo = px / opd, yo = py / opd;
+  // the chain of add_to_energy (no zeta gradient) with the scaling of px, py
+  const EnergyChain e(r, a.beta0, a.energy0, dE, gx, gy, 0.0, gd);
+  const double f = e.opdn / opd, xo = r.px[0] / opd, yo = r.py[0] / opd;
   TAN_ROWS(
       _Pragma("unroll")
       for (int c = 0; c < 6; ++c) {
         const double jx = J[X][c], jy = J[Y][c], jz = J[ZETA][c], jd = J[DELTA][c];
-        const double dP = px_ * jx + py_ * jy + pd_ * jd;
-        const double jdn = dd_dP * dP;
-        J[DELTA][c] = jdn;
-        J[ZETA][c] = (rvvn / rvv) * jz + zr * drvv_dP * dP - zr * (rvvn / rvv) * rv1 * jd;
+        const double jdn = e.rows(J, c, e.dP<false>(jx, jy, jz, jd), jz, jd);
         J[PX][c] = f * J[PX][c] + xo * (jdn - f * jd);
         J[PY][c] = f * J[PY][c] + yo * (jdn - f * jd);
       });
@@ -498,8 +531,8 @@ __device__ __forceinline__ void tan_radiate_half(Jac &J, const KArgs &a, Regs<1>
     const double nbar = (5.0 / (2.0 * 1.7320508075688772)) * q2 * al.x * gamma * kappa * lh;
     const double uc = 1.5 * ke.y * (gamma * g2) * kappa;
     const double V = nbar * (11.0 / 27.0) * (uc * uc);
-    const double gdw = dd_dP / energy0;
-    const double g[6] = {0.0, xo * gdw, 0.0, yo * gdw, zr * drvv_dP / energy0, gdw};
+    const double gdw = e.dd_dP / a.energy0;
+    const double g[6] = {0.0, xo * gdw, 0.0, yo * gdw, e.zr * e.drvv_dP / a.energy0, gdw};
 #pragma unroll
     for (int q = 0; q < 6; ++q)
 #pragma unroll
@@ -525,17 +558,8 @@ __device__ __forceinline__ void tan_multipole_rad(Jac &J, const KArgs &a, Regs<1
   const double x = r.x[0], y = r.y[0];
   double dpx[1], dpy[1];
   horner<1>(r, pairs, order, dpx, dpy);  // the tracker's field kick, bit for bit
-  // P' = dr + i di from the Horner sweep of jac_multipole
-  double pr = pairs[0].x, pi = pairs[0].y, dr = 0.0, di = 0.0;
-  for (int m = 1; m <= order; ++m) {
-    const double2 k = pairs[m];
-    const double tr = fma(dr, x, fma(-di, y, pr)), ti = fma(dr, y, fma(di, x, pi));
-    dr = tr;
-    di = ti;
-    const double ur = fma(pr, x, fma(-pi, y, k.x)), ui = fma(pr, y, fma(pi, x, k.y));
-    pr = ur;
-    pi = ui;
-  }
+  double dr, di;
+  horner_prime(pairs, order, x, y, dr, di);
   // fl^2 = (Re P)^2 + (Im P)^2:  d/dx = 2 (Re P Re P' + Im P Im P'),  d/dy = 2 (Im P Re P' - Re P Im P')
   const double f2x = 2.0 * (dpx[0] * dr + dpy[0] * di), f2y = 2.0 * (dpy[0] * dr - dpx[0] * di);
   const double fl = sqrt(fma(dpx[0], dpx[0], dpy[0] * dpy[0]));
@@ -552,27 +576,46 @@ __device__ __forceinline__ void tan_multipole_rad(Jac &J, const KArgs &a, Regs<1
   if (r.alive(0)) tan_radiate_half<MODE>(J, a, r, rec, fl, lh, f2x, f2y, hxl, hyl, eloss);
 }
 
+// One argument block for the three kernels; each uses the outputs of its mode.
 struct TArgs {
   KArgs k;
-  double *jac;            // [n][6][6]
-  long long *log2_scale;  // [n]
-  double *fli;            // [n]
+  double *jac;            // [n][6][6]: J, or Sigma (ENVELOPE)
+  long long *log2_scale;  // [n], TANGENT and TANGENT_R
+  double *fli;            // [n], TANGENT and TANGENT_R
+  double *energy_loss;    // [n], ENVELOPE
 };
 
-// envelope_kernel: t.jac is Sigma [n][6][6]; log2_scale and fli are not used
-struct EArgs {
-  TArgs t;
-  double *energy_loss;  // [n]
-};
+// J (or Sigma) of particle k (< n), and what the mode accumulates with it: the exponent and the
+// FLI, or the energy lost (eV).  J's 36 words are addressed with k, the other arrays with int(k).
+template <int MODE>
+__device__ __forceinline__ void load(const TArgs &t, long long k, Jac &J, long long &l2s, double &fli, double &el) {
+  const double *jin = t.jac + k * 36;
+  const int i = static_cast<int>(k);
+#pragma unroll
+  for (int q = 0; q < 6; ++q)
+#pragma unroll
+    for (int c = 0; c < 6; ++c) J[q][c] = jin[q * 6 + c];
+  if (MODE == ENVELOPE) {
+    el = t.energy_loss[i];
+  } else {
+    l2s = t.log2_scale[i];
+    fli = t.fli[i];
+  }
+}
 
-__device__ __forceinline__ void store_tangent(const TArgs &t, int i, const Jac &J, long long l2s, double fli) {
+template <int MODE>
+__device__ __forceinline__ void store(const TArgs &t, int i, const Jac &J, long long l2s, double fli, double el) {
   double *o = t.jac + static_cast<long long>(i) * 36;
 #pragma unroll
   for (int q = 0; q < 6; ++q)
 #pragma unroll
     for (int c = 0; c < 6; ++c) o[q * 6 + c] = J[q][c];
-  t.log2_scale[i] = l2s;
-  t.fli[i] = fli;
+  if (MODE == ENVELOPE) {
+    t.energy_loss[i] = el;
+  } else {
+    t.log2_scale[i] = l2s;
+    t.fli[i] = fli;
+  }
 }
 
 // End of a turn: the exact overflow guard, then the FLI.
@@ -605,25 +648,6 @@ __device__ __forceinline__ void end_turn(Jac &J, long long &l2s, double &fli) {
   fli = fmax(fli, f);
 }
 
-// The envelope's store: Sigma and the energy lost.
-__device__ __forceinline__ void store_envelope(const TArgs &t, double *eloss, int i, const Jac &S, double el) {
-  double *o = t.jac + static_cast<long long>(i) * 36;
-#pragma unroll
-  for (int q = 0; q < 6; ++q)
-#pragma unroll
-    for (int c = 0; c < 6; ++c) o[q * 6 + c] = S[q][c];
-  eloss[i] = el;
-}
-
-template <int MODE>
-__device__ __forceinline__ void store(const TArgs &t, double *eloss, int i, const Jac &J, long long l2s, double fli,
-                                      double el) {
-  if (MODE == ENVELOPE)
-    store_envelope(t, eloss, i, J, el);
-  else
-    store_tangent(t, i, J, l2s, fli);
-}
-
 // End of an envelope turn: Sigma made exactly symmetric (F(F(Sigma)^T) is symmetric up to rounding).
 __device__ __forceinline__ void symmetrize(Jac &S) {
 #pragma unroll
@@ -633,7 +657,7 @@ __device__ __forceinline__ void symmetrize(Jac &S) {
 }
 
 template <int MODE>
-__device__ __forceinline__ void tangent_body(const TArgs &t, double *eloss) {
+__device__ __forceinline__ void tangent_body(const TArgs &t) {
   const KArgs &a = t.k;
   const long long k = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   Regs<1> r;
@@ -655,17 +679,7 @@ __device__ __forceinline__ void tangent_body(const TArgs &t, double *eloss) {
       r.rpp[0] = a.rpp[i];
       r.rvv[0] = a.rvv[i];
       r.chi[0] = a.chi ? a.chi[i] : 1.0;
-      const double *jin = t.jac + k * 36;
-#pragma unroll
-      for (int q = 0; q < 6; ++q)
-#pragma unroll
-        for (int c = 0; c < 6; ++c) J[q][c] = jin[q * 6 + c];
-      if (MODE == ENVELOPE) {
-        el = eloss[i];
-      } else {
-        l2s = t.log2_scale[i];
-        fli = t.fli[i];
-      }
+      load<MODE>(t, k, J, l2s, fli, el);
     }
   }
   if (r.slot[0] < 0) {
@@ -701,12 +715,10 @@ __device__ __forceinline__ void tangent_body(const TArgs &t, double *eloss) {
       }
       switch (tag) {
         case XLB_T_DRIFT:
-          TAN_ROWS(jac_drift(J, r, a.beta0, p0));
-          el_drift<1>(r, p0);
+          tan_drift<MODE>(J, r, a.beta0, false, p0);
           break;
         case XLB_T_DRIFT_EXACT:
-          TAN_ROWS(jac_drift_exact(J, r, a.beta0, p0));
-          el_drift_exact<1>(r, p0);
+          tan_drift<MODE>(J, r, a.beta0, true, p0);
           break;
         case XLB_T_MULTIPOLE:
           TAN_ROWS(jac_multipole(J, r, cur + 1, aux, false, 0.0, 0.0, 0.0));
@@ -762,17 +774,13 @@ __device__ __forceinline__ void tangent_body(const TArgs &t, double *eloss) {
             in = (fabs(r.x[0]) <= c1.x) & (fabs(r.y[0]) <= c2.x);
           else
             in = (r.x[0] >= p0) & (r.x[0] <= c1.x) & (r.y[0] >= c1.y) & (r.y[0] <= c2.x);
-          const bool lost[1] = {r.alive(0) && !in};
-          apply_losses<1>(a, r, lost, cur, 1, 5);
-          if (aux & XLB_AUX_DRIFT) tan_drift<MODE>(J, r, a.beta0, aux, cur[3].x);
+          tan_limit<MODE>(J, a, r, cur, aux, in, 5, cur[3].x);
           break;
         }
         case XLB_T_LIMIT_ELLIPSE: {
           const double2 c1 = cur[1], c2 = cur[2];
           const double q = fma(r.x[0] * r.x[0], c1.y, (r.y[0] * r.y[0]) * c2.x);
-          const bool lost[1] = {r.alive(0) && !(q <= 1.0)};
-          apply_losses<1>(a, r, lost, cur, 1, 5);
-          if (aux & XLB_AUX_DRIFT) tan_drift<MODE>(J, r, a.beta0, aux, cur[3].x);
+          tan_limit<MODE>(J, a, r, cur, aux, q <= 1.0, 5, cur[3].x);
           break;
         }
         case XLB_T_LIMIT_RECT_ELLIPSE: {
@@ -780,9 +788,7 @@ __device__ __forceinline__ void tangent_body(const TArgs &t, double *eloss) {
           const double2 c1 = cur[1], c2 = cur[2], c3 = cur[3];
           const double q = fma(r.x[0] * r.x[0], c2.y, (r.y[0] * r.y[0]) * c3.x);
           const bool in = (r.x[0] >= -mx) & (r.x[0] <= mx) & (r.y[0] >= -c1.x) & (r.y[0] <= c1.x) & (q <= 1.0);
-          const bool lost[1] = {r.alive(0) && !in};
-          apply_losses<1>(a, r, lost, cur, 1, 7);
-          if (aux & XLB_AUX_DRIFT) tan_drift<MODE>(J, r, a.beta0, aux, cur[4].x);
+          tan_limit<MODE>(J, a, r, cur, aux, in, 7, cur[4].x);
           break;
         }
         case XLB_T_LIMIT_POLYGON: {
@@ -790,9 +796,7 @@ __device__ __forceinline__ void tangent_body(const TArgs &t, double *eloss) {
           const double2 *e = cur + 2;
           bool odd = false;
           for (int q = 0; q < n_edges; ++q, e += 2) odd ^= polygon_edge_crossed(r.x[0], r.y[0], e[0], e[1]);
-          const bool lost[1] = {r.alive(0) && !odd};
-          apply_losses<1>(a, r, lost, cur, 1, 2);
-          if (aux & XLB_AUX_DRIFT) tan_drift<MODE>(J, r, a.beta0, aux, cur[1].y);
+          tan_limit<MODE>(J, a, r, cur, aux, odd, 2, cur[1].y);
           break;
         }
         case XLB_T_BEAMBEAM4D:
@@ -802,13 +806,13 @@ __device__ __forceinline__ void tangent_body(const TArgs &t, double *eloss) {
         case XLB_T_SPACECHARGE:
           TAN_ROWS(jac_spacecharge(J, a, r, cur, aux & 0xf));
           bf::spacecharge<1>(a, r, cur, aux & 0xf);
-          if (aux & XLB_AUX_DRIFT) tan_drift<MODE>(J, r, a.beta0, aux, p0);
+          if (aux & XLB_AUX_DRIFT) tan_drift<MODE>(J, r, a.beta0, aux & XLB_AUX_DRIFT_EXACT, p0);
           break;
         default:  // XLB_T_MONITOR: the identity, nothing stored.  The host refuses every other tag.
           if (MODE != TANGENT && tag == XLB_T_MULTIPOLE_RAD) tan_multipole_rad<MODE>(J, a, r, cur, aux, el);
           break;
       }
-      if (was_alive && !r.alive(0)) store<MODE>(t, eloss, static_cast<int>(k), J, l2s, fli, el);  // frozen where lost
+      if (was_alive && !r.alive(0)) store<MODE>(t, static_cast<int>(k), J, l2s, fli, el);  // frozen where lost
     }
     if (r.alive(0)) {
       if (MODE == ENVELOPE)
@@ -831,57 +835,30 @@ __device__ __forceinline__ void tangent_body(const TArgs &t, double *eloss) {
     a.s[i] = a.s[i] + r.s_acc;
     a.at_turn[i] = a.at_turn[i] + r.turns_done;
     a.at_element[i] = 0;
-    store<MODE>(t, eloss, i, J, l2s, fli, el);
+    store<MODE>(t, i, J, l2s, fli, el);
   }
 }
 
-__global__ void __launch_bounds__(256) tangent_kernel(const __grid_constant__ TArgs t) {
-  tangent_body<TANGENT>(t, nullptr);
-}
+__global__ void __launch_bounds__(256) tangent_kernel(const __grid_constant__ TArgs t) { tangent_body<TANGENT>(t); }
 
 __global__ void __launch_bounds__(256) tangent_kernel_radiation(const __grid_constant__ TArgs t) {
-  tangent_body<TANGENT_R>(t, nullptr);
+  tangent_body<TANGENT_R>(t);
 }
 
-__global__ void __launch_bounds__(256) envelope_kernel(const __grid_constant__ EArgs e) {
-  tangent_body<ENVELOPE>(e.t, e.energy_loss);
-}
+__global__ void __launch_bounds__(256) envelope_kernel(const __grid_constant__ TArgs t) { tangent_body<ENVELOPE>(t); }
 
 }  // namespace tangent
 
-cudaError_t tangent_launch(const KArgs &a, double *jac, long long *log2_scale, double *fli, int threads,
-                           cudaStream_t st) {
-  tangent::TArgs t;
-  t.k = a;
-  t.jac = jac;
-  t.log2_scale = log2_scale;
-  t.fli = fli;
-  const long long blocks = (a.n + threads - 1) / threads;
-  tangent::tangent_kernel<<<static_cast<unsigned>(blocks), threads, 0, st>>>(t);
-  return cudaGetLastError();
-}
-
-cudaError_t tangent_radiation_launch(const KArgs &a, double *jac, long long *log2_scale, double *fli, int threads,
-                                     cudaStream_t st) {
-  tangent::TArgs t;
-  t.k = a;
-  t.jac = jac;
-  t.log2_scale = log2_scale;
-  t.fli = fli;
-  const long long blocks = (a.n + threads - 1) / threads;
-  tangent::tangent_kernel_radiation<<<static_cast<unsigned>(blocks), threads, 0, st>>>(t);
-  return cudaGetLastError();
-}
-
-cudaError_t envelope_launch(const KArgs &a, double *cov, double *energy_loss, int threads, cudaStream_t st) {
-  tangent::EArgs e;
-  e.t.k = a;
-  e.t.jac = cov;
-  e.t.log2_scale = nullptr;
-  e.t.fli = nullptr;
-  e.energy_loss = energy_loss;
-  const long long blocks = (a.n + threads - 1) / threads;
-  tangent::envelope_kernel<<<static_cast<unsigned>(blocks), threads, 0, st>>>(e);
+cudaError_t tangent_launch(tangent::Mode mode, const KArgs &a, double *jac, long long *log2_scale, double *fli,
+                           double *energy_loss, int threads, cudaStream_t st) {
+  const tangent::TArgs t = {a, jac, log2_scale, fli, energy_loss};
+  const unsigned blocks = static_cast<unsigned>((a.n + threads - 1) / threads);
+  if (mode == tangent::ENVELOPE)
+    tangent::envelope_kernel<<<blocks, threads, 0, st>>>(t);
+  else if (mode == tangent::TANGENT_R)
+    tangent::tangent_kernel_radiation<<<blocks, threads, 0, st>>>(t);
+  else
+    tangent::tangent_kernel<<<blocks, threads, 0, st>>>(t);
   return cudaGetLastError();
 }
 

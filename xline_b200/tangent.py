@@ -57,14 +57,21 @@ class TangentMap:
         return torch.ldexp(self.jacobian, self.log2_scale.to(torch.float64)[:, None, None])
 
     def _check_target(self, p):
-        if len(self) != len(p):
-            raise ValueError("TangentMap holds %d particles, the beam %d" % (len(self), len(p)))
-        if self.jacobian.device != p.x.device:
-            raise ValueError("TangentMap is on %s, the particles on %s" % (self.jacobian.device, p.x.device))
-        for name in ("jacobian", "log2_scale", "fli"):
-            t = getattr(self, name)
-            if not t.is_contiguous():
-                setattr(self, name, t.contiguous())
+        _check_target(self, p, ("jacobian", "log2_scale", "fli"))
+
+
+def _check_target(holder, p, names):
+    """Refuse a TangentMap or Envelope of another size or device than ``p``; make its tensors
+    ``names`` contiguous."""
+    what = type(holder).__name__
+    if len(holder) != len(p):
+        raise ValueError("%s holds %d particles, the beam %d" % (what, len(holder), len(p)))
+    if holder.device != p.x.device:
+        raise ValueError("%s is on %s, the particles on %s" % (what, holder.device, p.x.device))
+    for name in names:
+        t = getattr(holder, name)
+        if not t.is_contiguous():
+            setattr(holder, name, t.contiguous())
 
 
 def _launch(line, p, num_turns, threads_per_block, radiation, call):
@@ -137,14 +144,7 @@ class Envelope:
         return self.cov.device
 
     def _check_target(self, p):
-        if len(self) != len(p):
-            raise ValueError("Envelope holds %d particles, the beam %d" % (len(self), len(p)))
-        if self.cov.device != p.x.device:
-            raise ValueError("Envelope is on %s, the particles on %s" % (self.cov.device, p.x.device))
-        for name in ("cov", "energy_loss"):
-            t = getattr(self, name)
-            if not t.is_contiguous():
-                setattr(self, name, t.contiguous())
+        _check_target(self, p, ("cov", "energy_loss"))
 
 
 def track_envelope(line, p, envelope, num_turns=1, threads_per_block=0):
