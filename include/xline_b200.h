@@ -163,6 +163,35 @@ enum xlb_tag {
      the lattice in xlb_lattice_validate ("unknown tag").                                       */
   XLB_T_MULTIPOLE_RAD = 20,
   XLB_T__COUNT = 21,
+  /* Exciter (DESIGN.md §4.11): a thin multipole whose strength is read, per particle, from a sampled
+     waveform by turn and arrival time -- AC dipole, power-converter ripple, transverse excitation.
+     It lies outside the contiguous single-element tags 0 .. XLB_T__COUNT-1, which keep their meaning
+     for code written against them (a scan that refuses tag >= XLB_T__COUNT still refuses it); 0x40
+     has bit 7 clear, so none of the block-family masks (tag & 0xc0 == 0x80, tag & 0xe0) match it.
+     0x40 is the one valid tag in 0x40 .. 0x7f; every other value there is an unknown tag.  Fast
+     encoding only.  aux = order;
+       [hdr,A][B,i64 start_turn][i64 n_samples,i64 data_offset] then (kn_i,ks_i) i=order..0
+     with kn_i = knl[i]/i! as in MULTIPOLE, A = sampling_frequency/frev and B = sampling_frequency/c
+     taken at pack time.  The samples are n_samples fp64 words at words[data_offset ..], in the data
+     region after the chunks (see xlb_lattice_t::n_words): data_offset is an absolute word index.
+     Map, for a particle at turn T (its at_turn: the stored value + the turns of this call, as BeamMonitor
+     takes it) with beta0 from the call's reference particle:
+       t = (double)(T - start_turn)                 exact for |T - start_turn| < 2^53
+       u = t*A - (zeta*B)/beta0                      the products, the quotient and the difference
+       v = floor(u + 0.5)                            each rounded to nearest, no fused multiply-add
+                                                     (a quotient off by an ulp where |zeta*B| < 2^-960
+                                                     leaves u unchanged: the kernel's reciprocal form)
+       s = samples[(int64)v] if 0 <= v < n_samples, else 0 (no kick; a NaN or infinite zeta gives none)
+       (Px, Py) = the Horner polynomial of knl/ksl at (x, y), as MULTIPOLE (straight: no hxl/hyl)
+       px <- px - chi*(s*Px),  py <- py + chi*(s*Py)
+     The index is a fixed sequence of IEEE operations, so every implementation picks the same sample;
+     rounding to nearest makes a particle with |zeta| < C/2 read the sample of its own turn when
+     sampling_frequency == frev.  A lattice with these records carries XLB_F_EXCITER.  Refused: a
+     strict or segmented lattice (XLB_ELATTICE; a segment's kernel sees the segment's first chunk as
+     word 0) and the tangent and envelope entry points (XLB_EINVAL: a
+     turn-dependent map has no closed orbit).  Added without an ABI version change: a library that
+     predates the tag refuses the lattice in xlb_lattice_validate ("unknown tag").                */
+  XLB_T_EXCITER = 0x40,
   /* Fused thin multipole -> [aperture] -> [drift] records (pack-time peephole).  The tag
      has bit 7 set and describes the block: bits 0-1 aperture kind (0 none, 1 symmetric
      rect, 2 rect, 3 ellipse), bit 2 curved multipole, bit 3 drift present, bit 4 that drift
@@ -200,7 +229,10 @@ enum xlb_tag {
 #define XLB_HDR_HAS_A1 0x40000000u
 
 typedef struct xlb_lattice {
-  const uint64_t *words; /* n_chunks * chunk_words words                                */
+  const uint64_t *words; /* n_chunks * chunk_words words, then the data region (if any)  */
+  /* n_chunks * chunk_words, plus the words of the data region on a lattice flagged XLB_F_EXCITER:
+     n_data_words fp64 words after the last chunk that hold the exciters' waveforms.  The kernels
+     stream the chunks only; they read the data region through the read-only data path.          */
   int64_t n_words;
   int32_t chunk_words;   /* even, 16 <= chunk_words*8 <= 96 KiB                         */
   int32_t n_chunks;
@@ -234,6 +266,9 @@ typedef struct xlb_lattice {
 #define XLB_F_RADIATION 32u  /* the lattice holds MULTIPOLE_RAD records (mandatory: checked by
                                 xlb_lattice_validate; only the one-species thin-lens fast
                                 kernels carry the case)                                  */
+#define XLB_F_EXCITER 64u    /* the lattice holds EXCITER records (mandatory: checked by
+                                xlb_lattice_validate, which accepts a data region after the chunks
+                                only with this flag; the kernels that carry the case are used) */
 #define XLB_RAD_MEAN 1
 #define XLB_RAD_QUANTUM 2
 #define XLB_RAD_MAX_ELEMENTS (1 << 24)
@@ -432,7 +467,7 @@ int xlb_naff_device(const double *u, const double *pu, int64_t n, int64_t num_tu
  * orbits and one-turn matrices of the tracked map itself.
  *
  * Lattice: one record per element -- no block records (tags >= 0x80), no segments, the fast
- *   encoding (XLB_F_STRICT clear); BEAMBEAM6D is refused.  MONITOR records are the identity and
+ *   encoding (XLB_F_STRICT clear); BEAMBEAM6D and EXCITER are refused.  MONITOR records are the identity and
  *   store nothing.  rpp and rvv are functions of delta throughout.
  * Layout: jac[i*36 + r*6 + c] = dz_r/dz0_c of particle i (row-major 6x6, r, c in the order of z);
  *   the caller initialises it (the identity for a fresh start).  The true Jacobian is

@@ -308,7 +308,7 @@ struct Need {
 static bool admits(const Variant &v, const Need &q) {
   if ((v.strict != 0) != q.strict) return false;
   if ((v.radiation != 0) != q.radiation) return false;  // the twins with the MULTIPOLE_RAD case
-  // the twins with the LIMIT_POLYGON case (the radiation twins carry it as well)
+  // the twins with the LIMIT_POLYGON and EXCITER cases (the radiation twins carry them as well)
   if (!q.radiation && (v.polygons != 0) != q.polygons) return false;
   if (q.strict) return (v.beamfields != 0) == q.beamfields;
   const int bf = q.beamfields ? (q.bb6d ? 2 : 1) : 0;
@@ -391,8 +391,12 @@ static int check_lattice_header(const xlb_lattice_t *lat) {
   if (static_cast<long long>(lat->chunk_words) * 8 > 96 * 1024)
     return fail(XLB_ELATTICE, "chunk larger than 96 KiB");
   if (lat->n_chunks < 1) return fail(XLB_ELATTICE, "n_chunks < 1");
-  if (lat->n_words != static_cast<int64_t>(lat->chunk_words) * lat->n_chunks)
+  const int64_t chunk_region = static_cast<int64_t>(lat->chunk_words) * lat->n_chunks;
+  if (lat->flags & XLB_F_EXCITER) {  // the chunks, then the exciters' data region
+    if (lat->n_words < chunk_region) return fail(XLB_ELATTICE, "n_words < chunk_words * n_chunks");
+  } else if (lat->n_words != chunk_region) {
     return fail(XLB_ELATTICE, "n_words != chunk_words * n_chunks");
+  }
   if (reinterpret_cast<uintptr_t>(lat->words) & 15)
     return fail(XLB_ELATTICE, "lattice words must be 16-byte aligned");
   if (lat->n_segments < 0 || (lat->n_segments > 0 && !lat->segments))
@@ -441,6 +445,8 @@ static int check_call(const xlb_lattice_t *lat, const xlb_particles_t *p, const 
     return fail(XLB_EINVAL, "element-by-element trace needs num_turns == 1 and trace_particles >= 1");
   if (lat->n_segments > 1 && (o->trace || (lat->flags & XLB_F_STRICT)))
     return fail(XLB_EINVAL, "segmented lattices are for the fast kernels without trace");
+  if ((lat->flags & XLB_F_EXCITER) && ((lat->flags & XLB_F_STRICT) || lat->n_segments > 0))
+    return fail(XLB_ELATTICE, "exciter: a strict or segmented lattice cannot carry exciters");
   if (lat->flags & XLB_F_RADIATION) {
     if (lat->flags & (XLB_F_STRICT | XLB_F_BEAMFIELDS | XLB_F_BB6D))
       return fail(XLB_ELATTICE, "radiation: a strict or beam-field lattice cannot carry radiating multipoles");
@@ -557,7 +563,7 @@ static int track_device_impl(const xlb_lattice_t *lat, xlb_particles_t *p,
   const bool split = lat->n_segments > 1;  // 6D lenses run as kernels of their own
   const Need need{(lat->flags & XLB_F_STRICT) != 0, (lat->flags & XLB_F_BEAMFIELDS) != 0,
                   (lat->flags & XLB_F_BB6D) != 0 && !split, p->chi != nullptr, o->trace != nullptr,
-                  (lat->flags & XLB_F_POLYGONS) != 0, (lat->flags & XLB_F_LOW_ORDER) ? 3 : 255,
+                  (lat->flags & (XLB_F_POLYGONS | XLB_F_EXCITER)) != 0, (lat->flags & XLB_F_LOW_ORDER) ? 3 : 255,
                   (lat->flags & XLB_F_RADIATION) != 0};
   const size_t smem = XLB_STAGES * static_cast<size_t>(lat->chunk_words) * 8 +
                       (2 * XLB_STAGES + 2) * sizeof(unsigned long long);
@@ -814,6 +820,27 @@ int xlb_lattice_validate(const xlb_lattice_t *lat) {
           want = 4 + spairs;
           break;
         }
+        case XLB_T_EXCITER: {  // [hdr,A][B,start_turn][n_samples,data_offset] + (kn_i,ks_i) i=order..0
+          if (!(lat->flags & XLB_F_EXCITER)) return fail(XLB_ELATTICE, "exciter record without XLB_F_EXCITER");
+          if ((lat->flags & XLB_F_LOW_ORDER) && aux > 3)
+            return fail(XLB_ELATTICE, "XLB_F_LOW_ORDER set but an exciter has order > 3");
+          if (pos + 6 > lat->chunk_words) return fail(XLB_ELATTICE, "record runs past the end of its chunk");
+          double ab[2];
+          memcpy(&ab[0], &w[pos + 1], sizeof(double));
+          memcpy(&ab[1], &w[pos + 2], sizeof(double));
+          if (!(std::isfinite(ab[0]) && std::isfinite(ab[1]))) return fail(XLB_ELATTICE, "exciter: A or B not finite");
+          const int64_t n_samples = static_cast<int64_t>(w[pos + 4]), off = static_cast<int64_t>(w[pos + 5]);
+          const int64_t chunk_region = static_cast<int64_t>(lat->chunk_words) * lat->n_chunks;
+          if (n_samples < 0 || off < chunk_region || off > lat->n_words || n_samples > lat->n_words - off)
+            return fail(XLB_ELATTICE, "exciter: the samples are not inside the data region");
+          for (int64_t k = 0; k < n_samples; ++k) {
+            double v;
+            memcpy(&v, &lat->words[off + k], sizeof v);
+            if (!std::isfinite(v)) return fail(XLB_ELATTICE, "exciter: non-finite sample");
+          }
+          want = 3 + aux + 1;
+          break;
+        }
         case XLB_T_MONITOR: want = 5; break;
         case XLB_T_BEAMBEAM4D:
         case XLB_T_SPACECHARGE:
@@ -882,6 +909,8 @@ int xlb_lattice_validate(const xlb_lattice_t *lat) {
     if (!closed) return fail(XLB_ELATTICE, "chunk not terminated by END_CHUNK/END_TURN");
   }
   if (!saw_end_turn) return fail(XLB_ELATTICE, "no END_TURN record");
+  if ((lat->flags & XLB_F_EXCITER) && ((lat->flags & XLB_F_STRICT) || lat->n_segments > 0))
+    return fail(XLB_ELATTICE, "exciter: a strict or segmented lattice cannot carry exciters");
   if (lat->flags & XLB_F_RADIATION) {
     if (lat->flags & XLB_F_STRICT) return fail(XLB_ELATTICE, "radiation: the strict encoding has no radiating multipoles");
     if (lat->flags & (XLB_F_BEAMFIELDS | XLB_F_BB6D))
@@ -986,6 +1015,7 @@ static int tangent_scan(const xlb_lattice_t *lat, bool radiation, const char *wh
         char buf[160];
         snprintf(buf, sizeof buf, "%s: element %d is %s", what, static_cast<int>(hdr >> 32),
                  tag == XLB_T_BEAMBEAM6D ? "a BeamBeam6D lens (its Jacobian is not implemented)"
+                 : tag == XLB_T_EXCITER  ? "an Exciter (a turn-dependent map has no tangent map or closed orbit)"
                                          : "a fused block record (pack one record per element)");
         return fail(XLB_EINVAL, buf);
       }

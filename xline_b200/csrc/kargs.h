@@ -47,7 +47,7 @@ struct Variant {
   int strict, beamfields, ppt, threads, trace;
   int nochi;     // 1 = compiled for chi == 1 throughout (xlb_particles_t::chi == NULL)
   int maxorder;  // 0 = any multipole order; else the highest order the kernel evaluates (XLB_F_LOW_ORDER)
-  int polygons;  // 1 = track_kernel_polygons: for the lattices flagged XLB_F_POLYGONS, and only those
+  int polygons;  // 1 = track_kernel_polygons: for the lattices flagged XLB_F_POLYGONS or XLB_F_EXCITER, only those
   int radiation;  // 1 = track_kernel_radiation (with the polygon case too): for XLB_F_RADIATION, and only those
   const void *func;  // the kernel's host stub
 };

@@ -17,7 +17,7 @@ __all__ = [
     "Element", "Drift", "DriftExact", "Multipole", "RFMultipole", "Cavity", "SawtoothCavity",
     "XYShift", "SRotation", "LimitRect", "LimitEllipse", "LimitRectEllipse", "BeamMonitor",
     "DipoleEdge", "BeamBeam4D", "BeamBeam6D", "SCCoasting", "SCQGaussProfile",
-    "SCInterpolatedProfile", "Elens", "LimitPolygon", "element_classes",
+    "SCInterpolatedProfile", "Elens", "LimitPolygon", "Exciter", "element_classes",
 ]
 
 
@@ -324,6 +324,25 @@ class LimitPolygon(Element):
     The MAD-X ``octagon`` aperture (xline/loader_mad.py:229-242) maps to this class."""
 
     _base = (("x_vertices", tuple), ("y_vertices", tuple))
+
+
+class Exciter(Element):
+    """Thin multipole whose strength follows a sampled waveform: an AC dipole, power-converter ripple
+    or a transverse excitation (damper noise, chirps).  The field names follow xtrack's ``Exciter``;
+    the map is this project's own (include/xline_b200.h, DESIGN.md §4.11).  A particle at turn ``T``
+    (its ``at_turn``) with longitudinal position ``zeta`` reads sample
+    ``floor((T - start_turn) * sampling_frequency / frev - zeta * sampling_frequency / (c beta0) + 1/2)``
+    -- with ``sampling_frequency == frev`` the sample of its own turn -- and receives the kick of
+    ``Multipole(knl, ksl)`` times that sample; before the first sample and after the last it receives
+    none.  ``samples`` is copied into the lattice when the line is packed, and edits re-pack the line
+    like every other field.  Not a ``Multipole``: no fuser or merger treats it as one."""
+
+    _base = (("knl", _zero_list), ("ksl", _zero_list), ("samples", tuple), ("sampling_frequency", 0),
+             ("frev", 0), ("start_turn", 0))
+
+    @property
+    def order(self):
+        return max(len(self.knl), len(self.ksl)) - 1
 
 
 class Elens(Element):

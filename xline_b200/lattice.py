@@ -28,6 +28,7 @@ T_END_TURN, T_END_CHUNK, T_DRIFT, T_DRIFT_EXACT, T_MULTIPOLE, T_MULTIPOLE_CURVED
 T_CAVITY, T_RFMULTIPOLE, T_XYSHIFT, T_SROTATION, T_DIPOLE_EDGE = range(6, 11)
 T_LIMIT_RECT, T_LIMIT_ELLIPSE, T_LIMIT_RECT_ELLIPSE, T_MONITOR, T_SAWTOOTH_CAVITY = range(11, 16)
 T_BEAMBEAM4D, T_SPACECHARGE, T_BEAMBEAM6D, T_LIMIT_POLYGON, T_MULTIPOLE_RAD = 16, 17, 18, 19, 20
+T_EXCITER = 0x40  # outside the contiguous single-element tags 0..20 (include/xline_b200.h)
 
 F_STRICT = 1
 F_BEAMFIELDS = 2
@@ -35,6 +36,7 @@ F_BB6D = 4
 F_LOW_ORDER = 8  # every multipole-family record has order <= LOW_ORDER_MAX (straight-line Horner kernels)
 F_POLYGONS = 16  # the lattice holds LIMIT_POLYGON records (only the kernels that carry the case run it)
 F_RADIATION = 32  # the lattice holds MULTIPOLE_RAD records (only the kernels that carry the case run it)
+F_EXCITER = 64  # the lattice holds EXCITER records and their data region after the chunks
 RADIATION_MODES = {"mean": 1, "quantum": 2}
 RAD_MAX_ELEMENTS = 1 << 24
 LOW_ORDER_MAX = 3
@@ -43,6 +45,8 @@ DEFAULT_CHUNK_WORDS = 2048  # 16 KiB per TMA bulk copy, 3 in flight per CTA
 MONITOR_FIELDS = ("x", "px", "y", "py", "zeta", "delta", "at_turn")
 
 _FACT = [math.factorial(i) for i in range(64)]
+MAX_ORDER = len(_FACT) - 1  # the highest multipole order the packer has coefficients for
+EXCITER_MAX_SAMPLES = (1 << 31) - 1  # per Exciter (16 GiB of waveform): offsets and indices stay exact
 
 
 def _f2u(x):
@@ -349,7 +353,42 @@ def _pack_multipole_rad(el, idx, radiation, seed):
     return rec
 
 
-def _pack_element(el, idx, strict, monitors, polygons=False):
+def _finite_floats(values, what):
+    a = np.array(values, dtype=np.float64).reshape(-1)
+    if not np.all(np.isfinite(a)):
+        raise ValueError("Exciter has a non-finite %s" % what)
+    return a
+
+
+def _pack_exciter(el, idx, data):
+    """XLB_T_EXCITER: [hdr,A][B,start_turn][n_samples,data_offset] then (kn_i,ks_i) i=order..0, with
+    A = sampling_frequency/frev, B = sampling_frequency/c.  The samples are appended to ``data`` (the
+    data region); ``data_offset`` is relative to the region here and made absolute by pack_line."""
+    fs, frev = float(el.sampling_frequency), float(el.frev)
+    if not (math.isfinite(fs) and fs > 0 and math.isfinite(frev) and frev > 0):
+        raise ValueError("Exciter needs finite sampling_frequency > 0 and frev > 0 (got %r, %r)"
+                         % (el.sampling_frequency, el.frev))
+    if isinstance(el.start_turn, bool) or not isinstance(el.start_turn, (int, np.integer)) or \
+            not -(1 << 62) <= int(el.start_turn) < (1 << 62):
+        raise ValueError("Exciter.start_turn must be an integer (got %r)" % (el.start_turn,))
+    if len(el.samples) > EXCITER_MAX_SAMPLES:
+        raise ValueError("Exciter has %d samples, more than the %d a record can address"
+                         % (len(el.samples), EXCITER_MAX_SAMPLES))
+    samples = _finite_floats(el.samples, "sample")
+    order = el.order
+    if order > MAX_ORDER:
+        raise ValueError("Exciter of order %d: the highest order is %d" % (order, MAX_ORDER))
+    knl = _pad(_finite_floats(el.knl, "knl"), order + 1)
+    ksl = _pad(_finite_floats(el.ksl, "ksl"), order + 1)
+    rec = _Rec(T_EXCITER, order, idx, fs / frev)
+    rec.f(fs / clight).i(int(el.start_turn), len(samples), sum(len(d) for d in data))
+    for i in range(order, -1, -1):
+        rec.f(knl[i] / _FACT[i], ksl[i] / _FACT[i])
+    data.append(samples)
+    return rec
+
+
+def _pack_element(el, idx, strict, monitors, polygons=False, data=None):
     name = type(el).__name__
     if name == "Drift":
         rec = _Rec(T_DRIFT, 0, idx, el.length)
@@ -425,6 +464,10 @@ def _pack_element(el, idx, strict, monitors, polygons=False):
         return _pack_spacecharge(el, idx, strict)
     if name == "BeamBeam6D":
         return _pack_beambeam6d(el, idx)
+    if name == "Exciter":
+        if strict:
+            raise ValueError("Exciter: the strict encoding has no exciter records (track with strict=False)")
+        return _pack_exciter(el, idx, data)
     if name == "LimitPolygon":
         if polygons:
             return _pack_limit_polygon(el, idx)
@@ -646,6 +689,11 @@ def pack_line(elements, strict=False, chunk_words=DEFAULT_CHUNK_WORDS, drop_noop
     own definition, see include/xline_b200.h).  ``False``, the default, refuses them with
     ``NotImplementedError`` like the reference's ``LimitPolygon.track``.
 
+    ``Exciter`` elements pack as XLB_T_EXCITER records, their samples into a data region after the
+    chunks (``words`` holds ``chunk_words * n_chunks`` words, then the samples); fast encoding only
+    (``ValueError`` for ``strict=True``), and such a line keeps its BeamBeam6D lenses in the tracking
+    kernel (no ``split_lenses``): a segment's kernel could not address the data region.
+
     ``radiation`` (None, "mean" or "quantum") and ``radiation_seed``: synchrotron radiation in every
     Multipole of length > 0, packed as XLB_T_MULTIPOLE_RAD records that never enter a block
     (include/xline_b200.h, DESIGN.md §4.9).  Fast encoding, one-species thin-lens lattices only:
@@ -658,6 +706,7 @@ def pack_line(elements, strict=False, chunk_words=DEFAULT_CHUNK_WORDS, drop_noop
         if len(elements) > RAD_MAX_ELEMENTS:
             raise ValueError("radiation: lines of more than 2^24 elements are not supported")
     monitors = dict(layout=[], words=0)
+    data = []  # the exciters' samples, in record order: the data region
     recs = []
     flags = F_STRICT if strict else 0
     counts = {}
@@ -728,13 +777,14 @@ def pack_line(elements, strict=False, chunk_words=DEFAULT_CHUNK_WORDS, drop_noop
                 pos += 1
             rec = _pack_thin_block(el, idx, aper, drift, strict)
         else:
-            rec = _pack_element(el, idx, strict, monitors, polygons)
+            rec = _pack_element(el, idx, strict, monitors, polygons, data)
         tag = rec.tag
         counts[tag] = counts.get(tag, 0) + 1
         if not hx_only:
             rec.flags &= ~HDR_HX_ONLY
         recs.append((tag, rec.words(), rec.s_word, rec.drift_len, rec.drift_before))
-    split = bool(split_lenses) and not strict and any(r[0] == T_BEAMBEAM6D for r in recs)
+    exciters = any(r[0] == T_EXCITER for r in recs)
+    split = bool(split_lenses) and not strict and not exciters and any(r[0] == T_BEAMBEAM6D for r in recs)
     for tag, _, _, _, _ in recs:
         if tag == T_BEAMBEAM6D:
             flags |= F_BB6D
@@ -744,11 +794,14 @@ def pack_line(elements, strict=False, chunk_words=DEFAULT_CHUNK_WORDS, drop_noop
             flags |= F_POLYGONS
         if tag == T_MULTIPOLE_RAD:
             flags |= F_RADIATION
+        if tag == T_EXCITER:
+            flags |= F_EXCITER
     if (flags & F_RADIATION) and (flags & (F_BEAMFIELDS | F_BB6D)):
         raise ValueError("radiation: lines with beam-beam or space-charge elements are not supported "
                          "(set radiation=None)")
     horner_orders = [(int(r[0]) >> 8) & 0xFF for tag, r, _, _, _ in recs
-                     if tag in (T_MULTIPOLE, T_MULTIPOLE_CURVED, T_MULTIPOLE_RAD) or (tag & 0xC0) == T_THIN_BLOCK]
+                     if tag in (T_MULTIPOLE, T_MULTIPOLE_CURVED, T_MULTIPOLE_RAD, T_EXCITER)
+                     or (tag & 0xC0) == T_THIN_BLOCK]
     if all(o <= LOW_ORDER_MAX for o in horner_orders):
         flags |= F_LOW_ORDER
     biggest = max([len(r[1]) for r in recs] + [0])
@@ -769,6 +822,7 @@ def pack_line(elements, strict=False, chunk_words=DEFAULT_CHUNK_WORDS, drop_noop
         segments.append([first, len(chunks) - first, kind])
 
     cur, first, s_pass = [], 0, 0.0
+    exciter_words = []  # (chunk, word in the chunk) of every exciter's data_offset
     for tag, r, s_word, drift_len, drift_before in recs:
         if split and tag == T_BEAMBEAM6D:
             if cur or len(chunks) > first:  # a tracking segment precedes the lens
@@ -783,15 +837,22 @@ def pack_line(elements, strict=False, chunk_words=DEFAULT_CHUNK_WORDS, drop_noop
         if s_word is not None:
             r = list(r)
             r[s_word] = _f2u(s_pass + drift_before)
+        if tag == T_EXCITER:
+            exciter_words.append((len(chunks), len(cur) + 5))
         cur = cur + r
         s_pass = s_pass + drift_len
     close_segment(cur, first, SEG_MAIN, s_pass)  # the closing tracking segment (may be empty) counts the turn
-    words = np.zeros(len(chunks) * chunk_words, dtype=np.uint64)
+    region = len(chunks) * chunk_words
+    words = np.zeros(region + sum(len(d) for d in data), dtype=np.uint64)
     for i, (ch, last) in enumerate(chunks):
         words[i * chunk_words: i * chunk_words + len(ch)] = np.array(ch, dtype=np.uint64)
         # fill the tail with END_CHUNK/END_TURN so a stray read can never run away
         tail = _hdr(T_END_TURN if last else T_END_CHUNK, 0, 0)
         words[i * chunk_words + len(ch): (i + 1) * chunk_words: 2] = tail
+    for ci, w in exciter_words:  # data_offset: from the start of the data region to an absolute word index
+        words[ci * chunk_words + w] += np.uint64(region)
+    if data:
+        words[region:] = np.concatenate(data).view(np.uint64)
     seg = np.array(segments, dtype=np.int32).reshape(-1, 3) if split else None
     return PackedLattice(words, chunk_words, len(chunks), len(elements), flags, monitors, counts, seg)
 
@@ -809,6 +870,7 @@ def element_specs(elements):
 
 
 RAD_OPS = {"mean": 74, "quantum": 82}  # per radiating multipole, photon sampling not counted
+EXCITER_OPS = 8  # per Exciter on top of its multipole: the sample index (6) and the two scalings by it
 
 
 def algorithmic_ops(elements, radiation=None):
@@ -818,7 +880,7 @@ def algorithmic_ops(elements, radiation=None):
     path length (8), and per half the particle's gamma, beta, kappa (9), the energy loss (mean: 9;
     quantum: n̄, exp, the first Poisson step: 13), add_to_energy (13) and the px, py scaling (3).
     The data-dependent rest of the quantum mode (further Poisson steps, ~23 per photon) is not
-    counted."""
+    counted.  An Exciter counts as a straight multipole of its order plus ``EXCITER_OPS``."""
     WOFZ = 100
     total = 0
     for el in elements:
@@ -831,6 +893,8 @@ def algorithmic_ops(elements, radiation=None):
             total += 18
         elif name == "Multipole":
             total += 10 * el.order + 4 + (19 if (el.hxl != 0 or el.hyl != 0) else 0)
+        elif name == "Exciter":
+            total += 10 * el.order + 4 + EXCITER_OPS
         elif name in ("Cavity", "SawtoothCavity"):
             total += 33
         elif name == "RFMultipole":

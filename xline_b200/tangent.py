@@ -103,6 +103,7 @@ def _launch(line, p, num_turns, threads_per_block, radiation, call):
 
 def track_tangent(line, p, tangent, num_turns=1, threads_per_block=0, radiation=False):
     """``Line.track_tangent``: see there."""
+    _refuse_exciter(line, "track_tangent")
     if p.device.type != "cuda":
         raise RuntimeError("track_tangent needs particles resident on a CUDA device (got %s)" % p.device)
     tangent._check_target(p)
@@ -149,6 +150,7 @@ class Envelope:
 
 def track_envelope(line, p, envelope, num_turns=1, threads_per_block=0):
     """``Line.track_envelope``: see there."""
+    _refuse_exciter(line, "track_envelope")
     if p.device.type != "cuda":
         raise RuntimeError("track_envelope needs particles resident on a CUDA device (got %s)" % p.device)
     envelope._check_target(p)
@@ -170,6 +172,13 @@ def _refuse_radiation(line, what):
     if getattr(line, "radiation", None) is not None:
         raise ValueError("%s: radiation is left out of the tangent map unless asked for (pass radiation=True, "
                          "or set Line.radiation = None)" % what)
+
+
+def _refuse_exciter(line, what):
+    for i, el in enumerate(line.elements):
+        if isinstance(el, E.Exciter):
+            raise ValueError("%s: element %d is an Exciter, a turn-dependent map without a tangent map or "
+                             "closed orbit (remove it, e.g. track a copy of the line without it)" % (what, i))
 
 
 def has_rf(line):
@@ -196,6 +205,7 @@ def closed_orbit(line, particles_like, guess=None, mode="auto", tol=1e-14, max_i
     its radiation (for a ``"quantum"`` line as well: the damped orbit is that of the mean loss), and
     only the 6d orbit exists -- delta is not conserved, so ``"4d"`` is refused.  On a line without
     radiation ``radiation=True`` changes nothing."""
+    _refuse_exciter(line, "closed_orbit")
     rad = bool(radiation) and getattr(line, "radiation", None) is not None
     if not rad:
         _refuse_radiation(line, "closed_orbit")
@@ -309,6 +319,7 @@ def radiation_equilibrium(line, particles_like, guess=None, tol=1e-14, max_iter=
 
     from .particles import Particles
 
+    _refuse_exciter(line, "radiation_equilibrium")
     if getattr(line, "radiation", None) is None:
         raise ValueError("radiation_equilibrium: the line does not radiate (set Line.radiation = 'mean' or 'quantum')")
     if not has_rf(line):
